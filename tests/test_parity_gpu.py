@@ -74,6 +74,10 @@ ESTEP_SHAPES = [
 	(500, 400, 12, 150, 20),   # cfg-4 topic count: cluster of 2-4 CTAs per document
 	(1000, 600, 10, 150, 20),  # cfg-3 topic count: cluster of 8 CTAs per document
 	(1000, 600, 6, 150, 0),    # max_iter = 0: statistics from the initial gamma
+	(2048, 300, 8, 60, 20),    # fp64: cluster kernel, whole tile in shared memory
+	(1040, 400, 16, 300, 20),  # mixed: documents of > 192 pairs on the cluster kernel, the rest in tensor memory
+	(2560, 300, 6, 100, 10),   # mixed: K beyond the tensor-memory kernel
+	(4096, 200, 4, 60, 5),     # the topic limit: cluster of 8 CTAs, 512 rows each
 ]
 
 
@@ -102,6 +106,7 @@ def test_update_variables_vs_oracle(capi, oracle_built, precision, K, V, B, max_
 	assert np.sum(sstats) == pytest.approx(sum(c for doc in lists for _, c in doc), rel=1e-6)
 	if precision == 'fp64':
 		assert stats['estep_doc_iterations'] == int(want_it.sum())    # identical early exits
+	assert stats['estep_sweeps'] == stats['estep_doc_iterations'] + B  # every E-step kernel counts its sweeps
 
 
 def test_update_variables_draws_gamma_when_no_latents(capi):

@@ -44,7 +44,7 @@ def ext_path():
 def build_library(force=False, verbose=False):
 	headers = [os.path.join(CSRC, f) for f in os.listdir(CSRC) if f.endswith(('.cuh', '.h'))]
 	headers.append(os.path.join(ROOT, 'include', 'trlda_b200.h'))
-	sources = [os.path.join(CSRC, 'kernels.cu'), os.path.join(CSRC, 'estep_fast.cu'), os.path.join(CSRC, 'estep_stream.cu'),
+	sources = [os.path.join(CSRC, 'kernels.cu'), os.path.join(CSRC, 'estep_stream.cu'),
 		os.path.join(CSRC, 'estep_tmem.cu'), os.path.join(CSRC, 'sample.cu'), os.path.join(CSRC, 'csc.cu'), os.path.join(CSRC, 'ingest.cu'),
 		os.path.join(CSRC, 'model.cu')]
 	objects = []

@@ -16,17 +16,19 @@
 // the sufficient statistics); the first sweep comes from HBM, the re-sweeps from L2 (148 documents x 600 KB in flight).
 //
 // Launch shape: one CTA of 16 warps per document (fp32 tile; 8 warps for the fp64 tile and for short columns), handed
-// out by the hardware scheduler.  Kept behind environment switches because they were measured, and lost (DESIGN.md §4):
-// a CLUSTER of C CTAs per document that split its COLUMNS and exchange one K-vector of partial sums per sweep by DSMEM
-// bulk copies (every CTA then adds the C partial vectors in rank order — identical bits everywhere — and updates gamma
-// redundantly); a persistent grid with fewer documents in flight; deeper rings with fewer warps.
+// out by the hardware scheduler, two ring slots per warp.  Measured at cfg-3 (fresh minibatch per step), and lost
+// (DESIGN.md §4): clusters of 2 CTAs per document that split the columns and exchange their partial sums per sweep
+// (102 ms/step against 74); with the bulk-copy ring, 12 warps x 3 slots (59.5 ms/step of E-step against 56.9),
+// 12 x 2 (60.3) and 8 x 4 (75.1): warps, not slots; a persistent grid (7 % slower: the documents of a CTA differ in
+// sweeps).
 #include "kernels.cuh"
 #include "special.cuh"
 
 #include <algorithm>
-#include <cstdlib>
 
 namespace trlda {
+
+constexpr int STREAM_DEPTH = 2;    // ring slots per warp
 
 template <typename T> struct SVec;
 template <> struct SVec<float> { using type = float4; static constexpr int N = 4; };
@@ -42,24 +44,21 @@ __host__ __device__ constexpr int stream_reduce_width(int NW, int kp, int elem) 
 }
 
 struct StreamSmem {
-	size_t ring, red, eth, gam, wsum, xstage, xall, wid, cnt, bar, rbar, total;
+	size_t ring, red, eth, gam, wsum, wid, cnt, rbar, total;
 };
 
-__host__ __device__ inline StreamSmem stream_smem_layout(int NW, int C, int depth, int kp, int n_cap, int elem) {
+__host__ __device__ inline StreamSmem stream_smem_layout(int NW, int kp, int n_cap, int elem) {
 	StreamSmem L;
 	size_t o = 0;
 	auto take = [&o](size_t bytes) { size_t at = o; o += (bytes + 15) & ~size_t(15); return at; };
-	L.ring = take((size_t) NW * depth * kp * elem);
+	L.ring = take((size_t) NW * STREAM_DEPTH * kp * elem);
 	L.red = take((size_t) stream_reduce_width(NW, kp, elem) * kp * elem);
 	L.eth = take((size_t) kp * elem);
 	L.gam = take((size_t) kp * 8);
 	L.wsum = take((size_t) NW * 8);
-	L.xstage = take(C > 1 ? (size_t) 2 * kp * elem : 0);          // [2] outgoing partial vector
-	L.xall = take(C > 1 ? (size_t) 2 * C * kp * elem : 0);        // [2][C] incoming partial vectors
 	L.wid = take((size_t) n_cap * 4);
 	L.cnt = take((size_t) n_cap * 4);
-	L.bar = take(32);
-	L.rbar = take((size_t) NW * depth * 8);                // one mbarrier per ring slot (bulk-copy variant)
+	L.rbar = take((size_t) NW * STREAM_DEPTH * 8);         // one mbarrier per ring slot (bulk-copy variant)
 	L.total = o;
 	return L;
 }
@@ -72,26 +71,12 @@ static inline int stream_nvec(int K, int elem) {
 	return nvec;
 }
 
-// launch shape: cluster size, warps per CTA, ring slots per warp.  Measured at cfg-3 (fresh minibatch per step):
-// clusters lose to their per-sweep exchange (2 x 8 warps: 102 ms/step against 74); with the bulk-copy ring the E-step
-// takes 56.9 ms/step with 16 warps x 2 slots, 59.5 with 12 x 3, 60.3 with 12 x 2, 75.1 with 8 x 4: warps, not slots.
-// TRLDA_STREAM_CLUSTER / TRLDA_STREAM_WARPS / TRLDA_STREAM_DEPTH override (only compiled combinations are accepted).
-struct StreamShape { int C, NW, D; };
-static const StreamShape kFloatShapes[] = {{1, 16, 2}, {1, 12, 3}, {1, 12, 2}, {1, 8, 4}, {1, 8, 2}, {1, 4, 2}, {2, 8, 2}};
-static const StreamShape kDoubleShapes[] = {{1, 8, 2}, {1, 4, 2}, {1, 4, 4}, {2, 4, 2}};
-
-static StreamShape stream_shape(int elem, int K) {
-	const StreamShape* shapes = elem == 4 ? kFloatShapes : kDoubleShapes;
-	const int count = elem == 4 ? (int) (sizeof(kFloatShapes) / sizeof(StreamShape)) : (int) (sizeof(kDoubleShapes) / sizeof(StreamShape));
-	const char* ec = getenv("TRLDA_STREAM_CLUSTER");
-	const char* ew = getenv("TRLDA_STREAM_WARPS");
-	const char* ed = getenv("TRLDA_STREAM_DEPTH");
-	const int C = ec ? atoi(ec) : 0, NW = ew ? atoi(ew) : 0, D = ed ? atoi(ed) : 0;
-	for(int i = 0; i < count; ++i)
-		if((!C || shapes[i].C == C) && (!NW || shapes[i].NW == NW) && (!D || shapes[i].D == D))
-			return (C || NW || D) ? shapes[i] : (elem == 4 && K * elem < 2048 ? StreamShape{1, 8, 2} : shapes[i]);
-	return shapes[0];
-}
+// Columns of 2 KB and more travel by cp.async.bulk (one copy per column, written by the copy engine); 16-byte cp.async
+// (LDGSTS) costs the load/store pipe 8 cycles per 512 bytes: 63.8 against 56.9 ms/step of E-step at cfg-3.  Short
+// columns (K = 100 or 200: 400-1600 bytes) stay with cp.async, the per-copy cost of the bulk path does not pay: cfg-5
+// (K = 200) 117 ms per batch with bulk copies and one 16-warp CTA per SM against 33 ms with two 8-warp CTAs.
+static bool stream_bulk(int K, int elem) { return K * elem >= 2048; }
+static int stream_warps(int K, int elem) { return elem == 4 && stream_bulk(K, elem) ? 16 : 8; }
 
 // applicable?  (aligned columns, K small enough for the per-lane register tile, everything fits in shared memory)
 bool stream_estep_applicable(int K, int n_max, int elem, int smem_optin) {
@@ -102,17 +87,10 @@ bool stream_estep_applicable(int K, int n_max, int elem, int smem_optin) {
 		return false;
 	const int kp = nvec * 32 * (16 / elem);
 	const int n_cap = std::max(32, (n_max + 31) / 32 * 32);
-	const StreamShape sh = stream_shape(elem, K);
-	return stream_smem_layout(sh.NW, sh.C, sh.D, kp, n_cap, elem).total <= (size_t) smem_optin - 1024;
+	return stream_smem_layout(stream_warps(K, elem), kp, n_cap, elem).total <= (size_t) smem_optin - 1024;
 }
 
 __device__ __forceinline__ uint32_t s_smem_u32(const void* p) { return (uint32_t) __cvta_generic_to_shared(p); }
-
-__device__ __forceinline__ uint32_t s_map_to_rank(uint32_t smem_addr, int rank) {
-	uint32_t remote;
-	asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(remote) : "r"(smem_addr), "r"(rank));
-	return remote;
-}
 
 __device__ __forceinline__ void s_mbar_wait(uint32_t bar, uint32_t parity) {
 	uint32_t done = 0;
@@ -122,47 +100,28 @@ __device__ __forceinline__ void s_mbar_wait(uint32_t bar, uint32_t parity) {
 			: "=r"(done) : "r"(bar), "r"(parity) : "memory");
 }
 
-template <typename T, int NW, int NVEC, int C, bool BULK, int STREAM_DEPTH>
-__global__ void __launch_bounds__(NW * 32, (C == 1 && NW == 4 ? 3 : (C == 1 && NW == 8 && sizeof(T) == 4 ? 2 : 1)))
-k_estep_stream(EStepArgs a, DeviceDocs docs, const int32_t* __restrict__ order, int64_t doc_offset, int64_t count, int n_cap) {
+template <typename T, int NW, int NVEC, bool BULK>
+__global__ void __launch_bounds__(NW * 32, (NW == 8 && sizeof(T) == 4 ? 2 : 1))
+k_estep_stream(EStepArgs a, DeviceDocs docs, const int32_t* __restrict__ order, int64_t doc_offset, int n_cap) {
 	extern __shared__ __align__(128) unsigned char smem[];
 	using V = typename SVec<T>::type;
 	constexpr int VN = SVec<T>::N;
 	constexpr int KP = NVEC * 32 * VN;                       // padded number of topic rows
 	constexpr int NT = NW * 32;
-	constexpr int TW = NW * C;                               // warps working on one document
 	constexpr int RW = stream_reduce_width(NW, KP, (int) sizeof(T));
-	const StreamSmem L = stream_smem_layout(NW, C, STREAM_DEPTH, KP, n_cap, (int) sizeof(T));
+	const StreamSmem L = stream_smem_layout(NW, KP, n_cap, (int) sizeof(T));
 	T* ring = reinterpret_cast<T*>(smem + L.ring);
 	T* red = reinterpret_cast<T*>(smem + L.red);
 	T* eth = reinterpret_cast<T*>(smem + L.eth);
 	double* gam = reinterpret_cast<double*>(smem + L.gam);
 	double* wsum = reinterpret_cast<double*>(smem + L.wsum);
-	T* xstage = reinterpret_cast<T*>(smem + L.xstage);
-	T* xall = reinterpret_cast<T*>(smem + L.xall);
 	int* wid = reinterpret_cast<int*>(smem + L.wid);
 	int* cnt = reinterpret_cast<int*>(smem + L.cnt);
-	uint64_t* bar = reinterpret_cast<uint64_t*>(smem + L.bar);
 	uint64_t* rbar = reinterpret_cast<uint64_t*>(smem + L.rbar);
 
-	int rank = 0;
-	if(C > 1)
-		asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(rank));
 	const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-	const int gw = rank * NW + warp;                          // this warp's index among the document's warps
 	const int K = a.K;
 	const T* __restrict__ beta = static_cast<const T*>(a.beta);
-
-	if(C > 1) {
-		if(tid == 0) {
-			asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(s_smem_u32(bar)));
-			asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(s_smem_u32(bar + 1)));
-			asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-		}
-		__syncthreads();
-		// start-up cluster barrier (exchange barriers initialised everywhere): arrive now, wait before the first push
-		asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-	}
 
 	// this lane's rows: vectors v = 0..NVEC-1 cover rows (v * 32 + lane) * VN .. + VN
 	T* my_ring = ring + (size_t) warp * STREAM_DEPTH * KP;
@@ -218,22 +177,14 @@ k_estep_stream(EStepArgs a, DeviceDocs docs, const int32_t* __restrict__ order, 
 		__syncthreads();
 	}
 
-	const uint32_t xstage_addr = s_smem_u32(xstage), xall_addr = s_smem_u32(xall), bar_addr = s_smem_u32(bar);
-	constexpr uint32_t XBYTES = KP * sizeof(T);
-
-	int sweep = 0;         // counts the sweeps (= cluster exchanges) of all documents of this CTA
-	// debug phase timers (TRLDA_ESTEP_TICKS=1), thread 0's view: setup, stream, fold, exchange, update, test
+	// debug phase timers (TRLDA_ESTEP_TICKS=1), thread 0's view: setup, stream, fold, update, test
 	const bool timing = a.ticks != nullptr && tid == 0;
-	long long tk[6] = {0, 0, 0, 0, 0, 0}, t_mark = 0;
-	long long docs_done = 0;
+	long long tk[5] = {0, 0, 0, 0, 0}, t_mark = 0;
 	#define TRLDA_TICK(i) if(timing) { const long long now = clock64(); tk[i] += now - t_mark; t_mark = now; }
-	// persistent grid: the documents in flight (and with them the footprint of their tiles in L2) are set by the grid
-	for(int64_t item = blockIdx.x / C; item < count; item += gridDim.x / C) {
-	const int64_t slot = doc_offset + item;
+	const int64_t slot = doc_offset + blockIdx.x;
 	const int64_t d = order ? order[slot] : slot;
 	const int64_t begin = docs.doc_ptr[d];
 	const int n = (int) (docs.doc_ptr[d + 1] - begin);
-	__syncthreads();       // the previous document's last reads of the shared vectors
 	if(timing)
 		t_mark = clock64();
 	for(int j = tid; j < n; j += NT) {
@@ -269,7 +220,7 @@ k_estep_stream(EStepArgs a, DeviceDocs docs, const int32_t* __restrict__ order, 
 	int stage = 0;
 	while(true) {
 		const bool final_sweep = converged || it >= a.max_iter;
-		// ---- one sweep over the document's columns: this warp takes columns gw, gw + TW, ... ---------------------------
+		// ---- one sweep over the document's columns: this warp takes columns warp, warp + NW, ... ------------------------
 		T e[NVEC][VN], acc[NVEC][VN];
 		#pragma unroll
 		for(int v = 0; v < NVEC; ++v) {
@@ -279,12 +230,12 @@ k_estep_stream(EStepArgs a, DeviceDocs docs, const int32_t* __restrict__ order, 
 				acc[v][q] = T(0);
 		}
 		// M = number of columns of this warp.  If the ring was not primed by the previous sweep, fill it now.
-		const int M = gw < n ? (n - gw + TW - 1) / TW : 0;
+		const int M = warp < n ? (n - warp + NW - 1) / NW : 0;
 		if(!primed) {
 			#pragma unroll
 			for(int s = 0; s < STREAM_DEPTH; ++s) {
 				if(s < M)
-					issue(gw + s * TW, s);
+					issue(warp + s * NW, s);
 				commit();
 			}
 			stage = 0;
@@ -294,7 +245,7 @@ k_estep_stream(EStepArgs a, DeviceDocs docs, const int32_t* __restrict__ order, 
 		// the (L2) latency of the next sweep hides behind the reduction and the psi evaluations
 		const bool prime_next = !final_sweep && M >= STREAM_DEPTH;
 		for(int mcol = 0; mcol < M; ++mcol) {
-			const int j = gw + mcol * TW;
+			const int j = warp + mcol * NW;
 			wait_slot(stage);
 			__syncwarp();
 			const T* col = my_ring + (size_t) stage * KP;
@@ -340,9 +291,9 @@ k_estep_stream(EStepArgs a, DeviceDocs docs, const int32_t* __restrict__ order, 
 			__syncwarp();
 			const int mn = mcol + STREAM_DEPTH;
 			if(mn < M)
-				issue(gw + mn * TW, stage);
+				issue(warp + mn * NW, stage);
 			else if(prime_next)
-				issue(gw + (mn - M) * TW, stage);
+				issue(warp + (mn - M) * NW, stage);
 			commit();
 			stage = stage + 1 == STREAM_DEPTH ? 0 : stage + 1;
 		}
@@ -385,35 +336,6 @@ k_estep_stream(EStepArgs a, DeviceDocs docs, const int32_t* __restrict__ order, 
 		__syncthreads();
 
 		TRLDA_TICK(2)
-		const int buf = sweep & 1;
-		if(C > 1) {
-			// ---- cluster exchange: this CTA's partial K-vector goes to every CTA of the cluster (itself included) -------
-			if(tid == 0)
-				asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;"
-					::"r"(bar_addr + 8 * buf), "r"((uint32_t) C * XBYTES) : "memory");
-			T* out = xstage + (size_t) buf * KP;
-			for(int r = tid; r < KP; r += NT) {
-				double partial = 0.0;
-				#pragma unroll 4
-				for(int q = 0; q < RW; ++q)
-					partial += (double) red[(size_t) q * KP + r];
-				out[r] = (T) partial;
-			}
-			__syncthreads();
-			if(sweep == 0)
-				asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-			if(tid < C) {
-				asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-				const uint32_t dst = s_map_to_rank(xall_addr + (uint32_t) ((buf * C + rank) * XBYTES), tid);
-				const uint32_t dst_bar = s_map_to_rank(bar_addr + 8 * buf, tid);
-				asm volatile(
-					"cp.async.bulk.shared::cluster.shared::cta.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-					::"r"(dst), "r"(xstage_addr + (uint32_t) buf * XBYTES), "r"(XBYTES), "r"(dst_bar) : "memory");
-			}
-			s_mbar_wait(bar_addr + 8 * buf, (uint32_t) ((sweep >> 1) & 1));
-		}
-
-		TRLDA_TICK(3)
 		double delta_local = 0.0;
 		// two rows per thread and trip, so that their chains (sum of the partials, psi, exp) overlap
 		for(int r0 = tid; r0 < K; r0 += 2 * NT) {
@@ -425,27 +347,20 @@ k_estep_stream(EStepArgs a, DeviceDocs docs, const int32_t* __restrict__ order, 
 				live[u] = r0 + u * NT < K;
 				row[u] = live[u] ? r0 + u * NT : r0;
 				const int r = row[u];
-				total[u] = 0.0;
-				if(C > 1) {
-					#pragma unroll
-					for(int src = 0; src < C; ++src)
-						total[u] += (double) xall[(size_t) (buf * C + src) * KP + r];   // rank order: identical bits in every CTA
-				} else {
-					// the partials are T: they are added in T (mixed mode: one float32 rounding per partial, like the
-					// accumulators themselves) and converted once — F2F.F64.F32 per partial was a cost of its own
-					T part = red[r];
-					#pragma unroll
-					for(int q = 1; q < RW; ++q)
-						part += red[(size_t) q * KP + r];
-					total[u] = (double) part;
-				}
+				// the partials are T: they are added in T (mixed mode: one float32 rounding per partial, like the
+				// accumulators themselves) and converted once — F2F.F64.F32 per partial was a cost of its own
+				T part = red[r];
+				#pragma unroll
+				for(int q = 1; q < RW; ++q)
+					part += red[(size_t) q * KP + r];
+				total[u] = (double) part;
 				eo[u] = (double) eth[r];
 			}
 			if(final_sweep) {
 				#pragma unroll
 				for(int u = 0; u < 2; ++u) {
 					const int r = row[u];
-					if(live[u] && (C == 1 || r % C == rank)) {             // the CTAs share the output rows
+					if(live[u]) {
 						a.doc_stat[d * K + r] = total[u] * eo[u];
 						a.gamma[d * K + r] = gam[r];
 						a.etheta[d * K + r] = eo[u];
@@ -476,8 +391,7 @@ k_estep_stream(EStepArgs a, DeviceDocs docs, const int32_t* __restrict__ order, 
 				}
 			}
 		}
-		++sweep;
-		TRLDA_TICK(4)
+		TRLDA_TICK(3)
 		if(final_sweep)
 			break;
 		delta_local = warp_sum(delta_local);
@@ -490,121 +404,67 @@ k_estep_stream(EStepArgs a, DeviceDocs docs, const int32_t* __restrict__ order, 
 		++it;
 		converged = delta / K < a.threshold;                           // lda.cpp:202
 		// no second barrier: wsum and red are next written behind the barriers of the coming sweep's fold
-		TRLDA_TICK(5)
+		TRLDA_TICK(4)
 	}
-	++docs_done;
-	if(rank == 0 && tid == 0 && a.iterations)
+	if(tid == 0 && a.iterations)
 		a.iterations[d] = it;
-	if(rank == 0 && tid == 0 && a.sweeps)
+	if(tid == 0 && a.sweeps)
 		atomicAdd(a.sweeps, (unsigned long long) (it + 1));
-	}
-	if(timing && rank == 0) {
-		for(int i = 0; i < 6; ++i)
+	if(timing) {
+		for(int i = 0; i < 5; ++i)
 			atomicAdd(a.ticks + i, (unsigned long long) tk[i]);
-		atomicAdd(a.ticks + 14, (unsigned long long) sweep);
-		atomicAdd(a.ticks + 15, (unsigned long long) docs_done);
+		atomicAdd(a.ticks + 14, (unsigned long long) (it + 1));
+		atomicAdd(a.ticks + 15, 1ull);
 	}
 	#undef TRLDA_TICK
-	if(C > 1) {
-		// nobody reads this CTA's staging buffers any more once every CTA has passed its last exchange
-		asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-		asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-	}
 }
 
-// documents in flight: one CTA (cluster) per document, handed out by the hardware scheduler as SMs free up (a static
-// persistent grid measured 7 % slower: the documents of a CTA differ in sweeps).  TRLDA_STREAM_GRID = n runs a
-// persistent grid of n documents in flight instead (experiments on the L2 footprint of the tiles).
-static int64_t stream_grid_docs(int64_t count) {
-	if(const char* e = getenv("TRLDA_STREAM_GRID"))
-		if(atoi(e) > 0)
-			return std::min<int64_t>(count, atoi(e));
-	return count;
-}
-
-template <typename T, int NW, int NVEC, int C, bool BULK, int DEPTH>
-static void launch_stream_b(const EStepArgs& args, const DeviceDocs& docs, const int32_t* order, int64_t offset,
+template <typename T, int NW, int NVEC, bool BULK>
+static void launch_stream_k(const EStepArgs& args, const DeviceDocs& docs, const int32_t* order, int64_t offset,
                             int64_t count, int n_cap, size_t smem, cudaStream_t s) {
-	auto kernel = k_estep_stream<T, NW, NVEC, C, BULK, DEPTH>;
+	auto kernel = k_estep_stream<T, NW, NVEC, BULK>;
 	static size_t configured = 0;      // per instantiation: the attribute is set once (and again only if the tile grows)
 	if(smem > configured) {
 		cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem);
 		configured = smem;
 	}
-	cudaLaunchConfig_t cfg = {};
-	cfg.gridDim = dim3((unsigned) (stream_grid_docs(count) * C));
-	cfg.blockDim = dim3(NW * 32);
-	cfg.dynamicSmemBytes = smem;
-	cfg.stream = s;
-	cudaLaunchAttribute attr[1];
-	attr[0].id = cudaLaunchAttributeClusterDimension;
-	attr[0].val.clusterDim.x = C;
-	attr[0].val.clusterDim.y = 1;
-	attr[0].val.clusterDim.z = 1;
-	cfg.attrs = attr;
-	cfg.numAttrs = C > 1 ? 1 : 0;
-	cudaLaunchKernelEx(&cfg, kernel, args, docs, order, offset, count, n_cap);
+	kernel<<<(unsigned) count, NW * 32, smem, s>>>(args, docs, order, offset, n_cap);
 }
 
-// columns travel by cp.async.bulk (one copy per column, written by the copy engine); TRLDA_STREAM_BULK = 0 goes back to
-// 16-byte cp.async (LDGSTS), which costs the load/store pipe 8 cycles per 512 bytes: 63.8 against 56.9 ms/step of E-step
-// Short columns (K = 100 or 200: 400-1600 bytes) stay with cp.async, the per-copy cost of the bulk path does not pay:
-// cfg-5 (K = 200) 117 ms per batch with bulk copies and one 16-warp CTA per SM against 33 ms with two 8-warp CTAs.
-static bool stream_bulk(int column_bytes) {
-	static const int mode = [] { const char* e = getenv("TRLDA_STREAM_BULK"); return e ? (atoi(e) != 0 ? 1 : 0) : -1; }();
-	return mode < 0 ? column_bytes >= 2048 : mode == 1;
-}
-
-template <typename T, int NW, int NVEC, int C, int DEPTH>
-static void launch_stream_t(const EStepArgs& args, const DeviceDocs& docs, const int32_t* order, int64_t offset,
-                            int64_t count, int n_cap, size_t smem, cudaStream_t s) {
-	if(C == 1 && stream_bulk(args.K * (int) sizeof(T)))
-		launch_stream_b<T, NW, NVEC, 1, true, DEPTH>(args, docs, order, offset, count, n_cap, smem, s);
-	else
-		launch_stream_b<T, NW, NVEC, C, false, DEPTH>(args, docs, order, offset, count, n_cap, smem, s);
-}
-
-template <typename T, int NW, int C, int DEPTH>
+template <typename T, int NW, bool BULK>
 static void launch_stream_v(int nvec, const EStepArgs& args, const DeviceDocs& docs, const int32_t* order, int64_t offset,
                             int64_t count, int n_cap, size_t smem, cudaStream_t s) {
 	constexpr int MAXV = sizeof(T) == 4 ? 8 : 16;
 	switch(nvec) {
-		case 1: launch_stream_t<T, NW, 1, C, DEPTH>(args, docs, order, offset, count, n_cap, smem, s); break;
-		case 2: launch_stream_t<T, NW, 2, C, DEPTH>(args, docs, order, offset, count, n_cap, smem, s); break;
-		case 4: launch_stream_t<T, NW, 4, C, DEPTH>(args, docs, order, offset, count, n_cap, smem, s); break;
-		case 8: launch_stream_t<T, NW, 8, C, DEPTH>(args, docs, order, offset, count, n_cap, smem, s); break;
-		default: launch_stream_t<T, NW, MAXV, C, DEPTH>(args, docs, order, offset, count, n_cap, smem, s); break;
+		case 1: launch_stream_k<T, NW, 1, BULK>(args, docs, order, offset, count, n_cap, smem, s); break;
+		case 2: launch_stream_k<T, NW, 2, BULK>(args, docs, order, offset, count, n_cap, smem, s); break;
+		case 4: launch_stream_k<T, NW, 4, BULK>(args, docs, order, offset, count, n_cap, smem, s); break;
+		case 8: launch_stream_k<T, NW, 8, BULK>(args, docs, order, offset, count, n_cap, smem, s); break;
+		default: launch_stream_k<T, NW, MAXV, BULK>(args, docs, order, offset, count, n_cap, smem, s); break;
 	}
 }
 
+// one CTA per document, handed out by the hardware scheduler as SMs free up
 void launch_estep_stream(const EStepArgs& args, const DeviceDocs& docs, const int32_t* order, int64_t offset,
-                         int64_t count, int n_max, int elem_size, bool cold, cudaStream_t s) {
-	(void) cold;
+                         int64_t count, int n_max, int elem_size, cudaStream_t s) {
 	if(count == 0)
 		return;
-	const StreamShape sh = stream_shape(elem_size, args.K);
-	const int nvec = stream_nvec(args.K, elem_size);
+	const int K = args.K;
+	const int nvec = stream_nvec(K, elem_size);
 	const int n_cap = std::max(32, (n_max + 31) / 32 * 32);
 	const int kp = nvec * 32 * (16 / elem_size);
-	const size_t smem = stream_smem_layout(sh.NW, sh.C, sh.D, kp, n_cap, elem_size).total;
-#define TRLDA_STREAM_CASE(TYPE, CLUSTER, WARPS, DEPTH) \
-	if(sh.C == CLUSTER && sh.NW == WARPS && sh.D == DEPTH) { \
-		launch_stream_v<TYPE, WARPS, CLUSTER, DEPTH>(nvec, args, docs, order, offset, count, n_cap, smem, s); return; }
-	if(elem_size == 4) {                                  // keep in step with kFloatShapes / kDoubleShapes
-		TRLDA_STREAM_CASE(float, 1, 12, 3)
-		TRLDA_STREAM_CASE(float, 1, 16, 2)
-		TRLDA_STREAM_CASE(float, 1, 12, 2)
-		TRLDA_STREAM_CASE(float, 1, 8, 4)
-		TRLDA_STREAM_CASE(float, 1, 8, 2)
-		TRLDA_STREAM_CASE(float, 1, 4, 2)
-		TRLDA_STREAM_CASE(float, 2, 8, 2)
+	const size_t smem = stream_smem_layout(stream_warps(K, elem_size), kp, n_cap, elem_size).total;
+	if(elem_size == 4) {                                  // warps per CTA: stream_warps()
+		if(stream_bulk(K, elem_size))
+			launch_stream_v<float, 16, true>(nvec, args, docs, order, offset, count, n_cap, smem, s);
+		else
+			launch_stream_v<float, 8, false>(nvec, args, docs, order, offset, count, n_cap, smem, s);
 	} else {
-		TRLDA_STREAM_CASE(double, 1, 8, 2)
-		TRLDA_STREAM_CASE(double, 1, 4, 2)
-		TRLDA_STREAM_CASE(double, 1, 4, 4)
-		TRLDA_STREAM_CASE(double, 2, 4, 2)
+		if(stream_bulk(K, elem_size))
+			launch_stream_v<double, 8, true>(nvec, args, docs, order, offset, count, n_cap, smem, s);
+		else
+			launch_stream_v<double, 8, false>(nvec, args, docs, order, offset, count, n_cap, smem, s);
 	}
-#undef TRLDA_STREAM_CASE
 }
 
 }  // namespace trlda

@@ -208,7 +208,7 @@ __host__ __device__ inline EStepSmem estep_smem_layout(int C, int kc, int n_cap,
 	return L;
 }
 
-EStepPlan plan_estep(int K, int n_max, int elem, int smem_optin, int force_cluster) {
+EStepPlan plan_estep(int K, int n_max, int elem, int smem_optin) {
 	EStepPlan best;
 	const int n_cap = std::max(32, round_up(n_max, 32));
 	const size_t budget_full = (size_t) smem_optin - 1024;          // 1 KB per CTA is reserved by the driver
@@ -219,12 +219,10 @@ EStepPlan plan_estep(int K, int n_max, int elem, int smem_optin, int force_clust
 	for(int pass = 0; pass < 2 && chosen < 0; ++pass)
 		for(int ci = 0; ci < 4; ++ci) {
 			const int C = candidates[ci];
-			if(force_cluster > 0 && C != force_cluster)
-				continue;
 			const int kc = round_up(ceil_div(K, C), 32);
 			if((C - 1) * kc >= K && C > 1)
 				continue;                                              // a CTA without rows
-			if(kc > 256 && C < 8 && force_cluster <= 0)
+			if(kc > 256 && C < 8)
 				continue;
 			const EStepSmem L = estep_smem_layout(C, kc, n_cap, n_cap, elem);
 			if(L.total <= (pass == 0 ? budget_half : budget_full)) {
@@ -235,7 +233,7 @@ EStepPlan plan_estep(int K, int n_max, int elem, int smem_optin, int force_clust
 	int C = chosen;
 	if(C < 0) {
 		// nothing fits entirely: largest usable cluster, keep as many columns on chip as fit
-		C = force_cluster > 0 ? force_cluster : 8;
+		C = 8;
 		while(C > 1 && (C - 1) * round_up(ceil_div(K, C), 32) >= K)
 			C /= 2;
 	}
@@ -470,6 +468,8 @@ k_estep(EStepArgs a, DeviceDocs docs, const int32_t* __restrict__ order, int64_t
 	}
 	if(rank == 0 && tid == 0 && a.iterations)
 		a.iterations[d] = it;
+	if(rank == 0 && tid == 0 && a.sweeps)
+		atomicAdd(a.sweeps, (unsigned long long) (it + 1));
 }
 
 static int g_estep_smem_optin = 0;

@@ -53,11 +53,10 @@ struct EStepPlan {
 	int n_cap = 0;        // capacity of the per-column vectors in shared memory
 	int n_fit = 0;        // columns of the tile kept in shared memory (the rest stream from L2)
 	size_t smem = 0;      // dynamic shared memory per CTA
-	bool fast = false;    // whole tile resident + TMA gather + vectorised passes (estep_fast.cu)
 };
 
 // plans the E-step launch for (K, longest document, element size of the expElogbeta working copy)
-EStepPlan plan_estep(int K, int n_max, int elem_size, int smem_optin, int force_cluster);
+EStepPlan plan_estep(int K, int n_max, int elem_size, int smem_optin);
 
 struct EStepArgs {
 	int K = 0;
@@ -93,18 +92,11 @@ void launch_estep(const EStepPlan& plan, const EStepArgs& args, const DeviceDocs
                   int64_t offset, int64_t count, int elem_size, cudaStream_t s);
 void configure_estep(int smem_optin);
 
-// tuned kernel for documents whose tile fits in the cluster's shared memory (estep_fast.cu); plan.cluster == 0
-// means "not applicable" (use the generic kernel)
-EStepPlan plan_estep_fast(int K, int n_max, int elem_size, int smem_optin, int force_cluster);
-void launch_estep_fast(const EStepPlan& plan, const EStepArgs& args, const DeviceDocs& docs, const int32_t* order,
-                       int64_t offset, int64_t count, int elem_size, cudaStream_t s);
-void configure_estep_fast(int smem_optin);
-
-// streaming kernel for warm-started documents (estep_stream.cu): one CTA per document, columns streamed through
-// per-warp cp.async rings, one sweep per inner iteration
+// streaming kernel (estep_stream.cu): one CTA per document, columns streamed through per-warp cp.async rings, one sweep
+// per inner iteration
 bool stream_estep_applicable(int K, int n_max, int elem_size, int smem_optin);
 void launch_estep_stream(const EStepArgs& args, const DeviceDocs& docs, const int32_t* order, int64_t offset,
-                         int64_t count, int n_max, int elem_size, bool cold, cudaStream_t s);
+                         int64_t count, int n_max, int elem_size, cudaStream_t s);
 
 // tensor-memory-resident kernel for the mixed mode (estep_tmem.cu): a cluster of CTAs keeps a document's float32 tile
 // in tensor memory (+ registers) for all inner iterations; documents of up to tmem_estep_max_len() pairs

@@ -195,7 +195,6 @@ struct trlda_model {
 
 	cudaStream_t stream = nullptr;
 	int smem_optin = 0, num_sms = 0;
-	int force_cluster = 0;
 
 	// K x V state: lambda lives in lam[cur]; the other buffer receives the next lambda (lambda' = old buffer)
 	DevBuf lam[2];
@@ -216,7 +215,6 @@ struct trlda_model {
 	// documents longer than 192 / 160 / 128 / 64 pairs (prefix lengths of the length-sorted order): the cuts between
 	// the tile shapes of the tensor-memory E-step kernel
 	int64_t len_gt[4] = {0, 0, 0, 0};
-	bool force_generic = false;
 	// parked resident minibatches (trlda_upload_docs_slot / trlda_select_docs): the live buffers are swapped with a slot
 	// Multi-GPU "gather" exchange (default for the mixed mode): every rank holds the token list of the WHOLE minibatch,
 	// sorted by word and restricted to the words it owns; per trust-region iteration the ranks all-gather etheta and the
@@ -253,15 +251,14 @@ struct trlda_model {
 	static const int kAuxStreams = 3;
 	cudaStream_t aux[kAuxStreams] = {nullptr, nullptr, nullptr};
 	cudaEvent_t fork_event = nullptr, join_event[kAuxStreams] = {nullptr, nullptr, nullptr};
-	bool concurrent_buckets = true;
 	bool tmem_mode = true;       // TRLDA_ESTEP_TMEM=0: never use the tensor-memory-resident kernel (mixed mode)
-	int stream_mode = 2;   // TRLDA_ESTEP_STREAM: 0 never use the streaming kernel, 1 only for warm-started E-steps, 2 always (default)
+	bool stream_ran = false;     // the streaming E-step kernel has run (its phase timers are printed by trlda_destroy)
 	DevBuf sweeps;   // device counter behind trlda_stats.estep_sweeps
 	// trlda_sample: row-wise CDFs of beta ~ Dirichlet(lambda), padded token buffers, and the host copy handed to the caller
 	DevBuf sample_cdf, sample_tokens, sample_counts, sample_lengths;
 	std::vector<int64_t> sample_ptr;
 	std::vector<int32_t> sample_ids, sample_cts;
-	DevBuf ticks;    // debug phase timers of the fast E-step kernel (TRLDA_ESTEP_TICKS=1)
+	DevBuf ticks;    // debug phase timers of the E-step kernels (TRLDA_ESTEP_TICKS=1)
 	PinnedBuf staging, readback;
 	int64_t docs_total_count = 0;    // sum of all counts in the (global) minibatch
 	int64_t global_B = 0;            // documents over all ranks
@@ -918,6 +915,41 @@ int fresh_gamma(trlda_model* m) {
 	return check_launch(m, "gamma_rng");
 }
 
+// the shared-memory cluster kernel (kernels.cu) on the documents order[0, end): one launch per length bucket, its tile
+// sized for the bucket's longest document.  Bucket i runs on stream i % (1 + kAuxStreams) (0 = the main stream), so
+// that CTAs of buckets with different shared-memory footprints can share an SM and the buckets' tails overlap; the
+// main stream waits for all of them.
+int run_estep_buckets(trlda_model* m, const EStepArgs& a, int64_t end) {
+	size_t nb = 0;
+	while(nb < m->buckets.size() && m->buckets[nb].offset < end)
+		++nb;
+	const bool fork = nb > 1 && m->aux[0] != nullptr;
+	Launch span(m, KK_ESTEP);   // one timing span for the whole E-step (the bucket launches overlap)
+	m->stats.total_launches--;  // the span itself is not a kernel; the launches are counted below
+	if(fork) {
+		CUDA_TRY(m, cudaEventRecord(m->fork_event, m->stream));
+		for(int i = 0; i < trlda_model::kAuxStreams; ++i)
+			CUDA_TRY(m, cudaStreamWaitEvent(m->aux[i], m->fork_event, 0));
+	}
+	for(size_t i = 0; i < nb; ++i) {
+		const trlda_model::Bucket& bucket = m->buckets[i];
+		const int lane = fork ? (int) (i % (1 + trlda_model::kAuxStreams)) : 0;
+		cudaStream_t stream = lane == 0 ? m->stream : m->aux[lane - 1];
+		const EStepPlan plan = plan_estep(m->K, bucket.n_max, m->beta_elem, m->smem_optin);
+		if(plan.n_cap < bucket.n_max || plan.smem > (size_t) m->smem_optin)
+			return fail(m, TRLDA_ERR_UNSUPPORTED, "A document has too many distinct words for the E-step kernel.");
+		m->stats.total_launches++;
+		launch_estep(plan, a, m->docs, m->b_order.as<int32_t>(), bucket.offset, std::min(bucket.count, end - bucket.offset),
+		             m->beta_elem, stream);
+	}
+	if(fork)
+		for(int i = 0; i < trlda_model::kAuxStreams; ++i) {
+			CUDA_TRY(m, cudaEventRecord(m->join_event[i], m->aux[i]));
+			CUDA_TRY(m, cudaStreamWaitEvent(m->stream, m->join_event[i], 0));
+		}
+	return TRLDA_OK;
+}
+
 // LDA::updateVariablesVI without the scatter: gamma fixed point for every document of the resident minibatch
 int run_estep(trlda_model* m, GammaSource src, const double* host_gamma, int max_iter, double threshold) {
 	if(src == GAMMA_FRESH)
@@ -943,79 +975,31 @@ int run_estep(trlda_model* m, GammaSource src, const double* host_gamma, int max
 	a.sweeps = m->sweeps.as<unsigned long long>();
 	a.work = reinterpret_cast<int*>(m->sweeps.as<unsigned long long>() + 1);
 	m->stats.estep_calls++;
-	const bool warm = src == GAMMA_KEEP;
-	// Mixed mode: the tensor-memory-resident cluster kernel (estep_tmem.cu).  The documents are sorted by length, longest
-	// first: [0, len_gt[0]) do not fit the on-chip tile and go to the streaming kernel; everything else is one launch.
-	if(!m->force_generic && m->docs.B > 0 && m->tmem_mode && tmem_estep_applicable(m->K, m->beta_elem) &&
-	   (m->len_gt[0] == 0 || stream_estep_applicable(m->K, m->docs.n_max, m->beta_elem, m->smem_optin))) {
-		const int64_t B = m->docs.B;
-		const int64_t cut[5] = {m->len_gt[0], m->len_gt[1], m->len_gt[2], m->len_gt[3], B};
-		const int cap[5] = {0, 192, 160, 128, 64};
-		bool ok = true;
-		if(cut[0] > 0) {
+	// The documents are sorted by length, longest first.  In mixed mode the tensor-memory-resident kernel
+	// (estep_tmem.cu) takes every document that fits its on-chip tile, [long_end, B); the longer ones, and in fp64 mode
+	// all of them, go to the streaming kernel (estep_stream.cu), which re-reads the tile from L2 once per inner
+	// iteration, or, for what it does not cover (unaligned K, K beyond its per-lane register tile, documents too long
+	// for its shared memory), to the shared-memory cluster kernel (kernels.cu).
+	const int64_t B = m->docs.B;
+	const int32_t* order = m->b_order.as<int32_t>();
+	const bool tmem = m->tmem_mode && tmem_estep_applicable(m->K, m->beta_elem);
+	const int64_t long_end = tmem ? m->len_gt[0] : B;
+	if(long_end > 0) {
+		if(stream_estep_applicable(m->K, m->docs.n_max, m->beta_elem, m->smem_optin)) {
 			Launch l(m, KK_ESTEP);
-			launch_estep_stream(a, m->docs, m->b_order.as<int32_t>(), 0, cut[0], m->docs.n_max, m->beta_elem, !warm, m->stream);
-		}
-		if(B > cut[0]) {
-			// one persistent launch for all tile shapes: the kernel picks the shape per document
-			Launch l(m, KK_ESTEP);
-			ok = launch_estep_tmem(a, m->docs, m->b_order.as<int32_t>(), cut[0], B - cut[0], cap[1], m->stream) == 0;
-		}
-		if(ok) {
-			m->gamma_valid = true;
-			m->stats.estep_docs = m->docs.B;
-			return check_launch(m, "estep_tmem");
-		}
-		return fail(m, TRLDA_ERR_CUDA, "The tensor-memory E-step kernel could not be launched.");
-	}
-	// fp64 mode (and the shapes the TMEM kernel does not cover): the streaming kernel (estep_stream.cu), which re-reads
-	// the tile from L2 once per inner iteration; the shared-memory cluster kernels remain for what neither covers (K too
-	// large for the per-lane register tile, unaligned K, very long documents)
-	if(!m->force_generic && m->docs.B > 0 && (m->stream_mode == 2 || (m->stream_mode == 1 && warm)) &&
-	   stream_estep_applicable(m->K, m->docs.n_max, m->beta_elem, m->smem_optin)) {
-		{
-			Launch l(m, KK_ESTEP);
-			launch_estep_stream(a, m->docs, m->b_order.as<int32_t>(), 0, m->docs.B, m->docs.n_max, m->beta_elem, !warm, m->stream);
-		}
-		m->gamma_valid = true;
-		m->stats.estep_docs = m->docs.B;
-		return check_launch(m, "estep_stream");
-	}
-	// fork: bucket i runs on stream i % (1 + kAuxStreams) (0 = the main stream); join before anything else continues
-	const bool fork = m->concurrent_buckets && m->buckets.size() > 1 && m->aux[0] != nullptr;
-	Launch span(m, KK_ESTEP);   // one timing span for the whole E-step (the bucket launches overlap)
-	m->stats.total_launches--;  // the span itself is not a kernel; the launches are counted below
-	if(fork) {
-		CUDA_TRY(m, cudaEventRecord(m->fork_event, m->stream));
-		for(int i = 0; i < trlda_model::kAuxStreams; ++i)
-			CUDA_TRY(m, cudaStreamWaitEvent(m->aux[i], m->fork_event, 0));
-	}
-	int index = 0;
-	for(const auto& bucket : m->buckets) {
-		const int lane = fork ? index % (1 + trlda_model::kAuxStreams) : 0;
-		cudaStream_t stream = lane == 0 ? m->stream : m->aux[lane - 1];
-		++index;
-		EStepPlan plan;
-		plan.cluster = 0;
-		if(!m->force_generic)
-			plan = plan_estep_fast(m->K, bucket.n_max, m->beta_elem, m->smem_optin, m->force_cluster);
-		m->stats.total_launches++;
-		if(plan.cluster > 0) {
-			launch_estep_fast(plan, a, m->docs, m->b_order.as<int32_t>(), bucket.offset, bucket.count, m->beta_elem, stream);
+			launch_estep_stream(a, m->docs, order, 0, long_end, m->docs.n_max, m->beta_elem, m->stream);
+			m->stream_ran = true;
 		} else {
-			plan = plan_estep(m->K, bucket.n_max, m->beta_elem, m->smem_optin, m->force_cluster);
-			if(plan.n_cap < bucket.n_max || plan.smem > (size_t) m->smem_optin)
-				return fail(m, TRLDA_ERR_UNSUPPORTED, "A document has too many distinct words for the E-step kernel.");
-			launch_estep(plan, a, m->docs, m->b_order.as<int32_t>(), bucket.offset, bucket.count, m->beta_elem, stream);
+			TRY(run_estep_buckets(m, a, long_end));
 		}
 	}
-	if(fork)
-		for(int i = 0; i < trlda_model::kAuxStreams; ++i) {
-			CUDA_TRY(m, cudaEventRecord(m->join_event[i], m->aux[i]));
-			CUDA_TRY(m, cudaStreamWaitEvent(m->stream, m->join_event[i], 0));
-		}
+	if(long_end < B) {
+		Launch l(m, KK_ESTEP);
+		if(launch_estep_tmem(a, m->docs, order, long_end, B - long_end, tmem_estep_max_len(), m->stream) != 0)
+			return fail(m, TRLDA_ERR_CUDA, "The tensor-memory E-step kernel could not be launched.");
+	}
 	m->gamma_valid = true;
-	m->stats.estep_docs = m->docs.B;
+	m->stats.estep_docs = B;
 	return check_launch(m, "estep");
 }
 
@@ -1848,10 +1832,6 @@ int trlda_create(int kind, int num_words, int num_topics, int64_t num_documents,
 	m->device = device;
 	m->precision = precision;
 	m->psi_gamma_diff.assign(num_topics, 0.0);
-	if(const char* fc = getenv("TRLDA_ESTEP_CLUSTER"))
-		m->force_cluster = atoi(fc);
-	if(const char* fg = getenv("TRLDA_ESTEP_GENERIC"))
-		m->force_generic = atoi(fg) != 0;
 	if(const char* ft = getenv("TRLDA_ESTEP_TICKS"))
 		if(atoi(ft) != 0 && m->ticks.ensure(16 * sizeof(unsigned long long)) == cudaSuccess)
 			cudaMemset(m->ticks.p, 0, 16 * sizeof(unsigned long long));
@@ -1878,13 +1858,8 @@ int trlda_create(int kind, int num_words, int num_topics, int64_t num_documents,
 		return cleanup(TRLDA_ERR_CUDA);
 	}
 	configure_estep(m->smem_optin);
-	configure_estep_fast(m->smem_optin);
-	if(const char* sm = getenv("TRLDA_ESTEP_STREAM"))
-		m->stream_mode = atoi(sm);
 	if(const char* tm = getenv("TRLDA_ESTEP_TMEM"))
 		m->tmem_mode = atoi(tm) != 0;
-	if(const char* cb = getenv("TRLDA_CONCURRENT_BUCKETS"))
-		m->concurrent_buckets = atoi(cb) != 0;
 	cudaEventCreateWithFlags(&m->fork_event, cudaEventDisableTiming);
 	for(int i = 0; i < trlda_model::kAuxStreams; ++i) {
 		cudaStreamCreateWithFlags(&m->aux[i], cudaStreamNonBlocking);
@@ -1923,10 +1898,8 @@ void trlda_destroy(trlda_model* m) {
 	if(m->ticks.p) {
 		unsigned long long t[16];
 		cudaMemcpy(t, m->ticks.p, sizeof(t), cudaMemcpyDeviceToHost);
-		static const char* fast_names[10] = {"stage+gather issue+psi0", "gather wait", "initial pass2+push", "initial exchange+W",
-		                                     "pass1", "gamma/psi/delta", "pass2+push", "exchange+W", "results+doc_stat", "-"};
-		static const char* stream_names[10] = {"document setup", "sweep (stream columns)", "fold partial sums", "cluster exchange",
-		                                       "gamma/psi update + results", "convergence test", "-", "-", "-", "-"};
+		static const char* stream_names[5] = {"document setup", "sweep (stream columns)", "fold partial sums",
+		                                      "gamma/psi update + results", "convergence test"};
 		static const char* resident_names[8] = {"tile -> TMEM + psi0", "pass B (acc) + butterfly", "gamma/psi update", "pass A (phi) + butterflies",
 		                                        "fold in smem + barrier + send", "exchange wait", "weights", "results"};
 		if(m->tmem_mode && m->beta_elem == 4 && tmem_estep_applicable(m->K, m->beta_elem)) {
@@ -1938,12 +1911,11 @@ void trlda_destroy(trlda_model* m) {
 				fprintf(stderr, "[trlda]   busiest team %.0f cycles, mean %.0f over %llu teams (all launches): imbalance %.3f\n", (double) t[8],
 				        (double) t[9] / (double) t[10], t[10], (double) t[8] * (double) t[10] / (double) t[9]);
 		}
-		const bool streamed = m->stream_mode != 0;
-		fprintf(stderr, "[trlda] %s E-step phase timers: %llu documents, %llu %s\n", streamed ? "streaming" : "fast", t[15], t[14],
-		        streamed ? "sweeps" : "inner iterations");
-		for(int i = 0; i < (streamed ? 6 : 10); ++i)
-			fprintf(stderr, "[trlda]   %-26s %10.0f cycles/doc\n", (streamed ? stream_names : fast_names)[i],
-			        t[15] ? (double) t[i] / (double) t[15] : 0.0);
+		if(m->stream_ran) {
+			fprintf(stderr, "[trlda] streaming E-step phase timers: %llu documents, %llu sweeps\n", t[15], t[14]);
+			for(int i = 0; i < 5; ++i)
+				fprintf(stderr, "[trlda]   %-26s %10.0f cycles/doc\n", stream_names[i], t[15] ? (double) t[i] / (double) t[15] : 0.0);
+		}
 		m->ticks.release();
 	}
 	for(void* p : m->peer_opened)
