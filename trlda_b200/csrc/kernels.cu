@@ -254,11 +254,22 @@ EStepPlan plan_estep(int K, int n_max, int elem, int smem_optin) {
 	return best;
 }
 
-template <typename T, bool CLUSTERED>
+// LONG = true: the variant for documents whose per-pair vectors do not fit in shared memory (plan_estep_long).  The word
+// ids and counts are read from the CSR arrays, the weights W_j are kept in their output array a.weight, and the float32
+// weights and the C partial phi-norms of every pair live in `scratch`: for a launch over documents of P pairs in all,
+// C * P doubles of partials followed by P floats, each document at the pairs of the documents before it in the launch.
+// Those are written by one CTA of the cluster and read by others after cluster.sync(), so they are loaded through L2
+// (__ldcg), never from a possibly stale L1 line.  Shared memory holds only the K-sized vectors and n_fit tile columns.
+// The float32 products of the mixed mode are summed in float32 over groups of LONG_GROUP columns and the groups in
+// float64, so that the rounding error does not grow with the length of the document.
+constexpr int LONG_GROUP = 64;
+
+template <typename T, bool CLUSTERED, bool LONG>
 __global__ void __launch_bounds__(ESTEP_THREADS)
-k_estep(EStepArgs a, DeviceDocs docs, const int32_t* __restrict__ order, int64_t doc_offset, int C, int kc, int n_cap, int n_fit) {
+k_estep(EStepArgs a, DeviceDocs docs, const int32_t* __restrict__ order, int64_t doc_offset, int C, int kc, int n_cap, int n_fit,
+        double* __restrict__ scratch, int64_t scratch_pairs) {
 	extern __shared__ __align__(16) unsigned char smem[];
-	const EStepSmem L = estep_smem_layout(C, kc, n_cap, n_fit, (int) sizeof(T));
+	const EStepSmem L = estep_smem_layout(C, kc, LONG ? 0 : n_cap, n_fit, (int) sizeof(T));
 	T* tile = reinterpret_cast<T*>(smem + L.tile);
 	double* W = reinterpret_cast<double*>(smem + L.W);
 	float* W32 = reinterpret_cast<float*>(smem + L.W32);
@@ -268,8 +279,8 @@ k_estep(EStepArgs a, DeviceDocs docs, const int32_t* __restrict__ order, int64_t
 	double* eth = reinterpret_cast<double*>(smem + L.eth);
 	float* eth32 = reinterpret_cast<float*>(smem + L.eth32);
 	double* red = reinterpret_cast<double*>(smem + L.red);
-	int* wid = reinterpret_cast<int*>(smem + L.wid);
-	int* cnt = reinterpret_cast<int*>(smem + L.cnt);
+	const int* wid = reinterpret_cast<int*>(smem + L.wid);
+	const int* cnt = reinterpret_cast<int*>(smem + L.cnt);
 
 	cg::cluster_group cluster = cg::this_cluster();
 	const int rank = CLUSTERED ? (int) cluster.block_rank() : 0;
@@ -288,9 +299,22 @@ k_estep(EStepArgs a, DeviceDocs docs, const int32_t* __restrict__ order, int64_t
 	constexpr bool F32 = sizeof(T) == 4;
 
 	// ---- stage the document, the gamma slice and the tile ----------------------------------------------------
-	for(int j = tid; j < n; j += ESTEP_THREADS) {
-		wid[j] = docs.word_ids[begin + j];
-		cnt[j] = docs.counts[begin + j];
+	if constexpr(LONG) {
+		int64_t off = 0;                                         // pairs of the launch's documents before this one
+		for(int64_t s = doc_offset; s < slot; ++s) {
+			const int64_t e = order ? order[s] : s;
+			off += docs.doc_ptr[e + 1] - docs.doc_ptr[e];
+		}
+		wid = docs.word_ids + begin;
+		cnt = docs.counts + begin;
+		W = a.weight + begin;
+		P = scratch + (int64_t) C * off;
+		W32 = reinterpret_cast<float*>(scratch + (int64_t) C * scratch_pairs) + off;
+	} else {
+		for(int j = tid; j < n; j += ESTEP_THREADS) {
+			reinterpret_cast<int*>(smem + L.wid)[j] = docs.word_ids[begin + j];
+			reinterpret_cast<int*>(smem + L.cnt)[j] = docs.counts[begin + j];
+		}
 	}
 	for(int r = tid; r < kc; r += ESTEP_THREADS) {
 		double g = 0.0, e = 0.0;
@@ -341,9 +365,13 @@ k_estep(EStepArgs a, DeviceDocs docs, const int32_t* __restrict__ order, int64_t
 			}
 			part = warp_sum(part);
 			if(lane == 0) {
-				const int owner = j % C, jl = j / C;
-				double* dst = CLUSTERED ? cluster.map_shared_rank(P, owner) : P;
-				dst[rank * nl_cap + jl] = part;
+				if constexpr(LONG) {
+					__stcg(P + (int64_t) rank * n + j, part);
+				} else {
+					const int owner = j % C, jl = j / C;
+					double* dst = CLUSTERED ? cluster.map_shared_rank(P, owner) : P;
+					dst[rank * nl_cap + jl] = part;
+				}
 			}
 		}
 		if(tid < C) {
@@ -363,16 +391,21 @@ k_estep(EStepArgs a, DeviceDocs docs, const int32_t* __restrict__ order, int64_t
 			const int j = jl * C + rank;
 			double phi = 0.0;
 			for(int src = 0; src < C; ++src)
-				phi += P[src * nl_cap + jl];
+				phi += LONG ? __ldcg(P + (int64_t) src * n + j) : P[src * nl_cap + jl];
 			phi += 1e-100;
 			const double wv = (double) cnt[j] / phi;
-			for(int dst = 0; dst < C; ++dst) {
-				double* Wd = CLUSTERED ? cluster.map_shared_rank(W, dst) : W;
-				float* Wf = CLUSTERED ? cluster.map_shared_rank(W32, dst) : W32;
-				Wd[j] = wv;
-				// float32 products: a weight that overflowed float32 (phi underflowed, lda.cpp:183's 1e-100 floor) would turn
-				// 0 * inf into NaN where the fp64 reference gets 0
-				Wf[j] = (float) fmin(wv, 1e30);
+			if constexpr(LONG) {                                     // one copy, read by every CTA through L2
+				__stcg(W + j, wv);
+				__stcg(W32 + j, (float) fmin(wv, 1e30));
+			} else {
+				for(int dst = 0; dst < C; ++dst) {
+					double* Wd = CLUSTERED ? cluster.map_shared_rank(W, dst) : W;
+					float* Wf = CLUSTERED ? cluster.map_shared_rank(W32, dst) : W32;
+					Wd[j] = wv;
+					// float32 products: a weight that overflowed float32 (phi underflowed, lda.cpp:183's 1e-100 floor) would
+					// turn 0 * inf into NaN where the fp64 reference gets 0
+					Wf[j] = (float) fmin(wv, 1e30);
+				}
 			}
 		}
 		if(CLUSTERED) cluster.sync(); else __syncthreads();
@@ -384,7 +417,31 @@ k_estep(EStepArgs a, DeviceDocs docs, const int32_t* __restrict__ order, int64_t
 	const int S = ESTEP_THREADS / R;
 	const int r0 = tid % R, sp = tid / R;
 	auto pass1_partial = [&](int row) -> double {
-		if(F32) {
+		if constexpr(LONG && F32) {
+			double sum = 0.0;
+			for(int jg = sp; jg < n_in; jg += LONG_GROUP * S) {
+				float acc = 0.f;
+				for(int j = jg; j < min(n_in, jg + LONG_GROUP * S); j += S)
+					acc = fmaf(__ldcg(W32 + j), (float) tile[(size_t) j * kc + row], acc);
+				sum += (double) acc;
+			}
+			if(row < kn)
+				for(int jg = n_in + sp; jg < n; jg += LONG_GROUP * S) {
+					float acc = 0.f;
+					for(int j = jg; j < min(n, jg + LONG_GROUP * S); j += S)
+						acc = fmaf(__ldcg(W32 + j), (float) beta[(int64_t) wid[j] * K + k0 + row], acc);
+					sum += (double) acc;
+				}
+			return sum;
+		} else if constexpr(LONG) {
+			double acc = 0.0;
+			for(int j = sp; j < n_in; j += S)
+				acc = fma(__ldcg(W + j), (double) tile[(size_t) j * kc + row], acc);
+			if(row < kn)
+				for(int j = n_in + sp; j < n; j += S)
+					acc = fma(__ldcg(W + j), (double) beta[(int64_t) wid[j] * K + k0 + row], acc);
+			return acc;
+		} else if(F32) {
 			float acc = 0.f;
 			for(int j = sp; j < n_in; j += S)
 				acc = fmaf(W32[j], (float) tile[(size_t) j * kc + row], acc);
@@ -448,8 +505,9 @@ k_estep(EStepArgs a, DeviceDocs docs, const int32_t* __restrict__ order, int64_t
 		if(a.etheta32)
 			a.etheta32[d * K + k0 + r] = eth32[r];
 	}
-	for(int j = tid * C + rank; j < n; j += ESTEP_THREADS * C)
-		a.weight[begin + j] = W[j];
+	if(!LONG)                                                    // LONG: the weights are already in place
+		for(int j = tid * C + rank; j < n; j += ESTEP_THREADS * C)
+			a.weight[begin + j] = W[j];
 	if(a.doc_stat) {
 		for(int rb = 0; rb < kc; rb += R) {
 			const int row = rb + r0;
@@ -476,15 +534,19 @@ static int g_estep_smem_optin = 0;
 
 void configure_estep(int smem_optin) {
 	g_estep_smem_optin = smem_optin;
-	cudaFuncSetAttribute(k_estep<double, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_optin);
-	cudaFuncSetAttribute(k_estep<double, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_optin);
-	cudaFuncSetAttribute(k_estep<float, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_optin);
-	cudaFuncSetAttribute(k_estep<float, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_optin);
+	cudaFuncSetAttribute(k_estep<double, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_optin);
+	cudaFuncSetAttribute(k_estep<double, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_optin);
+	cudaFuncSetAttribute(k_estep<float, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_optin);
+	cudaFuncSetAttribute(k_estep<float, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_optin);
+	cudaFuncSetAttribute(k_estep<double, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_optin);
+	cudaFuncSetAttribute(k_estep<double, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_optin);
+	cudaFuncSetAttribute(k_estep<float, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_optin);
+	cudaFuncSetAttribute(k_estep<float, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_optin);
 }
 
-template <typename T, bool CLUSTERED>
+template <typename T, bool CLUSTERED, bool LONG>
 static void launch_estep_t(const EStepPlan& plan, const EStepArgs& args, const DeviceDocs& docs, const int32_t* order,
-                           int64_t offset, int64_t count, cudaStream_t s) {
+                           int64_t offset, int64_t count, double* scratch, int64_t scratch_pairs, cudaStream_t s) {
 	cudaLaunchConfig_t cfg = {};
 	cfg.gridDim = dim3((unsigned) (count * plan.cluster));
 	cfg.blockDim = dim3(ESTEP_THREADS);
@@ -497,7 +559,8 @@ static void launch_estep_t(const EStepPlan& plan, const EStepArgs& args, const D
 	attr[0].val.clusterDim.z = 1;
 	cfg.attrs = attr;
 	cfg.numAttrs = CLUSTERED ? 1 : 0;
-	cudaLaunchKernelEx(&cfg, k_estep<T, CLUSTERED>, args, docs, order, offset, plan.cluster, plan.kc, plan.n_cap, plan.n_fit);
+	cudaLaunchKernelEx(&cfg, k_estep<T, CLUSTERED, LONG>, args, docs, order, offset, plan.cluster, plan.kc, plan.n_cap, plan.n_fit,
+	                   scratch, scratch_pairs);
 }
 
 void launch_estep(const EStepPlan& plan, const EStepArgs& args, const DeviceDocs& docs, const int32_t* order,
@@ -505,11 +568,46 @@ void launch_estep(const EStepPlan& plan, const EStepArgs& args, const DeviceDocs
 	if(count == 0)
 		return;
 	if(elem_size == 8) {
-		if(plan.cluster > 1) launch_estep_t<double, true>(plan, args, docs, order, offset, count, s);
-		else launch_estep_t<double, false>(plan, args, docs, order, offset, count, s);
+		if(plan.cluster > 1) launch_estep_t<double, true, false>(plan, args, docs, order, offset, count, nullptr, 0, s);
+		else launch_estep_t<double, false, false>(plan, args, docs, order, offset, count, nullptr, 0, s);
 	} else {
-		if(plan.cluster > 1) launch_estep_t<float, true>(plan, args, docs, order, offset, count, s);
-		else launch_estep_t<float, false>(plan, args, docs, order, offset, count, s);
+		if(plan.cluster > 1) launch_estep_t<float, true, false>(plan, args, docs, order, offset, count, nullptr, 0, s);
+		else launch_estep_t<float, false, false>(plan, args, docs, order, offset, count, nullptr, 0, s);
+	}
+}
+
+EStepPlan plan_estep_long(int K, int n_max, int elem, int smem_optin) {
+	int C = 8;                                                     // the largest cluster that leaves no CTA without rows
+	while(C > 1 && (C - 1) * round_up(ceil_div(K, C), 32) >= K)
+		C /= 2;
+	const int kc = round_up(ceil_div(K, C), 32);
+	const size_t budget = (size_t) smem_optin - 1024;
+	const EStepSmem L0 = estep_smem_layout(C, kc, 0, 0, elem);
+	int n_fit = L0.total >= budget ? 0 : (int) ((budget - L0.total) / ((size_t) kc * elem));
+	n_fit = std::min(n_fit, n_max) / 4 * 4;
+	EStepPlan plan;
+	plan.cluster = C;
+	plan.kc = kc;
+	plan.n_cap = 0;
+	plan.n_fit = n_fit;
+	plan.smem = estep_smem_layout(C, kc, 0, n_fit, elem).total;
+	return plan;
+}
+
+size_t estep_long_scratch_bytes(const EStepPlan& plan, int64_t pairs) {
+	return (size_t) pairs * ((size_t) plan.cluster * sizeof(double) + sizeof(float));
+}
+
+void launch_estep_long(const EStepPlan& plan, const EStepArgs& args, const DeviceDocs& docs, const int32_t* order,
+                       int64_t offset, int64_t count, double* scratch, int64_t scratch_pairs, int elem_size, cudaStream_t s) {
+	if(count == 0)
+		return;
+	if(elem_size == 8) {
+		if(plan.cluster > 1) launch_estep_t<double, true, true>(plan, args, docs, order, offset, count, scratch, scratch_pairs, s);
+		else launch_estep_t<double, false, true>(plan, args, docs, order, offset, count, scratch, scratch_pairs, s);
+	} else {
+		if(plan.cluster > 1) launch_estep_t<float, true, true>(plan, args, docs, order, offset, count, scratch, scratch_pairs, s);
+		else launch_estep_t<float, false, true>(plan, args, docs, order, offset, count, scratch, scratch_pairs, s);
 	}
 }
 

@@ -92,6 +92,14 @@ void launch_estep(const EStepPlan& plan, const EStepArgs& args, const DeviceDocs
                   int64_t offset, int64_t count, int elem_size, cudaStream_t s);
 void configure_estep(int smem_optin);
 
+// the same kernel for documents too long for plan_estep's shared memory: the per-pair vectors live in global memory (the
+// CSR arrays, args.weight and `scratch`), so the shared memory of a launch does not depend on the document length.
+// scratch holds estep_long_scratch_bytes(plan, P) bytes for the P pairs of the documents order[offset .. offset+count).
+EStepPlan plan_estep_long(int K, int n_max, int elem_size, int smem_optin);
+size_t estep_long_scratch_bytes(const EStepPlan& plan, int64_t pairs);
+void launch_estep_long(const EStepPlan& plan, const EStepArgs& args, const DeviceDocs& docs, const int32_t* order,
+                       int64_t offset, int64_t count, double* scratch, int64_t scratch_pairs, int elem_size, cudaStream_t s);
+
 // streaming kernel (estep_stream.cu): one CTA per document, columns streamed through per-warp cp.async rings, one sweep
 // per inner iteration
 bool stream_estep_applicable(int K, int n_max, int elem_size, int smem_optin);

@@ -212,6 +212,7 @@ struct trlda_model {
 	// shared-memory tile is sized for the bucket's longest document
 	struct Bucket { int64_t offset, count; int n_max; };
 	std::vector<Bucket> buckets;
+	std::vector<int> sorted_len;    // length of every document in that order
 	// documents longer than 192 / 160 / 128 / 64 pairs (prefix lengths of the length-sorted order): the cuts between
 	// the tile shapes of the tensor-memory E-step kernel
 	int64_t len_gt[4] = {0, 0, 0, 0};
@@ -237,6 +238,7 @@ struct trlda_model {
 		DeviceDocs docs;
 		DevBuf b_doc_ptr, b_word_ids, b_counts, b_word_ptr, b_tok_doc, b_tok_src, b_order;
 		std::vector<Bucket> buckets;
+		std::vector<int> sorted_len;
 		int64_t len_gt[4] = {0, 0, 0, 0};
 		int64_t docs_total_count = 0, global_B = 0;
 	};
@@ -251,6 +253,11 @@ struct trlda_model {
 	static const int kAuxStreams = 3;
 	cudaStream_t aux[kAuxStreams] = {nullptr, nullptr, nullptr};
 	cudaEvent_t fork_event = nullptr, join_event[kAuxStreams] = {nullptr, nullptr, nullptr};
+	// documents too long for the shared-memory plan of k_estep run on their own stream, beside the other E-step kernels,
+	// with their per-pair vectors in long_scratch
+	cudaStream_t long_stream = nullptr;
+	cudaEvent_t long_join = nullptr;
+	DevBuf long_scratch;
 	bool tmem_mode = true;       // TRLDA_ESTEP_TMEM=0: never use the tensor-memory-resident kernel (mixed mode)
 	bool stream_ran = false;     // the streaming E-step kernel has run (its phase timers are printed by trlda_destroy)
 	DevBuf sweeps;   // device counter behind trlda_stats.estep_sweeps
@@ -473,6 +480,7 @@ void swap_with_slot(trlda_model* m, trlda_model::DocSlot& slot) {
 	std::swap(m->b_tok_src, slot.b_tok_src);
 	std::swap(m->b_order, slot.b_order);
 	std::swap(m->buckets, slot.buckets);
+	std::swap(m->sorted_len, slot.sorted_len);
 	std::swap(m->gdocs, slot.gdocs);
 	std::swap(m->len_gt, slot.len_gt);
 	std::swap(m->docs_total_count, slot.docs_total_count);
@@ -480,6 +488,30 @@ void swap_with_slot(trlda_model* m, trlda_model::DocSlot& slot) {
 }
 
 int build_global_docs(trlda_model* m, const int64_t* s_ptr, int64_t B, int64_t N);
+
+// cuts the length-sorted documents [begin, B) into length buckets, each one launch of k_estep whose shared-memory tile
+// is sized for the bucket's longest document
+void form_buckets(const std::vector<int>& len, int64_t begin, std::vector<trlda_model::Bucket>& buckets) {
+	auto cap_of = [](int n) {
+		int cap = 32;
+		while(cap < n)
+			cap += cap < 256 ? 32 : (cap < 512 ? 64 : cap / 4);
+		return cap;
+	};
+	const int64_t B = (int64_t) len.size();
+	const int64_t min_bucket = 128;
+	buckets.clear();
+	for(int64_t i = begin; i < B;) {
+		const int cap = cap_of(len[i]);
+		int64_t j = i;
+		while(j < B && (cap_of(len[j]) == cap || j - i < min_bucket))
+			++j;
+		if(B - j < min_bucket)
+			j = B;
+		buckets.push_back({i, j - i, len[i]});
+		i = j;
+	}
+}
 
 // ---- minibatch upload: CSR + word-sorted token list ---------------------------------------------------------------
 int upload_docs(trlda_model* m, const trlda_docs* docs) {
@@ -592,6 +624,7 @@ int upload_docs(trlda_model* m, const trlda_docs* docs) {
 
 	// length buckets for the E-step: counting sort by length, longest first
 	m->buckets.clear();
+	m->sorted_len.resize(B);
 	if(B) {
 		std::vector<int32_t> start(n_max + 2, 0);
 		for(int64_t d = 0; d < B; ++d)
@@ -600,24 +633,11 @@ int upload_docs(trlda_model* m, const trlda_docs* docs) {
 			start[i + 1] += start[i];
 		for(int64_t d = 0; d < B; ++d)
 			s_order[start[n_max - (int) (s_ptr[d + 1] - s_ptr[d])]++] = (int32_t) d;
-		auto cap_of = [](int n) {
-			int cap = 32;
-			while(cap < n)
-				cap += cap < 256 ? 32 : (cap < 512 ? 64 : cap / 4);
-			return cap;
-		};
-		auto len_of = [&](int64_t i) { const int32_t d = s_order[i]; return (int) (s_ptr[d + 1] - s_ptr[d]); };
-		const int64_t min_bucket = 128;
-		for(int64_t i = 0; i < B;) {
-			const int cap = cap_of(len_of(i));
-			int64_t j = i;
-			while(j < B && (cap_of(len_of(j)) == cap || j - i < min_bucket))
-				++j;
-			if(B - j < min_bucket)
-				j = B;
-			m->buckets.push_back({i, j - i, len_of(i)});
-			i = j;
+		for(int64_t i = 0; i < B; ++i) {
+			const int32_t d = s_order[i];
+			m->sorted_len[i] = (int) (s_ptr[d + 1] - s_ptr[d]);
 		}
+		form_buckets(m->sorted_len, 0, m->buckets);
 	}
 
 	const double t_host = ms_since(t_begin);
@@ -915,29 +935,25 @@ int fresh_gamma(trlda_model* m) {
 	return check_launch(m, "gamma_rng");
 }
 
-// the shared-memory cluster kernel (kernels.cu) on the documents order[0, end): one launch per length bucket, its tile
-// sized for the bucket's longest document.  Bucket i runs on stream i % (1 + kAuxStreams) (0 = the main stream), so
-// that CTAs of buckets with different shared-memory footprints can share an SM and the buckets' tails overlap; the
-// main stream waits for all of them.
-int run_estep_buckets(trlda_model* m, const EStepArgs& a, int64_t end) {
+// the shared-memory cluster kernel (kernels.cu) on the documents of `buckets` before `end`: one launch per length
+// bucket, its tile sized for the bucket's longest document.  Bucket i runs on stream i % (1 + kAuxStreams) (0 = the main
+// stream), so that CTAs of buckets with different shared-memory footprints can share an SM and the buckets' tails
+// overlap; the main stream waits for all of them.
+int launch_buckets(trlda_model* m, const EStepArgs& a, const std::vector<trlda_model::Bucket>& buckets, int64_t end) {
 	size_t nb = 0;
-	while(nb < m->buckets.size() && m->buckets[nb].offset < end)
+	while(nb < buckets.size() && buckets[nb].offset < end)
 		++nb;
 	const bool fork = nb > 1 && m->aux[0] != nullptr;
-	Launch span(m, KK_ESTEP);   // one timing span for the whole E-step (the bucket launches overlap)
-	m->stats.total_launches--;  // the span itself is not a kernel; the launches are counted below
 	if(fork) {
 		CUDA_TRY(m, cudaEventRecord(m->fork_event, m->stream));
 		for(int i = 0; i < trlda_model::kAuxStreams; ++i)
 			CUDA_TRY(m, cudaStreamWaitEvent(m->aux[i], m->fork_event, 0));
 	}
 	for(size_t i = 0; i < nb; ++i) {
-		const trlda_model::Bucket& bucket = m->buckets[i];
+		const trlda_model::Bucket& bucket = buckets[i];
 		const int lane = fork ? (int) (i % (1 + trlda_model::kAuxStreams)) : 0;
 		cudaStream_t stream = lane == 0 ? m->stream : m->aux[lane - 1];
 		const EStepPlan plan = plan_estep(m->K, bucket.n_max, m->beta_elem, m->smem_optin);
-		if(plan.n_cap < bucket.n_max || plan.smem > (size_t) m->smem_optin)
-			return fail(m, TRLDA_ERR_UNSUPPORTED, "A document has too many distinct words for the E-step kernel.");
 		m->stats.total_launches++;
 		launch_estep(plan, a, m->docs, m->b_order.as<int32_t>(), bucket.offset, std::min(bucket.count, end - bucket.offset),
 		             m->beta_elem, stream);
@@ -947,6 +963,61 @@ int run_estep_buckets(trlda_model* m, const EStepArgs& a, int64_t end) {
 			CUDA_TRY(m, cudaEventRecord(m->join_event[i], m->aux[i]));
 			CUDA_TRY(m, cudaStreamWaitEvent(m->stream, m->join_event[i], 0));
 		}
+	return TRLDA_OK;
+}
+
+int run_estep_buckets(trlda_model* m, const EStepArgs& a, int64_t end) {
+	Launch span(m, KK_ESTEP);   // one timing span for the whole E-step (the bucket launches overlap)
+	m->stats.total_launches--;  // the span itself is not a kernel; the launches are counted by launch_buckets
+	return launch_buckets(m, a, m->buckets, end);
+}
+
+// whether plan_estep keeps all per-pair vectors of a document of n pairs in shared memory
+bool estep_fits(const trlda_model* m, int n) {
+	const EStepPlan plan = plan_estep(m->K, n, m->beta_elem, m->smem_optin);
+	return plan.n_cap >= n && plan.smem <= (size_t) m->smem_optin;
+}
+
+// E-step of a minibatch whose longest documents, order[0, n_over), fit neither the shared memory of k_estep nor that of
+// the streaming kernel.  They go to the global-memory variant of k_estep on the long-document stream, beside the kernels
+// of the other documents.  Those are routed as if the long documents were absent: [n_over, long_end) to the streaming
+// kernel when it takes the longest of them, else to k_estep over buckets formed without the long documents, and
+// [long_end, B) to the tensor-memory kernel.  One timing span covers the whole E-step.
+int run_estep_with_long(trlda_model* m, const EStepArgs& a, int64_t n_over, int64_t long_end) {
+	const int64_t B = m->docs.B;
+	const int32_t* order = m->b_order.as<int32_t>();
+	Launch span(m, KK_ESTEP);
+	m->stats.total_launches--;  // the span itself is not a kernel
+	int64_t pairs = 0;
+	for(int64_t i = 0; i < n_over; ++i)
+		pairs += m->sorted_len[i];
+	// no length limit is left to check: the plan's shared memory is the K-sized vectors (12 KB at K = 4096) plus as many
+	// tile columns as fit beside them, and the scratch grows with the documents
+	const EStepPlan plan = plan_estep_long(m->K, m->sorted_len[0], m->beta_elem, m->smem_optin);
+	CUDA_TRY(m, m->long_scratch.ensure(estep_long_scratch_bytes(plan, pairs)));
+	CUDA_TRY(m, cudaEventRecord(m->fork_event, m->stream));
+	CUDA_TRY(m, cudaStreamWaitEvent(m->long_stream, m->fork_event, 0));
+	m->stats.total_launches++;
+	launch_estep_long(plan, a, m->docs, order, 0, n_over, m->long_scratch.as<double>(), pairs, m->beta_elem, m->long_stream);
+	CUDA_TRY(m, cudaEventRecord(m->long_join, m->long_stream));
+	if(n_over < long_end) {
+		const int n_rest = m->sorted_len[n_over];
+		if(stream_estep_applicable(m->K, n_rest, m->beta_elem, m->smem_optin)) {
+			m->stats.total_launches++;
+			launch_estep_stream(a, m->docs, order, n_over, long_end - n_over, n_rest, m->beta_elem, m->stream);
+			m->stream_ran = true;
+		} else {
+			std::vector<trlda_model::Bucket> buckets;
+			form_buckets(m->sorted_len, n_over, buckets);
+			TRY(launch_buckets(m, a, buckets, long_end));
+		}
+	}
+	if(long_end < B) {
+		m->stats.total_launches++;
+		if(launch_estep_tmem(a, m->docs, order, long_end, B - long_end, tmem_estep_max_len(), m->stream) != 0)
+			return fail(m, TRLDA_ERR_CUDA, "The tensor-memory E-step kernel could not be launched.");
+	}
+	CUDA_TRY(m, cudaStreamWaitEvent(m->stream, m->long_join, 0));
 	return TRLDA_OK;
 }
 
@@ -984,7 +1055,14 @@ int run_estep(trlda_model* m, GammaSource src, const double* host_gamma, int max
 	const int32_t* order = m->b_order.as<int32_t>();
 	const bool tmem = m->tmem_mode && tmem_estep_applicable(m->K, m->beta_elem);
 	const int64_t long_end = tmem ? m->len_gt[0] : B;
-	if(long_end > 0) {
+	// documents too long for both the streaming kernel and the shared memory of k_estep: order[0, n_over)
+	int64_t n_over = 0;
+	if(long_end > 0 && !stream_estep_applicable(m->K, m->docs.n_max, m->beta_elem, m->smem_optin))
+		while(n_over < long_end && !estep_fits(m, m->sorted_len[n_over]))
+			++n_over;
+	if(n_over > 0) {
+		TRY(run_estep_with_long(m, a, n_over, long_end));
+	} else if(long_end > 0) {
 		if(stream_estep_applicable(m->K, m->docs.n_max, m->beta_elem, m->smem_optin)) {
 			Launch l(m, KK_ESTEP);
 			launch_estep_stream(a, m->docs, order, 0, long_end, m->docs.n_max, m->beta_elem, m->stream);
@@ -993,7 +1071,7 @@ int run_estep(trlda_model* m, GammaSource src, const double* host_gamma, int max
 			TRY(run_estep_buckets(m, a, long_end));
 		}
 	}
-	if(long_end < B) {
+	if(long_end < B && n_over == 0) {
 		Launch l(m, KK_ESTEP);
 		if(launch_estep_tmem(a, m->docs, order, long_end, B - long_end, tmem_estep_max_len(), m->stream) != 0)
 			return fail(m, TRLDA_ERR_CUDA, "The tensor-memory E-step kernel could not be launched.");
@@ -1865,6 +1943,8 @@ int trlda_create(int kind, int num_words, int num_topics, int64_t num_documents,
 		cudaStreamCreateWithFlags(&m->aux[i], cudaStreamNonBlocking);
 		cudaEventCreateWithFlags(&m->join_event[i], cudaEventDisableTiming);
 	}
+	cudaStreamCreateWithFlags(&m->long_stream, cudaStreamNonBlocking);
+	cudaEventCreateWithFlags(&m->long_join, cudaEventDisableTiming);
 
 	int status = TRLDA_OK;
 	auto init = [&]() -> int {
@@ -1929,7 +2009,7 @@ void trlda_destroy(trlda_model* m) {
 	                  &m->psi_rows, &m->d_alpha, &m->partials, &m->vpartials, &m->scalars, &m->b_doc_ptr, &m->b_word_ids,
 	                  &m->b_counts, &m->b_word_ptr, &m->b_tok_doc, &m->b_tok_src, &m->b_order, &m->wordcount, &m->gamma, &m->etheta,
 	                  &m->etheta32, &m->weight, &m->doc_stat, &m->iterations, &m->gibbs_occ, &m->gibbs_topics, &m->sweeps,
-	                  &m->sample_cdf, &m->sample_tokens, &m->sample_counts, &m->sample_lengths};
+	                  &m->sample_cdf, &m->sample_tokens, &m->sample_counts, &m->sample_lengths, &m->long_scratch};
 	for(DevBuf* b : bufs)
 		b->release();
 	{
@@ -1956,6 +2036,10 @@ void trlda_destroy(trlda_model* m) {
 	}
 	if(m->fork_event)
 		cudaEventDestroy(m->fork_event);
+	if(m->long_stream)
+		cudaStreamDestroy(m->long_stream);
+	if(m->long_join)
+		cudaEventDestroy(m->long_join);
 	if(m->stream)
 		cudaStreamDestroy(m->stream);
 	delete m;
