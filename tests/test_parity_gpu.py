@@ -450,6 +450,32 @@ def test_parked_minibatch_survives_other_calls(capi):
 	assert np.array_equal(model.lambdas, host.lambdas)
 
 
+def test_parked_minibatches_survive_slot_growth_and_teardown(capi):
+	"""uploads into slots 2, 0 and 5 grow the slot vector and move the minibatches parked before; selecting each slot
+	then trains on its own documents.  Closing the model with its slots parked frees every buffer once: a second free
+	would leave a CUDA error behind that fails the next call on this thread"""
+	from trlda_b200.synth import gamma_matrix, make_corpus
+	K, V = 64, 500
+	batches = {slot: capi.CSR(*make_corpus(B, V, K, .1, .2, seed=10 + slot)) for slot, B in ((2, 50), (0, 40), (5, 30))}
+	g0 = {slot: gamma_matrix(K, docs.num_docs, 20 + slot) for slot, docs in batches.items()}
+	lam0 = gamma_matrix(K, V, 4)
+	host = capi.Model('online', V, K, 10000, .1, .2)
+	host.lambdas = lam0
+	model = capi.Model('online', V, K, 10000, .1, .2)
+	model.lambdas = lam0
+	for slot in (2, 0, 5):
+		model.upload_docs_slot(batches[slot], slot)
+	for slot in (0, 2, 5):
+		host.update_parameters(batches[slot], gamma0=g0[slot], max_iter_inference=20)
+		model.select_docs(slot)
+		model.update_parameters_resident(gamma0=g0[slot], max_iter_inference=20)
+		assert np.array_equal(model.lambdas, host.lambdas)
+	model.close()
+	again = capi.Model('online', V, K, 10000, .1, .2)
+	again.update_parameters(batches[0], max_iter_inference=20)
+	assert np.all(np.isfinite(again.lambdas))
+
+
 def test_csr_input_is_validated(capi):
 	model = capi.Model('online', 20, 4, 10)
 	with pytest.raises(RuntimeError, match='Word counts should not be negative.'):

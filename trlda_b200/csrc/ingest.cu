@@ -19,17 +19,35 @@
 #include <mutex>
 #include <string>
 #include <thread>
+#include <utility>
 #include <vector>
 
 namespace {
 
 thread_local std::string g_reader_error;
 
-// one batch in host memory: page-locked where a CUDA device exists, plain otherwise (CPU-only tooling, tests)
+// one batch in host memory: page-locked where a CUDA device exists, plain otherwise (CPU-only tooling, tests); freed by
+// its owner and move-only, so that two owners of one allocation cannot exist
 struct HostArray {
 	void* p = nullptr;
 	size_t cap = 0;
 	bool pinned = false;
+
+	HostArray() = default;
+	HostArray(const HostArray&) = delete;
+	HostArray& operator=(const HostArray&) = delete;
+	HostArray(HostArray&& o) noexcept { *this = std::move(o); }
+	HostArray& operator=(HostArray&& o) noexcept {
+		if(this != &o) {
+			release();
+			p = std::exchange(o.p, nullptr);
+			cap = std::exchange(o.cap, 0);
+			pinned = o.pinned;
+		}
+		return *this;
+	}
+	~HostArray() { release(); }
+
 	bool ensure(size_t bytes, bool want_pinned) {
 		if(bytes <= cap)
 			return true;
@@ -280,11 +298,6 @@ void trlda_reader_close(trlda_reader* r) {
 	r->cv.notify_all();
 	if(r->worker.joinable())
 		r->worker.join();
-	for(Batch& b : r->ring) {
-		b.ptr.release();
-		b.ids.release();
-		b.cts.release();
-	}
 	if(r->data)
 		munmap(const_cast<char*>(r->data), r->size);
 	if(r->fd >= 0)

@@ -20,6 +20,7 @@
 #include <mutex>
 #include <string>
 #include <thread>
+#include <utility>
 #include <vector>
 
 using namespace trlda;
@@ -44,56 +45,53 @@ uint64_t current_seed() {
 	return g_seed;
 }
 
-struct DevBuf {
+// device (cudaMalloc) or page-locked host (cudaHostAlloc) memory that grows on demand and is freed by its owner;
+// move-only, so that two owners of one allocation cannot exist
+template <bool Pinned> struct Buf {
 	void* p = nullptr;
 	size_t cap = 0;
-	cudaError_t ensure(size_t bytes) {
-		if(bytes <= cap)
-			return cudaSuccess;
-		if(p)
-			cudaFree(p);
-		p = nullptr;
-		cap = 0;
-		// grow geometrically for the per-minibatch buffers, exact for the big K x V ones
-		size_t want = bytes < (64u << 20) ? bytes + bytes / 4 + 256 : bytes;
-		cudaError_t e = cudaMalloc(&p, want);
-		if(e == cudaSuccess)
-			cap = want;
-		return e;
-	}
-	void release() {
-		if(p)
-			cudaFree(p);
-		p = nullptr;
-		cap = 0;
-	}
-	template <typename T> T* as() const { return static_cast<T*>(p); }
-};
 
-struct PinnedBuf {
-	void* p = nullptr;
-	size_t cap = 0;
+	Buf() = default;
+	Buf(const Buf&) = delete;
+	Buf& operator=(const Buf&) = delete;
+	Buf(Buf&& o) noexcept { *this = std::move(o); }
+	Buf& operator=(Buf&& o) noexcept {
+		if(this != &o) {
+			release();
+			p = std::exchange(o.p, nullptr);
+			cap = std::exchange(o.cap, 0);
+		}
+		return *this;
+	}
+	~Buf() { release(); }
+
 	cudaError_t ensure(size_t bytes) {
 		if(bytes <= cap)
 			return cudaSuccess;
-		if(p)
-			cudaFreeHost(p);
-		p = nullptr;
-		cap = 0;
-		size_t want = bytes + bytes / 4 + 256;
-		cudaError_t e = cudaHostAlloc(&p, want, cudaHostAllocDefault);
+		release();
+		// grow geometrically; device buffers from 64 MB up (the big K x V ones) are allocated exactly
+		const size_t want = Pinned || bytes < (64u << 20) ? bytes + bytes / 4 + 256 : bytes;
+		const cudaError_t e = Pinned ? cudaHostAlloc(&p, want, cudaHostAllocDefault) : cudaMalloc(&p, want);
 		if(e == cudaSuccess)
 			cap = want;
+		else
+			p = nullptr;
 		return e;
 	}
 	void release() {
-		if(p)
-			cudaFreeHost(p);
+		if(p) {
+			if(Pinned)
+				cudaFreeHost(p);
+			else
+				cudaFree(p);
+		}
 		p = nullptr;
 		cap = 0;
 	}
 	template <typename T> T* as() const { return static_cast<T*>(p); }
 };
+using DevBuf = Buf<false>;
+using PinnedBuf = Buf<true>;
 
 // ---- NCCL through dlopen: no link-time dependency, only needed once trlda_comm_init is called -------------------
 struct NcclApi {
@@ -205,18 +203,9 @@ struct trlda_model {
 	DevBuf sstats;
 	DevBuf rows, rows_prev, rows_stat, psi_rows, d_alpha, partials, vpartials, scalars;
 
-	// minibatch
-	DeviceDocs docs;
-	DevBuf b_doc_ptr, b_word_ids, b_counts, b_word_ptr, b_tok_doc, b_tok_src, b_order, wordcount;
 	// documents sorted by length (descending) and cut into buckets; each bucket is one E-step launch whose
 	// shared-memory tile is sized for the bucket's longest document
 	struct Bucket { int64_t offset, count; int n_max; };
-	std::vector<Bucket> buckets;
-	std::vector<int> sorted_len;    // length of every document in that order
-	// documents longer than 192 / 160 / 128 / 64 pairs (prefix lengths of the length-sorted order): the cuts between
-	// the tile shapes of the tensor-memory E-step kernel
-	int64_t len_gt[4] = {0, 0, 0, 0};
-	// parked resident minibatches (trlda_upload_docs_slot / trlda_select_docs): the live buffers are swapped with a slot
 	// Multi-GPU "gather" exchange (default for the mixed mode): every rank holds the token list of the WHOLE minibatch,
 	// sorted by word and restricted to the words it owns; per trust-region iteration the ranks all-gather etheta and the
 	// token weights (43 MB at cfg-3), every rank scatters + blends + prepares beta for ITS word range with the single-GPU
@@ -229,21 +218,28 @@ struct trlda_model {
 		DevBuf len, ids, word_ptr, tok_doc, tok_src, etheta32, weight, scratch;
 		DeviceDocs view;                                               // word_ptr / tok_doc / tok_src of the global batch
 	};
-	GlobalDocs gdocs;
-	bool use_gather = true;                    // TRLDA_MULTI_GPU=gather (default) | peer | allreduce
-	PinnedBuf gstage;
-	struct DocSlot {
-		bool used = false;
-		GlobalDocs gdocs;
+	// one uploaded minibatch: the resident one is `mb`, parked ones (trlda_upload_docs_slot / trlda_select_docs) sit in
+	// `slots` and are exchanged with it whole
+	struct Minibatch {
 		DeviceDocs docs;
 		DevBuf b_doc_ptr, b_word_ids, b_counts, b_word_ptr, b_tok_doc, b_tok_src, b_order;
 		std::vector<Bucket> buckets;
-		std::vector<int> sorted_len;
+		std::vector<int> sorted_len;    // length of every document in the length-sorted order
+		// documents longer than 192 / 160 / 128 / 64 pairs (prefix lengths of the length-sorted order): the cuts between
+		// the tile shapes of the tensor-memory E-step kernel
 		int64_t len_gt[4] = {0, 0, 0, 0};
-		int64_t docs_total_count = 0, global_B = 0;
+		GlobalDocs gdocs;
+		int64_t docs_total_count = 0;    // sum of all counts in the (global) minibatch
+		int64_t global_B = 0;            // documents over all ranks
 	};
-	std::vector<DocSlot> slots;
+	Minibatch mb;
+	struct Slot {
+		bool used = false;
+		Minibatch mb;
+	};
+	std::vector<Slot> slots;
 	int live_slot = -1;
+	bool use_gather = true;                    // TRLDA_MULTI_GPU=gather (default) | peer | allreduce
 	// the word-sorted token list of the resident minibatch is built lazily (ensure_csc)
 	bool csc_pending = false;
 	int csc_threads = 1;
@@ -267,12 +263,10 @@ struct trlda_model {
 	std::vector<int32_t> sample_ids, sample_cts;
 	DevBuf ticks;    // debug phase timers of the E-step kernels (TRLDA_ESTEP_TICKS=1)
 	PinnedBuf staging, readback;
-	int64_t docs_total_count = 0;    // sum of all counts in the (global) minibatch
-	int64_t global_B = 0;            // documents over all ranks
 	bool docs_resident = false;
 
 	// per-minibatch E-step buffers
-	DevBuf gamma, etheta, etheta32, weight, doc_stat, iterations;
+	DevBuf gamma, etheta, etheta32, weight, doc_stat, iterations, wordcount;
 	DevBuf gibbs_occ, gibbs_topics;            // Gibbs E-step scratch: occurrences before each document, one topic per occurrence
 	bool gamma_valid = false;
 
@@ -310,6 +304,24 @@ struct trlda_model {
 
 	double* lambda() { return lam[cur].as<double>(); }
 	double* lambda_next() { return lam[1 - cur].as<double>(); }
+
+	// the buffers free themselves after this body has run (trlda_destroy closes what refers to them first)
+	~trlda_model() {
+		for(int i = 0; i < kAuxStreams; ++i) {
+			if(aux[i])
+				cudaStreamDestroy(aux[i]);
+			if(join_event[i])
+				cudaEventDestroy(join_event[i]);
+		}
+		if(fork_event)
+			cudaEventDestroy(fork_event);
+		if(long_stream)
+			cudaStreamDestroy(long_stream);
+		if(long_join)
+			cudaEventDestroy(long_join);
+		if(stream)
+			cudaStreamDestroy(stream);
+	}
 };
 
 namespace {
@@ -426,7 +438,7 @@ int allreduce(trlda_model* m, void* buf, size_t count, ncclDataType_t type) {
 // rows = row sums of `matrix`
 int compute_rows(trlda_model* m, const double* matrix, double* out) {
 	int P = rowsum_num_partials(m->V);
-	CUDA_TRY(m, m->partials.ensure(sizeof(double) * (size_t) std::max(P, colsum_num_partials(std::max<int64_t>(m->docs.B, 1))) * m->K));
+	CUDA_TRY(m, m->partials.ensure(sizeof(double) * (size_t) std::max(P, colsum_num_partials(std::max<int64_t>(m->mb.docs.B, 1))) * m->K));
 	{
 		Launch l(m, KK_ROWSUM);
 		launch_rowsum(matrix, m->K, m->V, m->partials.as<double>(), &P, m->stream);
@@ -469,25 +481,7 @@ int prepare_beta(trlda_model* m, bool want_psi_partials = false) {
 	return check_launch(m, "beta_prep");
 }
 
-// exchanges the live minibatch state with a parking slot (pointer swaps only)
-void swap_with_slot(trlda_model* m, trlda_model::DocSlot& slot) {
-	std::swap(m->docs, slot.docs);
-	std::swap(m->b_doc_ptr, slot.b_doc_ptr);
-	std::swap(m->b_word_ids, slot.b_word_ids);
-	std::swap(m->b_counts, slot.b_counts);
-	std::swap(m->b_word_ptr, slot.b_word_ptr);
-	std::swap(m->b_tok_doc, slot.b_tok_doc);
-	std::swap(m->b_tok_src, slot.b_tok_src);
-	std::swap(m->b_order, slot.b_order);
-	std::swap(m->buckets, slot.buckets);
-	std::swap(m->sorted_len, slot.sorted_len);
-	std::swap(m->gdocs, slot.gdocs);
-	std::swap(m->len_gt, slot.len_gt);
-	std::swap(m->docs_total_count, slot.docs_total_count);
-	std::swap(m->global_B, slot.global_B);
-}
-
-int build_global_docs(trlda_model* m, const int64_t* s_ptr, int64_t B, int64_t N);
+int build_global_docs(trlda_model* m, int64_t B, int64_t N);
 
 // cuts the length-sorted documents [begin, B) into length buckets, each one launch of k_estep whose shared-memory tile
 // is sized for the bucket's longest document
@@ -518,9 +512,10 @@ int upload_docs(trlda_model* m, const trlda_docs* docs) {
 	TRY(set_device(m));
 	// the live buffers may belong to a parked minibatch (trlda_select_docs): hand them back before overwriting
 	if(m->live_slot >= 0) {
-		swap_with_slot(m, m->slots[m->live_slot]);
+		std::swap(m->mb, m->slots[m->live_slot].mb);
 		m->live_slot = -1;
 	}
+	trlda_model::Minibatch& mb = m->mb;
 	if(!docs || docs->num_docs < 0 || (docs->num_docs > 0 && !docs->doc_ptr))
 		return fail(m, TRLDA_ERR_ARG, "Documents must be given in CSR form.");
 	const int64_t B = docs->num_docs;
@@ -580,7 +575,7 @@ int upload_docs(trlda_model* m, const trlda_docs* docs) {
 		len_gt[3] += n > 64;
 	}
 	for(int i = 0; i < 4; ++i)
-		m->len_gt[i] = len_gt[i];
+		mb.len_gt[i] = len_gt[i];
 	// copy the id / count arrays into the pinned staging buffer (parallel slices), summing the counts and checking
 	// the id range on the way.  The word-sorted token list is built later, by ensure_csc(), right before the
 	// first kernel that needs it — by then the device is busy with the first E-step and the host work is hidden.
@@ -623,8 +618,8 @@ int upload_docs(trlda_model* m, const trlda_docs* docs) {
 	m->csc_threads = T;
 
 	// length buckets for the E-step: counting sort by length, longest first
-	m->buckets.clear();
-	m->sorted_len.resize(B);
+	mb.buckets.clear();
+	mb.sorted_len.resize(B);
 	if(B) {
 		std::vector<int32_t> start(n_max + 2, 0);
 		for(int64_t d = 0; d < B; ++d)
@@ -635,41 +630,41 @@ int upload_docs(trlda_model* m, const trlda_docs* docs) {
 			s_order[start[n_max - (int) (s_ptr[d + 1] - s_ptr[d])]++] = (int32_t) d;
 		for(int64_t i = 0; i < B; ++i) {
 			const int32_t d = s_order[i];
-			m->sorted_len[i] = (int) (s_ptr[d + 1] - s_ptr[d]);
+			mb.sorted_len[i] = (int) (s_ptr[d + 1] - s_ptr[d]);
 		}
-		form_buckets(m->sorted_len, 0, m->buckets);
+		form_buckets(mb.sorted_len, 0, mb.buckets);
 	}
 
 	const double t_host = ms_since(t_begin);
-	CUDA_TRY(m, m->b_order.ensure(sizeof(int32_t) * std::max<int64_t>(B, 1)));
-	CUDA_TRY(m, m->b_doc_ptr.ensure(sizeof(int64_t) * (B + 1)));
-	CUDA_TRY(m, m->b_word_ids.ensure(sizeof(int32_t) * std::max<int64_t>(N, 1)));
-	CUDA_TRY(m, m->b_counts.ensure(sizeof(int32_t) * std::max<int64_t>(N, 1)));
-	CUDA_TRY(m, m->b_word_ptr.ensure(sizeof(int32_t) * ((size_t) V + 1)));
-	CUDA_TRY(m, m->b_tok_doc.ensure(sizeof(int32_t) * std::max<int64_t>(N, 1)));
-	CUDA_TRY(m, m->b_tok_src.ensure(sizeof(int32_t) * std::max<int64_t>(N, 1)));
-	CUDA_TRY(m, cudaMemcpyAsync(m->b_doc_ptr.p, s_ptr, sizeof(int64_t) * (B + 1), cudaMemcpyHostToDevice, m->stream));
+	CUDA_TRY(m, mb.b_order.ensure(sizeof(int32_t) * std::max<int64_t>(B, 1)));
+	CUDA_TRY(m, mb.b_doc_ptr.ensure(sizeof(int64_t) * (B + 1)));
+	CUDA_TRY(m, mb.b_word_ids.ensure(sizeof(int32_t) * std::max<int64_t>(N, 1)));
+	CUDA_TRY(m, mb.b_counts.ensure(sizeof(int32_t) * std::max<int64_t>(N, 1)));
+	CUDA_TRY(m, mb.b_word_ptr.ensure(sizeof(int32_t) * ((size_t) V + 1)));
+	CUDA_TRY(m, mb.b_tok_doc.ensure(sizeof(int32_t) * std::max<int64_t>(N, 1)));
+	CUDA_TRY(m, mb.b_tok_src.ensure(sizeof(int32_t) * std::max<int64_t>(N, 1)));
+	CUDA_TRY(m, cudaMemcpyAsync(mb.b_doc_ptr.p, s_ptr, sizeof(int64_t) * (B + 1), cudaMemcpyHostToDevice, m->stream));
 	if(N) {
-		CUDA_TRY(m, cudaMemcpyAsync(m->b_word_ids.p, s_ids, sizeof(int32_t) * N, cudaMemcpyHostToDevice, m->stream));
-		CUDA_TRY(m, cudaMemcpyAsync(m->b_counts.p, s_cts, sizeof(int32_t) * N, cudaMemcpyHostToDevice, m->stream));
+		CUDA_TRY(m, cudaMemcpyAsync(mb.b_word_ids.p, s_ids, sizeof(int32_t) * N, cudaMemcpyHostToDevice, m->stream));
+		CUDA_TRY(m, cudaMemcpyAsync(mb.b_counts.p, s_cts, sizeof(int32_t) * N, cudaMemcpyHostToDevice, m->stream));
 	}
 	(void) s_wptr; (void) s_tdoc; (void) s_tsrc;
 	m->stage_off[0] = o_ptr; m->stage_off[1] = o_ids; m->stage_off[2] = o_wptr; m->stage_off[3] = o_tdoc; m->stage_off[4] = o_tsrc;
 	if(B)
-		CUDA_TRY(m, cudaMemcpyAsync(m->b_order.p, s_order, sizeof(int32_t) * B, cudaMemcpyHostToDevice, m->stream));
+		CUDA_TRY(m, cudaMemcpyAsync(mb.b_order.p, s_order, sizeof(int32_t) * B, cudaMemcpyHostToDevice, m->stream));
 	m->stats.h2d_bytes += total;
 
-	m->docs.B = B;
-	m->docs.N = N;
-	m->docs.n_max = n_max;
-	m->docs.doc_ptr = m->b_doc_ptr.as<int64_t>();
-	m->docs.word_ids = m->b_word_ids.as<int32_t>();
-	m->docs.counts = m->b_counts.as<int32_t>();
-	m->docs.word_ptr = m->b_word_ptr.as<int32_t>();
-	m->docs.tok_doc = m->b_tok_doc.as<int32_t>();
-	m->docs.tok_src = m->b_tok_src.as<int32_t>();
-	m->docs_total_count = total_count;
-	m->global_B = B;
+	mb.docs.B = B;
+	mb.docs.N = N;
+	mb.docs.n_max = n_max;
+	mb.docs.doc_ptr = mb.b_doc_ptr.as<int64_t>();
+	mb.docs.word_ids = mb.b_word_ids.as<int32_t>();
+	mb.docs.counts = mb.b_counts.as<int32_t>();
+	mb.docs.word_ptr = mb.b_word_ptr.as<int32_t>();
+	mb.docs.tok_doc = mb.b_tok_doc.as<int32_t>();
+	mb.docs.tok_src = mb.b_tok_src.as<int32_t>();
+	mb.docs_total_count = total_count;
+	mb.global_B = B;
 	m->gamma_valid = false;
 	m->docs_resident = true;
 
@@ -683,8 +678,8 @@ int upload_docs(trlda_model* m, const trlda_docs* docs) {
 		TRY(allreduce(m, m->scalars.p, 2, ncclInt64));
 		CUDA_TRY(m, cudaMemcpyAsync(h, m->scalars.p, 2 * sizeof(int64_t), cudaMemcpyDeviceToHost, m->stream));
 		CUDA_TRY(m, cudaStreamSynchronize(m->stream));
-		m->global_B = h[0];
-		m->docs_total_count = h[1];
+		mb.global_B = h[0];
+		mb.docs_total_count = h[1];
 	}
 
 	// per-minibatch buffers
@@ -695,9 +690,9 @@ int upload_docs(trlda_model* m, const trlda_docs* docs) {
 	CUDA_TRY(m, m->doc_stat.ensure(kb));
 	CUDA_TRY(m, m->weight.ensure(sizeof(double) * std::max<int64_t>(N, 1)));
 	CUDA_TRY(m, m->iterations.ensure(sizeof(int32_t) * std::max<int64_t>(B, 1)));
-	m->gdocs.ready = false;
+	mb.gdocs.ready = false;
 	if(m->nranks > 1 && m->use_gather && m->beta_elem == 4 && m->K % 4 == 0 && m->K <= 4096)
-		TRY(build_global_docs(m, s_ptr, B, N));
+		TRY(build_global_docs(m, B, N));
 	if(host_timing)
 		fprintf(stderr, "[trlda] upload_docs: wait for stream %.2f ms, host packing (copy + counting sort + buckets) %.2f ms, total incl. H2D enqueue %.2f ms\n",
 		        t_sync, t_host - t_sync, ms_since(t_begin));
@@ -729,8 +724,8 @@ int gather_segments(trlda_model* m, void* buf, const std::vector<int64_t>& off, 
 	return TRLDA_OK;
 }
 
-int build_global_docs(trlda_model* m, const int64_t* s_ptr, int64_t B, int64_t N) {
-	trlda_model::GlobalDocs& g = m->gdocs;
+int build_global_docs(trlda_model* m, int64_t B, int64_t N) {
+	trlda_model::GlobalDocs& g = m->mb.gdocs;
 	g.ready = false;
 	const int R = m->nranks;
 	// sizes of all shards
@@ -769,134 +764,31 @@ int build_global_docs(trlda_model* m, const int64_t* s_ptr, int64_t B, int64_t N
 		return fail(m, TRLDA_ERR_ARG, "Too many (word, count) pairs in one minibatch.");
 	CUDA_TRY(m, g.len.ensure(sizeof(int32_t) * std::max<int64_t>(g.B, 1)));
 	CUDA_TRY(m, g.ids.ensure(sizeof(int32_t) * std::max<int64_t>(g.N, 1)));
-	// TRLDA_GLOBAL_CSC=host: the first version of this function (ids back to the host, sorted by host threads, lists
-	// uploaded); default: everything on the device (csc.cu), no copy and no synchronisation after the sizes are known
-	static const bool host_sort = [] { const char* e = getenv("TRLDA_GLOBAL_CSC"); return e && !strcmp(e, "host"); }();
-	int32_t* h_len = nullptr;
-	int32_t* h_ids = nullptr;
-	if(host_sort) {
-		CUDA_TRY(m, m->gstage.ensure(sizeof(int32_t) * (size_t) (std::max<int64_t>(g.B, 1) + 3 * std::max<int64_t>(g.N, 1) + m->V + 2)));
-		h_len = m->gstage.as<int32_t>();
-		h_ids = h_len + std::max<int64_t>(g.B, 1);
-	}
-	launch_doc_lengths(m->b_doc_ptr.as<int64_t>(), B, g.pad_B[m->rank], g.len.as<int32_t>() + g.doc_off[m->rank], m->stream);
+	// everything on the device (csc.cu): no copy and no synchronisation after the sizes are known
+	launch_doc_lengths(m->mb.b_doc_ptr.as<int64_t>(), B, g.pad_B[m->rank], g.len.as<int32_t>() + g.doc_off[m->rank], m->stream);
 	if(g.pad_N[m->rank])
 		CUDA_TRY(m, cudaMemsetAsync(g.ids.as<int32_t>() + g.tok_off[m->rank], 0xff, sizeof(int32_t) * g.pad_N[m->rank], m->stream));   // -1: no word
 	if(N)
-		CUDA_TRY(m, cudaMemcpyAsync(g.ids.as<int32_t>() + g.tok_off[m->rank], m->b_word_ids.p, sizeof(int32_t) * N,
+		CUDA_TRY(m, cudaMemcpyAsync(g.ids.as<int32_t>() + g.tok_off[m->rank], m->mb.b_word_ids.p, sizeof(int32_t) * N,
 		                            cudaMemcpyDeviceToDevice, m->stream));
 	TRY(gather_segments(m, g.len.p, g.doc_off, g.pad_B, sizeof(int32_t), ncclInt32));
 	TRY(gather_segments(m, g.ids.p, g.tok_off, g.pad_N, sizeof(int32_t), ncclInt32));
-	if(!host_sort) {
-		const int v0 = word_begin(m, m->rank), v1 = word_begin(m, m->rank + 1);
-		CUDA_TRY(m, g.word_ptr.ensure(sizeof(int32_t) * ((size_t) m->V + 1)));
-		CUDA_TRY(m, g.tok_doc.ensure(sizeof(int32_t) * std::max<int64_t>(g.N, 1)));
-		CUDA_TRY(m, g.tok_src.ensure(sizeof(int32_t) * std::max<int64_t>(g.N, 1)));
-		CUDA_TRY(m, g.scratch.ensure(sizeof(int32_t) * global_csc_scratch_ints(g.B, g.N, v0, v1)));
-		CUDA_TRY(m, g.etheta32.ensure(sizeof(float) * (size_t) m->K * std::max<int64_t>(g.B, 1)));
-		CUDA_TRY(m, g.weight.ensure(sizeof(double) * std::max<int64_t>(g.N, 1)));
-		launch_global_csc(g.len.as<int32_t>(), g.ids.as<int32_t>(), R, g.pad_B[0], g.pad_N[0], v0, v1, m->V, g.scratch.as<int32_t>(),
-		                  g.word_ptr.as<int32_t>(), g.tok_doc.as<int32_t>(), g.tok_src.as<int32_t>(), m->stream);
-		TRY(check_launch(m, "word-sorted token list of the gathered minibatch"));
-		g.view = DeviceDocs{};
-		g.view.B = g.B;
-		g.view.N = g.N;
-		g.view.word_ptr = g.word_ptr.as<int32_t>();
-		g.view.tok_doc = g.tok_doc.as<int32_t>();
-		g.view.tok_src = g.tok_src.as<int32_t>();
-		g.ready = true;
-		return TRLDA_OK;
-	}
-	if(g.B)
-		CUDA_TRY(m, cudaMemcpyAsync(h_len, g.len.p, sizeof(int32_t) * g.B, cudaMemcpyDeviceToHost, m->stream));
-	if(g.N)
-		CUDA_TRY(m, cudaMemcpyAsync(h_ids, g.ids.p, sizeof(int32_t) * g.N, cudaMemcpyDeviceToHost, m->stream));
-	CUDA_TRY(m, cudaStreamSynchronize(m->stream));
-	// word-sorted token list of this rank's words [v0, v1): stable counting sort over the global token stream, the
-	// threads taking contiguous document ranges (as in ensure_csc)
-	const int v0 = word_begin(m, m->rank), v1 = word_begin(m, m->rank + 1), nv = v1 - v0;
-	int32_t* h_tdoc = h_ids + std::max<int64_t>(g.N, 1);
-	int32_t* h_tsrc = h_tdoc + std::max<int64_t>(g.N, 1);
-	int32_t* h_wptr = h_tsrc + std::max<int64_t>(g.N, 1);
-	// gptr[d] .. gptr[d] + len[d]: the tokens of (padded) global document d; a rank's documents are contiguous from tok_off
-	std::vector<int64_t> gptr((size_t) g.B + 1, 0);
-	for(int r = 0; r < R; ++r) {
-		int64_t at = g.tok_off[r];
-		for(int64_t d = g.doc_off[r]; d < g.doc_off[r] + g.pad_B[r]; ++d) {
-			gptr[d] = at;
-			at += h_len[d];
-		}
-	}
-	gptr[g.B] = g.N;
-	const int T = (int) std::max(1u, std::min(8u, std::min(std::thread::hardware_concurrency(), (unsigned) (g.N / 65536 + 1))));
-	std::vector<int64_t> cut(T + 1, g.B);
-	cut[0] = 0;
-	for(int t = 1; t < T; ++t)
-		cut[t] = g.B * t / T;
-	std::vector<std::vector<int32_t>> hist(T);
-	auto run = [&](auto&& fn) {
-		std::vector<std::thread> pool;
-		for(int t = 1; t < T; ++t)
-			pool.emplace_back(fn, t);
-		fn(0);
-		for(auto& th : pool)
-			th.join();
-	};
-	run([&](int t) {
-		hist[t].assign((size_t) std::max(nv, 1), 0);
-		int32_t* h = hist[t].data();
-		for(int64_t d = cut[t]; d < cut[t + 1]; ++d)
-			for(int64_t i = gptr[d]; i < gptr[d] + h_len[d]; ++i) {
-				const int32_t w = h_ids[i];
-				if(w >= v0 && w < v1)
-					h[w - v0]++;
-			}
-	});
-	int32_t total = 0;
-	for(int w = 0; w <= v0; ++w)
-		h_wptr[w] = 0;
-	for(int w = v0; w < v1; ++w) {
-		h_wptr[w] = total;
-		for(int t = 0; t < T; ++t) {
-			const int32_t c = hist[t][w - v0];
-			hist[t][w - v0] = total;
-			total += c;
-		}
-	}
-	for(int w = v1; w <= m->V; ++w)
-		h_wptr[w] = total;
-	const int64_t own = total;
-	run([&](int t) {
-		int32_t* cursor = hist[t].data();
-		for(int64_t d = cut[t]; d < cut[t + 1]; ++d)
-			for(int64_t i = gptr[d]; i < gptr[d] + h_len[d]; ++i) {
-				const int32_t w = h_ids[i];
-				if(w >= v0 && w < v1) {
-					const int32_t pos = cursor[w - v0]++;
-					h_tdoc[pos] = (int32_t) d;
-					h_tsrc[pos] = (int32_t) i;
-				}
-			}
-	});
+	const int v0 = word_begin(m, m->rank), v1 = word_begin(m, m->rank + 1);
 	CUDA_TRY(m, g.word_ptr.ensure(sizeof(int32_t) * ((size_t) m->V + 1)));
-	CUDA_TRY(m, g.tok_doc.ensure(sizeof(int32_t) * std::max<int64_t>(own, 1)));
-	CUDA_TRY(m, g.tok_src.ensure(sizeof(int32_t) * std::max<int64_t>(own, 1)));
+	CUDA_TRY(m, g.tok_doc.ensure(sizeof(int32_t) * std::max<int64_t>(g.N, 1)));
+	CUDA_TRY(m, g.tok_src.ensure(sizeof(int32_t) * std::max<int64_t>(g.N, 1)));
+	CUDA_TRY(m, g.scratch.ensure(sizeof(int32_t) * global_csc_scratch_ints(g.B, g.N, v0, v1)));
 	CUDA_TRY(m, g.etheta32.ensure(sizeof(float) * (size_t) m->K * std::max<int64_t>(g.B, 1)));
 	CUDA_TRY(m, g.weight.ensure(sizeof(double) * std::max<int64_t>(g.N, 1)));
-	CUDA_TRY(m, cudaMemcpyAsync(g.word_ptr.p, h_wptr, sizeof(int32_t) * ((size_t) m->V + 1), cudaMemcpyHostToDevice, m->stream));
-	if(own) {
-		CUDA_TRY(m, cudaMemcpyAsync(g.tok_doc.p, h_tdoc, sizeof(int32_t) * own, cudaMemcpyHostToDevice, m->stream));
-		CUDA_TRY(m, cudaMemcpyAsync(g.tok_src.p, h_tsrc, sizeof(int32_t) * own, cudaMemcpyHostToDevice, m->stream));
-	}
-	CUDA_TRY(m, cudaStreamSynchronize(m->stream));       // the pinned staging area is reused by the next upload
+	launch_global_csc(g.len.as<int32_t>(), g.ids.as<int32_t>(), R, g.pad_B[0], g.pad_N[0], v0, v1, m->V, g.scratch.as<int32_t>(),
+	                  g.word_ptr.as<int32_t>(), g.tok_doc.as<int32_t>(), g.tok_src.as<int32_t>(), m->stream);
+	TRY(check_launch(m, "word-sorted token list of the gathered minibatch"));
 	g.view = DeviceDocs{};
 	g.view.B = g.B;
 	g.view.N = g.N;
 	g.view.word_ptr = g.word_ptr.as<int32_t>();
 	g.view.tok_doc = g.tok_doc.as<int32_t>();
 	g.view.tok_src = g.tok_src.as<int32_t>();
-	m->stats.h2d_bytes += sizeof(int32_t) * (size_t) (m->V + 1 + 2 * own + B);
-	m->stats.d2h_bytes += sizeof(int32_t) * (size_t) (g.B + g.N);
 	g.ready = true;
 	return TRLDA_OK;
 }
@@ -904,13 +796,13 @@ int build_global_docs(trlda_model* m, const int64_t* s_ptr, int64_t B, int64_t N
 // where the E-step leaves exp(psi(gamma)) (float32) and the token weights: in the gather exchange straight into this
 // rank's segment of the global arrays
 float* estep_etheta32(trlda_model* m) {
-	if(m->gdocs.ready)
-		return m->gdocs.etheta32.as<float>() + (size_t) m->gdocs.doc_off[m->rank] * m->K;
+	if(m->mb.gdocs.ready)
+		return m->mb.gdocs.etheta32.as<float>() + (size_t) m->mb.gdocs.doc_off[m->rank] * m->K;
 	return m->etheta32.as<float>();
 }
 double* estep_weight(trlda_model* m) {
-	if(m->gdocs.ready)
-		return m->gdocs.weight.as<double>() + m->gdocs.tok_off[m->rank];
+	if(m->mb.gdocs.ready)
+		return m->mb.gdocs.weight.as<double>() + m->mb.gdocs.tok_off[m->rank];
 	return m->weight.as<double>();
 }
 
@@ -919,7 +811,7 @@ enum GammaSource { GAMMA_FRESH, GAMMA_KEEP, GAMMA_HOST };
 
 // fresh gamma: injected values if the parity seam is armed, else Gamma(100, 1/100) from the device generator
 int fresh_gamma(trlda_model* m) {
-	const int64_t B = m->docs.B;
+	const int64_t B = m->mb.docs.B;
 	if(m->inj_gamma_cols >= 0) {
 		if(m->inj_gamma_cols != B)
 			return fail(m, TRLDA_ERR_ARG, "Initial gamma has wrong dimensionality.");
@@ -955,7 +847,7 @@ int launch_buckets(trlda_model* m, const EStepArgs& a, const std::vector<trlda_m
 		cudaStream_t stream = lane == 0 ? m->stream : m->aux[lane - 1];
 		const EStepPlan plan = plan_estep(m->K, bucket.n_max, m->beta_elem, m->smem_optin);
 		m->stats.total_launches++;
-		launch_estep(plan, a, m->docs, m->b_order.as<int32_t>(), bucket.offset, std::min(bucket.count, end - bucket.offset),
+		launch_estep(plan, a, m->mb.docs, m->mb.b_order.as<int32_t>(), bucket.offset, std::min(bucket.count, end - bucket.offset),
 		             m->beta_elem, stream);
 	}
 	if(fork)
@@ -969,7 +861,7 @@ int launch_buckets(trlda_model* m, const EStepArgs& a, const std::vector<trlda_m
 int run_estep_buckets(trlda_model* m, const EStepArgs& a, int64_t end) {
 	Launch span(m, KK_ESTEP);   // one timing span for the whole E-step (the bucket launches overlap)
 	m->stats.total_launches--;  // the span itself is not a kernel; the launches are counted by launch_buckets
-	return launch_buckets(m, a, m->buckets, end);
+	return launch_buckets(m, a, m->mb.buckets, end);
 }
 
 // whether plan_estep keeps all per-pair vectors of a document of n pairs in shared memory
@@ -984,37 +876,37 @@ bool estep_fits(const trlda_model* m, int n) {
 // kernel when it takes the longest of them, else to k_estep over buckets formed without the long documents, and
 // [long_end, B) to the tensor-memory kernel.  One timing span covers the whole E-step.
 int run_estep_with_long(trlda_model* m, const EStepArgs& a, int64_t n_over, int64_t long_end) {
-	const int64_t B = m->docs.B;
-	const int32_t* order = m->b_order.as<int32_t>();
+	const int64_t B = m->mb.docs.B;
+	const int32_t* order = m->mb.b_order.as<int32_t>();
 	Launch span(m, KK_ESTEP);
 	m->stats.total_launches--;  // the span itself is not a kernel
 	int64_t pairs = 0;
 	for(int64_t i = 0; i < n_over; ++i)
-		pairs += m->sorted_len[i];
+		pairs += m->mb.sorted_len[i];
 	// no length limit is left to check: the plan's shared memory is the K-sized vectors (12 KB at K = 4096) plus as many
 	// tile columns as fit beside them, and the scratch grows with the documents
-	const EStepPlan plan = plan_estep_long(m->K, m->sorted_len[0], m->beta_elem, m->smem_optin);
+	const EStepPlan plan = plan_estep_long(m->K, m->mb.sorted_len[0], m->beta_elem, m->smem_optin);
 	CUDA_TRY(m, m->long_scratch.ensure(estep_long_scratch_bytes(plan, pairs)));
 	CUDA_TRY(m, cudaEventRecord(m->fork_event, m->stream));
 	CUDA_TRY(m, cudaStreamWaitEvent(m->long_stream, m->fork_event, 0));
 	m->stats.total_launches++;
-	launch_estep_long(plan, a, m->docs, order, 0, n_over, m->long_scratch.as<double>(), pairs, m->beta_elem, m->long_stream);
+	launch_estep_long(plan, a, m->mb.docs, order, 0, n_over, m->long_scratch.as<double>(), pairs, m->beta_elem, m->long_stream);
 	CUDA_TRY(m, cudaEventRecord(m->long_join, m->long_stream));
 	if(n_over < long_end) {
-		const int n_rest = m->sorted_len[n_over];
+		const int n_rest = m->mb.sorted_len[n_over];
 		if(stream_estep_applicable(m->K, n_rest, m->beta_elem, m->smem_optin)) {
 			m->stats.total_launches++;
-			launch_estep_stream(a, m->docs, order, n_over, long_end - n_over, n_rest, m->beta_elem, m->stream);
+			launch_estep_stream(a, m->mb.docs, order, n_over, long_end - n_over, n_rest, m->beta_elem, m->stream);
 			m->stream_ran = true;
 		} else {
 			std::vector<trlda_model::Bucket> buckets;
-			form_buckets(m->sorted_len, n_over, buckets);
+			form_buckets(m->mb.sorted_len, n_over, buckets);
 			TRY(launch_buckets(m, a, buckets, long_end));
 		}
 	}
 	if(long_end < B) {
 		m->stats.total_launches++;
-		if(launch_estep_tmem(a, m->docs, order, long_end, B - long_end, tmem_estep_max_len(), m->stream) != 0)
+		if(launch_estep_tmem(a, m->mb.docs, order, long_end, B - long_end, tmem_estep_max_len(), m->stream) != 0)
 			return fail(m, TRLDA_ERR_CUDA, "The tensor-memory E-step kernel could not be launched.");
 	}
 	CUDA_TRY(m, cudaStreamWaitEvent(m->stream, m->long_join, 0));
@@ -1025,10 +917,10 @@ int run_estep_with_long(trlda_model* m, const EStepArgs& a, int64_t n_over, int6
 int run_estep(trlda_model* m, GammaSource src, const double* host_gamma, int max_iter, double threshold) {
 	if(src == GAMMA_FRESH)
 		TRY(fresh_gamma(m));
-	else if(src == GAMMA_HOST && m->docs.B) {
-		CUDA_TRY(m, cudaMemcpyAsync(m->gamma.p, host_gamma, sizeof(double) * (size_t) m->K * m->docs.B,
+	else if(src == GAMMA_HOST && m->mb.docs.B) {
+		CUDA_TRY(m, cudaMemcpyAsync(m->gamma.p, host_gamma, sizeof(double) * (size_t) m->K * m->mb.docs.B,
 		                            cudaMemcpyHostToDevice, m->stream));
-		m->stats.h2d_bytes += sizeof(double) * (size_t) m->K * m->docs.B;
+		m->stats.h2d_bytes += sizeof(double) * (size_t) m->K * m->mb.docs.B;
 	}
 	EStepArgs a;
 	a.K = m->K;
@@ -1051,21 +943,21 @@ int run_estep(trlda_model* m, GammaSource src, const double* host_gamma, int max
 	// all of them, go to the streaming kernel (estep_stream.cu), which re-reads the tile from L2 once per inner
 	// iteration, or, for what it does not cover (unaligned K, K beyond its per-lane register tile, documents too long
 	// for its shared memory), to the shared-memory cluster kernel (kernels.cu).
-	const int64_t B = m->docs.B;
-	const int32_t* order = m->b_order.as<int32_t>();
+	const int64_t B = m->mb.docs.B;
+	const int32_t* order = m->mb.b_order.as<int32_t>();
 	const bool tmem = m->tmem_mode && tmem_estep_applicable(m->K, m->beta_elem);
-	const int64_t long_end = tmem ? m->len_gt[0] : B;
+	const int64_t long_end = tmem ? m->mb.len_gt[0] : B;
 	// documents too long for both the streaming kernel and the shared memory of k_estep: order[0, n_over)
 	int64_t n_over = 0;
-	if(long_end > 0 && !stream_estep_applicable(m->K, m->docs.n_max, m->beta_elem, m->smem_optin))
-		while(n_over < long_end && !estep_fits(m, m->sorted_len[n_over]))
+	if(long_end > 0 && !stream_estep_applicable(m->K, m->mb.docs.n_max, m->beta_elem, m->smem_optin))
+		while(n_over < long_end && !estep_fits(m, m->mb.sorted_len[n_over]))
 			++n_over;
 	if(n_over > 0) {
 		TRY(run_estep_with_long(m, a, n_over, long_end));
 	} else if(long_end > 0) {
-		if(stream_estep_applicable(m->K, m->docs.n_max, m->beta_elem, m->smem_optin)) {
+		if(stream_estep_applicable(m->K, m->mb.docs.n_max, m->beta_elem, m->smem_optin)) {
 			Launch l(m, KK_ESTEP);
-			launch_estep_stream(a, m->docs, order, 0, long_end, m->docs.n_max, m->beta_elem, m->stream);
+			launch_estep_stream(a, m->mb.docs, order, 0, long_end, m->mb.docs.n_max, m->beta_elem, m->stream);
 			m->stream_ran = true;
 		} else {
 			TRY(run_estep_buckets(m, a, long_end));
@@ -1073,7 +965,7 @@ int run_estep(trlda_model* m, GammaSource src, const double* host_gamma, int max
 	}
 	if(long_end < B && n_over == 0) {
 		Launch l(m, KK_ESTEP);
-		if(launch_estep_tmem(a, m->docs, order, long_end, B - long_end, tmem_estep_max_len(), m->stream) != 0)
+		if(launch_estep_tmem(a, m->mb.docs, order, long_end, B - long_end, tmem_estep_max_len(), m->stream) != 0)
 			return fail(m, TRLDA_ERR_CUDA, "The tensor-memory E-step kernel could not be launched.");
 	}
 	m->gamma_valid = true;
@@ -1083,11 +975,11 @@ int run_estep(trlda_model* m, GammaSource src, const double* host_gamma, int max
 
 // row sums of the sufficient statistics of the last E-step (summed over ranks) -> rows_stat
 int reduce_doc_stat(trlda_model* m) {
-	const int P = colsum_num_partials(m->docs.B);
+	const int P = colsum_num_partials(m->mb.docs.B);
 	CUDA_TRY(m, m->partials.ensure(sizeof(double) * (size_t) std::max(P, rowsum_num_partials(m->V)) * m->K));
 	{
 		Launch l(m, KK_REDUCE);
-		launch_colsum(m->doc_stat.as<double>(), m->K, m->docs.B, m->partials.as<double>(), m->rows_stat.as<double>(), m->stream);
+		launch_colsum(m->doc_stat.as<double>(), m->K, m->mb.docs.B, m->partials.as<double>(), m->rows_stat.as<double>(), m->stream);
 	}
 	TRY(check_launch(m, "colsum"));
 	return allreduce(m, m->rows_stat.p, m->K, ncclDouble);
@@ -1101,7 +993,7 @@ int ensure_csc(trlda_model* m) {
 	if(!m->csc_pending)
 		return TRLDA_OK;
 	m->csc_pending = false;
-	const int64_t B = m->docs.B, N = m->docs.N;
+	const int64_t B = m->mb.docs.B, N = m->mb.docs.N;
 	const int V = m->V;
 	const int T = std::max(1, m->csc_threads);
 	char* base = m->staging.as<char>();
@@ -1151,10 +1043,10 @@ int ensure_csc(trlda_model* m) {
 			}
 	});
 	if(N) {
-		CUDA_TRY(m, cudaMemcpyAsync(m->b_tok_doc.p, s_tdoc, sizeof(int32_t) * N, cudaMemcpyHostToDevice, m->stream));
-		CUDA_TRY(m, cudaMemcpyAsync(m->b_tok_src.p, s_tsrc, sizeof(int32_t) * N, cudaMemcpyHostToDevice, m->stream));
+		CUDA_TRY(m, cudaMemcpyAsync(m->mb.b_tok_doc.p, s_tdoc, sizeof(int32_t) * N, cudaMemcpyHostToDevice, m->stream));
+		CUDA_TRY(m, cudaMemcpyAsync(m->mb.b_tok_src.p, s_tsrc, sizeof(int32_t) * N, cudaMemcpyHostToDevice, m->stream));
 	}
-	CUDA_TRY(m, cudaMemcpyAsync(m->b_word_ptr.p, s_wptr, sizeof(int32_t) * ((size_t) V + 1), cudaMemcpyHostToDevice, m->stream));
+	CUDA_TRY(m, cudaMemcpyAsync(m->mb.b_word_ptr.p, s_wptr, sizeof(int32_t) * ((size_t) V + 1), cudaMemcpyHostToDevice, m->stream));
 	return TRLDA_OK;
 }
 
@@ -1183,7 +1075,7 @@ int run_scatter_dense(trlda_model* m, bool reduce_over_ranks = true, bool for_pe
 	a.fused = false;
 	{
 		Launch l(m, KK_SCATTER);
-		launch_scatter(a, m->docs, m->stream);
+		launch_scatter(a, m->mb.docs, m->stream);
 	}
 	TRY(check_launch(m, "scatter"));
 	if(!reduce_over_ranks)
@@ -1223,11 +1115,11 @@ int run_mstep(trlda_model* m, const MStepCoef& coef, const double* prime, double
 		launch_rows_update(coef.mode == MSTEP_BATCH ? nullptr : m->rows_prev.as<double>(), m->rows_stat.as<double>(), a, b, c,
 		                   m->K, m->rows.as<double>(), m->psi_rows.as<double>(), m->stream);
 	}
-	if(m->nranks > 1 && m->gdocs.ready && !force_dense) {
+	if(m->nranks > 1 && m->mb.gdocs.ready && !force_dense) {
 		// gather exchange: (1) every rank receives all documents' etheta and token weights; (2) the single-GPU kernel
 		// (scatter + blend + beta-prep) runs on this rank's words over the tokens of ALL documents; (3) the ranks
 		// exchange their slices of the new beta (and, when the caller needs lambda afterwards, of lambda)
-		trlda_model::GlobalDocs& g = m->gdocs;
+		trlda_model::GlobalDocs& g = m->mb.gdocs;
 		const int v0 = word_begin(m, m->rank), v1 = word_begin(m, m->rank + 1);
 		{
 			std::vector<int64_t> eoff(m->nranks), en(m->nranks);
@@ -1408,7 +1300,7 @@ int run_mstep(trlda_model* m, const MStepCoef& coef, const double* prime, double
 		sa.write_beta = write_beta;
 		sa.psi_partials = want_psi_partials ? m->vpartials.as<double>() : nullptr;
 		Launch l(m, KK_SCATTER_MSTEP);
-		launch_scatter(sa, m->docs, m->stream);
+		launch_scatter(sa, m->mb.docs, m->stream);
 	}
 	m->beta_valid = write_beta;
 	return check_launch(m, "mstep");
@@ -1429,13 +1321,13 @@ int alpha_statistics(trlda_model* m, std::vector<double>& diff) {
 	// doc_stat is free after the M-step: reuse it for the per-document terms
 	{
 		Launch l(m, KK_ALPHA_STATS);
-		launch_alpha_stats(m->gamma.as<double>(), m->K, m->docs.B, m->doc_stat.as<double>(), m->stream);
+		launch_alpha_stats(m->gamma.as<double>(), m->K, m->mb.docs.B, m->doc_stat.as<double>(), m->stream);
 	}
-	const int P = colsum_num_partials(m->docs.B);
+	const int P = colsum_num_partials(m->mb.docs.B);
 	CUDA_TRY(m, m->partials.ensure(sizeof(double) * (size_t) std::max(P, rowsum_num_partials(m->V)) * m->K));
 	{
 		Launch l(m, KK_REDUCE);
-		launch_colsum(m->doc_stat.as<double>(), m->K, m->docs.B, m->partials.as<double>(), m->rows_stat.as<double>(), m->stream);
+		launch_colsum(m->doc_stat.as<double>(), m->K, m->mb.docs.B, m->partials.as<double>(), m->rows_stat.as<double>(), m->stream);
 	}
 	TRY(check_launch(m, "alpha_stats"));
 	TRY(allreduce(m, m->rows_stat.p, m->K, ncclDouble));
@@ -1544,7 +1436,7 @@ void consume_injections(trlda_model* m) {
 
 // ---- OnlineLDA::updateParameters, onlinelda.cpp:53-180 ---------------------------------------------------------------
 int online_update(trlda_model* m, const trlda_params* p, double* result) {
-	const int64_t B = m->global_B;
+	const int64_t B = m->mb.global_B;
 	if(B == 0) {
 		*result = 1.0;                                               // :54-56 (returns `true`), counter untouched
 		return TRLDA_OK;
@@ -1574,19 +1466,19 @@ int online_update(trlda_model* m, const trlda_params* p, double* result) {
 			CUDA_TRY(m, m->wordcount.ensure(sizeof(double) * m->V));
 			{
 				Launch l(m, KK_MISC);
-				launch_wordcount(m->docs, m->V, m->wordcount.as<double>(), m->stream);
+				launch_wordcount(m->mb.docs, m->V, m->wordcount.as<double>(), m->stream);
 			}
 			TRY(allreduce(m, m->wordcount.p, m->V, ncclDouble));
 			const double scale_k = (double) m->num_documents / (double) B / (double) m->K;
 			{
 				Launch l(m, KK_MISC);
 				launch_rows_update(m->rows_prev.as<double>(), nullptr, 1. - rho,
-				                   rho * (m->V * m->eta + scale_k * (double) m->docs_total_count), 0., m->K,
+				                   rho * (m->V * m->eta + scale_k * (double) m->mb.docs_total_count), 0., m->K,
 				                   m->rows.as<double>(), m->psi_rows.as<double>(), m->stream);
 			}
 			{
 				Launch l(m, KK_INIT_UPDATE);
-				launch_init_update(m->docs, m->K, m->V, rho, m->eta, scale_k, prime, target, m->psi_rows.as<double>(),
+				launch_init_update(m->mb.docs, m->K, m->V, rho, m->eta, scale_k, prime, target, m->psi_rows.as<double>(),
 				                   m->beta.p, m->beta_elem, m->wordcount.as<double>(), m->stream);
 			}
 			TRY(check_launch(m, "init_update"));
@@ -1676,7 +1568,7 @@ int online_update(trlda_model* m, const trlda_params* p, double* result) {
 
 // ---- BatchLDA::updateParameters, batchlda.cpp:43-209 -------------------------------------------------------------------
 int batch_update(trlda_model* m, const trlda_params* p, double* result) {
-	const int64_t B = m->global_B;
+	const int64_t B = m->mb.global_B;
 	*result = 1.;
 	if(B == 0)
 		return TRLDA_OK;
@@ -1746,7 +1638,7 @@ int batch_update(trlda_model* m, const trlda_params* p, double* result) {
 
 // ---- CumulativeLDA::updateParameters, cumulativelda.cpp:49-153 ----------------------------------------------------------
 int cumulative_update(trlda_model* m, const trlda_params* p, double* result) {
-	const int64_t B = m->global_B;
+	const int64_t B = m->mb.global_B;
 	*result = 1.;
 	if(B == 0)
 		return TRLDA_OK;
@@ -1996,8 +1888,8 @@ void trlda_destroy(trlda_model* m) {
 			for(int i = 0; i < 5; ++i)
 				fprintf(stderr, "[trlda]   %-26s %10.0f cycles/doc\n", stream_names[i], t[15] ? (double) t[i] / (double) t[15] : 0.0);
 		}
-		m->ticks.release();
 	}
+	// the peer mappings and the communicator refer to this model's buffers: gone before the buffers are freed
 	for(void* p : m->peer_opened)
 		cudaIpcCloseMemHandle(p);
 	if(m->comm && nccl_api().ok)
@@ -2005,43 +1897,6 @@ void trlda_destroy(trlda_model* m) {
 	collect_spans(m);
 	for(cudaEvent_t e : m->event_pool)
 		cudaEventDestroy(e);
-	DevBuf* bufs[] = {&m->ada_gradient, &m->lam[0], &m->lam[1], &m->beta, &m->sstats, &m->sstats32, &m->rows, &m->rows_prev, &m->rows_stat,
-	                  &m->psi_rows, &m->d_alpha, &m->partials, &m->vpartials, &m->scalars, &m->b_doc_ptr, &m->b_word_ids,
-	                  &m->b_counts, &m->b_word_ptr, &m->b_tok_doc, &m->b_tok_src, &m->b_order, &m->wordcount, &m->gamma, &m->etheta,
-	                  &m->etheta32, &m->weight, &m->doc_stat, &m->iterations, &m->gibbs_occ, &m->gibbs_topics, &m->sweeps,
-	                  &m->sample_cdf, &m->sample_tokens, &m->sample_counts, &m->sample_lengths, &m->long_scratch};
-	for(DevBuf* b : bufs)
-		b->release();
-	{
-		DevBuf* gb[] = {&m->gdocs.len, &m->gdocs.ids, &m->gdocs.word_ptr, &m->gdocs.tok_doc, &m->gdocs.tok_src, &m->gdocs.etheta32, &m->gdocs.weight, &m->gdocs.scratch};
-		for(DevBuf* b : gb)
-			b->release();
-		m->gstage.release();
-	}
-	for(auto& slot : m->slots) {
-		DevBuf* gb[] = {&slot.gdocs.len, &slot.gdocs.ids, &slot.gdocs.word_ptr, &slot.gdocs.tok_doc, &slot.gdocs.tok_src, &slot.gdocs.etheta32, &slot.gdocs.weight, &slot.gdocs.scratch};
-		for(DevBuf* b : gb)
-			b->release();
-		DevBuf* sb[] = {&slot.b_doc_ptr, &slot.b_word_ids, &slot.b_counts, &slot.b_word_ptr, &slot.b_tok_doc, &slot.b_tok_src, &slot.b_order};
-		for(DevBuf* b : sb)
-			b->release();
-	}
-	m->staging.release();
-	m->readback.release();
-	for(int i = 0; i < trlda_model::kAuxStreams; ++i) {
-		if(m->aux[i])
-			cudaStreamDestroy(m->aux[i]);
-		if(m->join_event[i])
-			cudaEventDestroy(m->join_event[i]);
-	}
-	if(m->fork_event)
-		cudaEventDestroy(m->fork_event);
-	if(m->long_stream)
-		cudaStreamDestroy(m->long_stream);
-	if(m->long_join)
-		cudaEventDestroy(m->long_join);
-	if(m->stream)
-		cudaStreamDestroy(m->stream);
 	delete m;
 }
 
@@ -2166,14 +2021,14 @@ int trlda_upload_docs_slot(trlda_model* m, const trlda_docs* docs, int slot) {
 		m->slots.resize(slot + 1);
 	// park the live minibatch (if it belongs to a slot), upload into fresh live buffers, finish the token list, park
 	if(m->live_slot >= 0)
-		swap_with_slot(m, m->slots[m->live_slot]);
+		std::swap(m->mb, m->slots[m->live_slot].mb);
 	m->live_slot = -1;
 	if(m->slots[slot].used)
-		swap_with_slot(m, m->slots[slot]);                     // reuse the slot's buffers
+		std::swap(m->mb, m->slots[slot].mb);                   // reuse the slot's buffers
 	TRY(upload_docs(m, docs));
 	TRY(ensure_csc(m));
 	CUDA_TRY(m, cudaStreamSynchronize(m->stream));            // the pinned staging buffer is reused by the next upload
-	swap_with_slot(m, m->slots[slot]);
+	std::swap(m->mb, m->slots[slot].mb);
 	m->slots[slot].used = true;
 	m->docs_resident = false;
 	return TRLDA_OK;
@@ -2186,8 +2041,8 @@ int trlda_select_docs(trlda_model* m, int slot) {
 	if(m->live_slot == slot)
 		return TRLDA_OK;
 	if(m->live_slot >= 0)
-		swap_with_slot(m, m->slots[m->live_slot]);
-	swap_with_slot(m, m->slots[slot]);
+		std::swap(m->mb, m->slots[m->live_slot].mb);
+	std::swap(m->mb, m->slots[slot].mb);
 	m->live_slot = slot;
 	m->docs_resident = true;
 	m->csc_pending = false;
@@ -2208,7 +2063,7 @@ static int gibbs_variables(trlda_model* m, const trlda_docs* docs, const double*
 		return fail(m, TRLDA_ERR_UNSUPPORTED, "The Gibbs E-step is not sharded over GPUs.");
 	TRY(upload_docs(m, docs));
 	TRY(prepare_beta(m));
-	const int64_t B = m->docs.B;
+	const int64_t B = m->mb.docs.B;
 	const size_t kb = sizeof(double) * (size_t) m->K * (size_t) B;
 	std::vector<int64_t> occ((size_t) B + 1, 0);
 	for(int64_t d = 0; d < B; ++d) {
@@ -2228,7 +2083,7 @@ static int gibbs_variables(trlda_model* m, const trlda_docs* docs, const double*
 	}
 	{
 		Launch l(m, KK_ESTEP);
-		launch_gibbs(m->docs, m->K, m->beta.p, m->beta_elem, m->d_alpha.as<double>(), latents ? m->etheta.as<double>() : nullptr,
+		launch_gibbs(m->mb.docs, m->K, m->beta.p, m->beta_elem, m->d_alpha.as<double>(), latents ? m->etheta.as<double>() : nullptr,
 		             m->gibbs_occ.as<int64_t>(), m->gibbs_topics.as<uint16_t>(), params->num_samples, params->burn_in,
 		             current_seed() ^ (next_stream_id() * 0x9E3779B97F4A7C15ull), m->gamma.as<double>(), m->sstats.as<double>(),
 		             m->stream);
@@ -2260,9 +2115,9 @@ int trlda_update_variables(trlda_model* m, const trlda_docs* docs, const double*
 	TRY(run_estep(m, latents ? GAMMA_HOST : GAMMA_FRESH, latents, params->max_iter_inference, params->threshold));
 	if(sstats_out)
 		TRY(run_scatter_dense(m));
-	if(gamma_out && m->docs.B) {
-		CUDA_TRY(m, cudaMemcpyAsync(gamma_out, m->gamma.p, sizeof(double) * (size_t) m->K * m->docs.B, cudaMemcpyDeviceToHost, m->stream));
-		m->stats.d2h_bytes += sizeof(double) * (size_t) m->K * m->docs.B;
+	if(gamma_out && m->mb.docs.B) {
+		CUDA_TRY(m, cudaMemcpyAsync(gamma_out, m->gamma.p, sizeof(double) * (size_t) m->K * m->mb.docs.B, cudaMemcpyDeviceToHost, m->stream));
+		m->stats.d2h_bytes += sizeof(double) * (size_t) m->K * m->mb.docs.B;
 	}
 	if(sstats_out) {
 		CUDA_TRY(m, cudaMemcpyAsync(sstats_out, m->sstats.p, kv_bytes(m), cudaMemcpyDeviceToHost, m->stream));
@@ -2270,9 +2125,9 @@ int trlda_update_variables(trlda_model* m, const trlda_docs* docs, const double*
 	}
 	CUDA_TRY(m, cudaStreamSynchronize(m->stream));
 	// iteration statistics of this E-step
-	if(m->docs.B) {
-		std::vector<int32_t> it(m->docs.B);
-		CUDA_TRY(m, cudaMemcpy(it.data(), m->iterations.p, sizeof(int32_t) * m->docs.B, cudaMemcpyDeviceToHost));
+	if(m->mb.docs.B) {
+		std::vector<int32_t> it(m->mb.docs.B);
+		CUDA_TRY(m, cudaMemcpy(it.data(), m->iterations.p, sizeof(int32_t) * m->mb.docs.B, cudaMemcpyDeviceToHost));
 		int64_t total = 0;
 		for(int32_t v : it)
 			total += v;
@@ -2305,10 +2160,10 @@ int trlda_lower_bound(trlda_model* m, const trlda_docs* docs, const double* late
 	if(latents && (latents_rows != m->K || latents_cols != docs->num_docs))
 		return fail(m, TRLDA_ERR_ARG, "Initial gamma has wrong dimensionality.");
 	TRY(upload_docs(m, docs));
-	const int64_t B = m->docs.B;
+	const int64_t B = m->mb.docs.B;
 	if(m->kind == TRLDA_KIND_ONLINE && num_documents < 0)
 		num_documents = m->num_documents;                                      // onlinelda.cpp:184-191
-	const double factor = num_documents >= 0 ? (double) num_documents / (double) m->global_B : 1.;   // lda.cpp:303-304
+	const double factor = num_documents >= 0 ? (double) num_documents / (double) m->mb.global_B : 1.;   // lda.cpp:303-304
 	TRY(prepare_beta(m));                                                      // also leaves rows / psi_rows of lambda
 	TRY(run_estep(m, latents ? GAMMA_HOST : GAMMA_FRESH, latents, params->max_iter_inference, params->threshold));   // :307
 
@@ -2322,7 +2177,7 @@ int trlda_lower_bound(trlda_model* m, const trlda_docs* docs, const double* late
 	double* per_doc = m->doc_stat.as<double>();
 	{
 		Launch l(m, KK_ELBO);
-		launch_elbo_docs(m->docs, m->K, m->lambda(), m->psi_rows.as<double>(), m->d_alpha.as<double>(), alpha_const,
+		launch_elbo_docs(m->mb.docs, m->K, m->lambda(), m->psi_rows.as<double>(), m->d_alpha.as<double>(), alpha_const,
 		                 m->gamma.as<double>(), per_doc, m->stream);
 	}
 	{
@@ -2363,36 +2218,29 @@ int trlda_debug_global_csc(trlda_model* m, const int32_t* len, const int32_t* id
 		return fail(m, TRLDA_ERR_ARG, "debug_global_csc: bad arguments.");
 	const int64_t B = (int64_t) ranks * max_docs, N = (int64_t) ranks * max_pairs;
 	DevBuf d_len, d_ids, d_wptr, d_tdoc, d_tsrc, d_scratch;
-	auto run = [&]() -> int {
-		CUDA_TRY(m, d_len.ensure(sizeof(int32_t) * std::max<int64_t>(B, 1)));
-		CUDA_TRY(m, d_ids.ensure(sizeof(int32_t) * std::max<int64_t>(N, 1)));
-		CUDA_TRY(m, d_wptr.ensure(sizeof(int32_t) * ((size_t) m->V + 1)));
-		CUDA_TRY(m, d_tdoc.ensure(sizeof(int32_t) * std::max<int64_t>(N, 1)));
-		CUDA_TRY(m, d_tsrc.ensure(sizeof(int32_t) * std::max<int64_t>(N, 1)));
-		CUDA_TRY(m, d_scratch.ensure(sizeof(int32_t) * global_csc_scratch_ints(B, N, v0, v1)));
-		if(B)
-			CUDA_TRY(m, cudaMemcpyAsync(d_len.p, len, sizeof(int32_t) * B, cudaMemcpyHostToDevice, m->stream));
-		if(N) {
-			CUDA_TRY(m, cudaMemcpyAsync(d_ids.p, ids, sizeof(int32_t) * N, cudaMemcpyHostToDevice, m->stream));
-			CUDA_TRY(m, cudaMemsetAsync(d_tdoc.p, 0xff, sizeof(int32_t) * N, m->stream));
-			CUDA_TRY(m, cudaMemsetAsync(d_tsrc.p, 0xff, sizeof(int32_t) * N, m->stream));
-		}
-		launch_global_csc(d_len.as<int32_t>(), d_ids.as<int32_t>(), ranks, max_docs, max_pairs, v0, v1, m->V, d_scratch.as<int32_t>(),
-		                  d_wptr.as<int32_t>(), d_tdoc.as<int32_t>(), d_tsrc.as<int32_t>(), m->stream);
-		TRY(check_launch(m, "debug_global_csc"));
-		CUDA_TRY(m, cudaMemcpyAsync(word_ptr, d_wptr.p, sizeof(int32_t) * ((size_t) m->V + 1), cudaMemcpyDeviceToHost, m->stream));
-		if(N) {
-			CUDA_TRY(m, cudaMemcpyAsync(tok_doc, d_tdoc.p, sizeof(int32_t) * N, cudaMemcpyDeviceToHost, m->stream));
-			CUDA_TRY(m, cudaMemcpyAsync(tok_src, d_tsrc.p, sizeof(int32_t) * N, cudaMemcpyDeviceToHost, m->stream));
-		}
-		CUDA_TRY(m, cudaStreamSynchronize(m->stream));
-		return TRLDA_OK;
-	};
-	const int status = run();
-	DevBuf* all[] = {&d_len, &d_ids, &d_wptr, &d_tdoc, &d_tsrc, &d_scratch};
-	for(DevBuf* b : all)
-		b->release();
-	return status;
+	CUDA_TRY(m, d_len.ensure(sizeof(int32_t) * std::max<int64_t>(B, 1)));
+	CUDA_TRY(m, d_ids.ensure(sizeof(int32_t) * std::max<int64_t>(N, 1)));
+	CUDA_TRY(m, d_wptr.ensure(sizeof(int32_t) * ((size_t) m->V + 1)));
+	CUDA_TRY(m, d_tdoc.ensure(sizeof(int32_t) * std::max<int64_t>(N, 1)));
+	CUDA_TRY(m, d_tsrc.ensure(sizeof(int32_t) * std::max<int64_t>(N, 1)));
+	CUDA_TRY(m, d_scratch.ensure(sizeof(int32_t) * global_csc_scratch_ints(B, N, v0, v1)));
+	if(B)
+		CUDA_TRY(m, cudaMemcpyAsync(d_len.p, len, sizeof(int32_t) * B, cudaMemcpyHostToDevice, m->stream));
+	if(N) {
+		CUDA_TRY(m, cudaMemcpyAsync(d_ids.p, ids, sizeof(int32_t) * N, cudaMemcpyHostToDevice, m->stream));
+		CUDA_TRY(m, cudaMemsetAsync(d_tdoc.p, 0xff, sizeof(int32_t) * N, m->stream));
+		CUDA_TRY(m, cudaMemsetAsync(d_tsrc.p, 0xff, sizeof(int32_t) * N, m->stream));
+	}
+	launch_global_csc(d_len.as<int32_t>(), d_ids.as<int32_t>(), ranks, max_docs, max_pairs, v0, v1, m->V, d_scratch.as<int32_t>(),
+	                  d_wptr.as<int32_t>(), d_tdoc.as<int32_t>(), d_tsrc.as<int32_t>(), m->stream);
+	TRY(check_launch(m, "debug_global_csc"));
+	CUDA_TRY(m, cudaMemcpyAsync(word_ptr, d_wptr.p, sizeof(int32_t) * ((size_t) m->V + 1), cudaMemcpyDeviceToHost, m->stream));
+	if(N) {
+		CUDA_TRY(m, cudaMemcpyAsync(tok_doc, d_tdoc.p, sizeof(int32_t) * N, cudaMemcpyDeviceToHost, m->stream));
+		CUDA_TRY(m, cudaMemcpyAsync(tok_src, d_tsrc.p, sizeof(int32_t) * N, cudaMemcpyDeviceToHost, m->stream));
+	}
+	CUDA_TRY(m, cudaStreamSynchronize(m->stream));
+	return TRLDA_OK;
 }
 
 int trlda_sample(trlda_model* m, int64_t num_documents, double length, int collapse, trlda_docs* out) {
@@ -2524,8 +2372,6 @@ int trlda_comm_init(trlda_model* m, const void* id_bytes, int rank, int nranks) 
 	NCCL_TRY(m, nccl_api().AllGather(send.p, recv.p, sizeof(local), ncclUint8, m->comm, m->stream));
 	CUDA_TRY(m, cudaMemcpyAsync(handles.data(), recv.p, sizeof(local) * nranks, cudaMemcpyDeviceToHost, m->stream));
 	CUDA_TRY(m, cudaStreamSynchronize(m->stream));
-	send.release();
-	recv.release();
 	bool ok = true;
 	for(int r = 0; r < nranks && ok; ++r) {
 		void* ptrs[4];
@@ -2582,14 +2428,14 @@ int trlda_get_stats(trlda_model* m, trlda_stats* out) {
 	CUDA_TRY(m, cudaStreamSynchronize(m->stream));
 	collect_spans(m);
 	// inner-iteration total of the most recent E-step
-	if(m->gamma_valid && m->docs.B) {
-		std::vector<int32_t> it(m->docs.B);
-		CUDA_TRY(m, cudaMemcpy(it.data(), m->iterations.p, sizeof(int32_t) * m->docs.B, cudaMemcpyDeviceToHost));
+	if(m->gamma_valid && m->mb.docs.B) {
+		std::vector<int32_t> it(m->mb.docs.B);
+		CUDA_TRY(m, cudaMemcpy(it.data(), m->iterations.p, sizeof(int32_t) * m->mb.docs.B, cudaMemcpyDeviceToHost));
 		int64_t total = 0;
 		for(int32_t v : it)
 			total += v;
 		m->stats.estep_doc_iterations = total;
-		m->stats.estep_docs = m->docs.B;
+		m->stats.estep_docs = m->mb.docs.B;
 	}
 	if(m->sweeps.p) {
 		unsigned long long total = 0;
@@ -2622,16 +2468,12 @@ int trlda_get_row_sums(trlda_model* m, double* out) {
 int trlda_device_special(int device, int which, const double* x, int64_t n, double* out) {
 	if(cudaSetDevice(device) != cudaSuccess)
 		return fail(nullptr, TRLDA_ERR_CUDA, "No CUDA device available; trlda_b200 has no CPU fallback.");
-	double *dx = nullptr, *dy = nullptr;
-	if(cudaMalloc(&dx, sizeof(double) * n) != cudaSuccess || cudaMalloc(&dy, sizeof(double) * n) != cudaSuccess) {
-		cudaFree(dx);
+	DevBuf dx, dy;
+	if(dx.ensure(sizeof(double) * n) != cudaSuccess || dy.ensure(sizeof(double) * n) != cudaSuccess)
 		return fail(nullptr, TRLDA_ERR_CUDA, "cudaMalloc failed.");
-	}
-	cudaMemcpy(dx, x, sizeof(double) * n, cudaMemcpyHostToDevice);
-	launch_special(which, dx, n, dy, 0);
-	cudaError_t e = cudaMemcpy(out, dy, sizeof(double) * n, cudaMemcpyDeviceToHost);
-	cudaFree(dx);
-	cudaFree(dy);
+	cudaMemcpy(dx.p, x, sizeof(double) * n, cudaMemcpyHostToDevice);
+	launch_special(which, dx.as<double>(), n, dy.as<double>(), 0);
+	const cudaError_t e = cudaMemcpy(out, dy.p, sizeof(double) * n, cudaMemcpyDeviceToHost);
 	if(e != cudaSuccess)
 		return fail(nullptr, TRLDA_ERR_CUDA, std::string("CUDA error: ") + cudaGetErrorString(e));
 	return TRLDA_OK;
