@@ -170,6 +170,16 @@ TRLDA_API int trlda_lower_bound(trlda_model* m, const trlda_docs* docs, const do
                       int64_t latents_cols, const trlda_params* params, int64_t num_documents,
                       double* bound_out, double* per_doc_out);
 
+/* Document-completion predictive log-likelihood (Hoffman et al. 2013, §5); no reference counterpart.
+ * Fits gamma on `observed` (the VI E-step, exactly as trlda_update_variables / trlda_lower_bound do: `latents` = initial
+ * gamma or NULL for a fresh draw, params->max_iter_inference / threshold), then scores every pair of `held_out`
+ * (same number of documents, document d of both belongs to the same text).  *total_out = sum over documents of
+ * per_doc_out[d]; *tokens_out = sum of the held-out counts.  Multi-GPU: both CSRs are this rank's shard; total and
+ * tokens are summed over ranks, per_doc_out (B values, may be NULL) is this rank's. */
+TRLDA_API int trlda_predictive_log_likelihood(trlda_model* m, const trlda_docs* observed, const trlda_docs* held_out,
+        const double* latents, int latents_rows, int64_t latents_cols, const trlda_params* params,
+        double* total_out, int64_t* tokens_out, double* per_doc_out);
+
 /* ---- parity seams ---------------------------------------------------------------------------------------------
  * The reference draws gamma0 (lda.cpp:135) and Cumulative's lambda (cumulativelda.cpp:60) from libc rand()
  * inside updateParameters and offers no way to pass them in.  These two calls install values that the NEXT

@@ -1,3 +1,3 @@
-from trlda_b200.utils import load_documents, load_documents_csr, random_select, sample_dirichlet, polygamma
+from trlda_b200.utils import load_documents, load_documents_csr, random_select, sample_dirichlet, split_documents, polygamma
 
-__all__ = ['load_documents', 'load_documents_csr', 'random_select', 'sample_dirichlet', 'polygamma']
+__all__ = ['load_documents', 'load_documents_csr', 'random_select', 'sample_dirichlet', 'split_documents', 'polygamma']

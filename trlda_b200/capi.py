@@ -105,6 +105,8 @@ PROTOTYPES = {
 	'trlda_select_docs': (C.c_int, [C.c_void_p, C.c_int]),
 	'trlda_update_parameters_resident': (C.c_int, [C.c_void_p, _P(Params), _dbl]),
 	'trlda_lower_bound': (C.c_int, [C.c_void_p, _P(Docs), _dbl, C.c_int, C.c_int64, _P(Params), C.c_int64, _dbl, _dbl]),
+	'trlda_predictive_log_likelihood': (C.c_int, [C.c_void_p, _P(Docs), _P(Docs), _dbl, C.c_int, C.c_int64, _P(Params), _dbl,
+		_P(C.c_int64), _dbl]),
 	'trlda_inject_initial_gamma': (C.c_int, [C.c_void_p, _dbl, C.c_int, C.c_int64]),
 	'trlda_inject_initial_lambda': (C.c_int, [C.c_void_p, _dbl, C.c_int, C.c_int]),
 	'trlda_comm_unique_id': (C.c_int, [C.c_void_p]),
@@ -358,6 +360,21 @@ class Model(object):
 			self.h, C.byref(docs.c), _dptr(latents), rows, cols, C.byref(params), int(num_documents),
 			C.byref(total), _dptr(per_doc)))
 		return total.value, per_doc
+
+	def predictive_log_likelihood(self, docs, held_out, latents=None, max_iter=100, threshold=.001):
+		"""document-completion predictive log-likelihood: gamma is fitted on `docs`, the pairs of `held_out` are scored;
+		returns (total, tokens, per_doc)"""
+		params = default_params(max_iter_inference=max_iter, threshold=threshold)
+		rows, cols = 0, 0
+		if latents is not None:
+			latents = _fortran(latents)
+			rows, cols = latents.shape
+		total, tokens = C.c_double(0.), C.c_int64(0)
+		per_doc = np.empty(docs.num_docs)
+		self._check(self._lib.trlda_predictive_log_likelihood(
+			self.h, C.byref(docs.c), C.byref(held_out.c), _dptr(latents), rows, cols, C.byref(params),
+			C.byref(total), C.byref(tokens), _dptr(per_doc)))
+		return total.value, tokens.value, per_doc
 
 	# ---- multi-GPU / instrumentation --------------------------------------------------------------------------------
 	def comm_init(self, unique_id, rank, nranks):

@@ -1600,6 +1600,76 @@ void launch_elbo_beta(const double* lambda, const double* psi_rows, int K, int V
 }
 
 // ------------------------------------------------------------------------------------------------------------
+// document-completion predictive log-likelihood (Hoffman, Blei, Wang & Paisley 2013, section 5)
+// ------------------------------------------------------------------------------------------------------------
+// One CTA per document.  s_d = gamma_d / rows goes to shared memory; warp w then takes the groups of HELDOUT_GROUP
+// consecutive held-out pairs g = w, w + nw, ... and walks their lambda columns side by side, so that every lane has
+// HELDOUT_GROUP independent loads in flight per step (a lane walking one column at a time is bound by L2 latency).
+// Each dot product is reduced with xor shuffles, which leave the same bits in every lane; the warp partials are added in
+// warp order.  The result of a document therefore depends on K alone (through the block size), not on the launch.
+constexpr int HELDOUT_GROUP = 4;
+
+__global__ void __launch_bounds__(256) k_heldout_loglik(DeviceDocs docs, int K, const double* __restrict__ lambda,
+                                                        const double* __restrict__ rows, const double* __restrict__ gamma,
+                                                        double* __restrict__ per_doc) {
+	extern __shared__ double s[];   // K
+	__shared__ double scratch[32], partial[32];
+	const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
+	for(int64_t d = blockIdx.x; d < docs.B; d += gridDim.x) {
+		const double* g = gamma + d * K;
+		double local = 0.0;
+		for(int k = threadIdx.x; k < K; k += blockDim.x) {
+			const double v = g[k];
+			s[k] = v / rows[k];
+			local += v;
+		}
+		const double log_gsum = log(block_sum(local, scratch));   // the barriers of block_sum also publish s
+		const int64_t end = docs.doc_ptr[d + 1];
+		double acc = 0.0;
+		for(int64_t j0 = docs.doc_ptr[d] + (int64_t) warp * HELDOUT_GROUP; j0 < end; j0 += (int64_t) nw * HELDOUT_GROUP) {
+			const double* col[HELDOUT_GROUP];
+			double dot[HELDOUT_GROUP];
+			#pragma unroll
+			for(int p = 0; p < HELDOUT_GROUP; ++p) {
+				// a slot past the document's end re-reads the group's first column and is not counted
+				col[p] = lambda + (int64_t) docs.word_ids[j0 + p < end ? j0 + p : j0] * K;
+				dot[p] = 0.0;
+			}
+			#pragma unroll 2
+			for(int k = lane; k < K; k += 32) {
+				const double sk = s[k];
+				#pragma unroll
+				for(int p = 0; p < HELDOUT_GROUP; ++p)
+					dot[p] = fma(sk, __ldg(col[p] + k), dot[p]);
+			}
+			#pragma unroll
+			for(int p = 0; p < HELDOUT_GROUP; ++p) {
+				const double total = warp_sum(dot[p]);
+				if(j0 + p < end)
+					acc += docs.counts[j0 + p] * (log(total) - log_gsum);
+			}
+		}
+		if(lane == 0)
+			partial[warp] = acc;
+		__syncthreads();   // also: every warp is done with s before the next document overwrites it
+		if(threadIdx.x == 0) {
+			double total = 0.0;
+			for(int i = 0; i < nw; ++i)
+				total += partial[i];
+			per_doc[d] = total;
+		}
+	}
+}
+
+void launch_heldout_loglik(const DeviceDocs& held_out, int K, const double* lambda, const double* rows, const double* gamma,
+                           double* per_doc, cudaStream_t s) {
+	if(held_out.B == 0)
+		return;
+	k_heldout_loglik<<<(unsigned) std::min<int64_t>(held_out.B, sm_count() * 8), block_for_k(K), (size_t) K * 8, s>>>(
+		held_out, K, lambda, rows, gamma, per_doc);
+}
+
+// ------------------------------------------------------------------------------------------------------------
 // special-function test hook
 // ------------------------------------------------------------------------------------------------------------
 __global__ void k_special(int which, const double* __restrict__ x, int64_t n, double* __restrict__ out) {

@@ -230,6 +230,10 @@ void launch_elbo_docs(const DeviceDocs& docs, int K, const double* lambda, const
 // partial[w] = sum_k (eta - lambda_kw)(psi(lambda_kw) - psi_rows_k) + lgamma(lambda_kw)
 void launch_elbo_beta(const double* lambda, const double* psi_rows, int K, int V, double eta, double* partial,
                       cudaStream_t s);
+// document-completion predictive log-likelihood: per_doc[d] = sum_j c_j (log sum_k s_dk lambda_{k,w_j} - log sum_k gamma_dk)
+// over the pairs of `held_out` (CSR arrays only), s_dk = gamma_dk / rows_k; lambda K x V and rows K are fp64
+void launch_heldout_loglik(const DeviceDocs& held_out, int K, const double* lambda, const double* rows, const double* gamma,
+                           double* per_doc, cudaStream_t s);
 // out[k] = lgamma(in[k])
 void launch_lgamma_vector(const double* in, int K, double* out, cudaStream_t s);
 

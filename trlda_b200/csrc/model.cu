@@ -268,6 +268,7 @@ struct trlda_model {
 	// per-minibatch E-step buffers
 	DevBuf gamma, etheta, etheta32, weight, doc_stat, iterations, wordcount;
 	DevBuf gibbs_occ, gibbs_topics;            // Gibbs E-step scratch: occurrences before each document, one topic per occurrence
+	DevBuf ho_doc_ptr, ho_word_ids, ho_counts; // held-out CSR of trlda_predictive_log_likelihood
 	bool gamma_valid = false;
 
 	// parity seams
@@ -2201,6 +2202,103 @@ int trlda_lower_bound(trlda_model* m, const trlda_docs* docs, const double* late
 	beta_terms += m->K * lgamma(m->V * m->eta) - h[2];                          // :356
 	if(bound_out)
 		*bound_out = beta_terms + factor * h[0];
+	if(per_doc_out && B) {
+		CUDA_TRY(m, cudaMemcpy(per_doc_out, per_doc, sizeof(double) * B, cudaMemcpyDeviceToHost));
+		m->stats.d2h_bytes += sizeof(double) * B;
+	}
+	consume_injections(m);
+	return TRLDA_OK;
+}
+
+// checks the held-out CSR like upload_docs does, sums its counts and copies it into the model's held-out buffers
+static int upload_held_out(trlda_model* m, const trlda_docs* docs, DeviceDocs* out, int64_t* tokens) {
+	if(!docs || docs->num_docs < 0 || (docs->num_docs > 0 && !docs->doc_ptr))
+		return fail(m, TRLDA_ERR_ARG, "Documents must be given in CSR form.");
+	const int64_t B = docs->num_docs;
+	const int64_t N = B ? docs->doc_ptr[B] : 0;
+	if(B && docs->doc_ptr[0] != 0)
+		return fail(m, TRLDA_ERR_ARG, "Document offsets must start at zero.");
+	if(N < 0 || N > INT32_MAX)
+		return fail(m, TRLDA_ERR_ARG, "Too many (word, count) pairs in one minibatch.");
+	if(N > 0 && (!docs->word_ids || !docs->counts))
+		return fail(m, TRLDA_ERR_ARG, "Documents must be given in CSR form.");
+	for(int64_t d = 0; d < B; ++d)
+		if(docs->doc_ptr[d + 1] < docs->doc_ptr[d])
+			return fail(m, TRLDA_ERR_ARG, "Document offsets must be non-decreasing.");
+	int64_t total = 0;
+	int bad = 0;
+	for(int64_t i = 0; i < N; ++i) {
+		total += docs->counts[i];
+		bad |= (docs->word_ids[i] < 0) | (docs->word_ids[i] >= m->V) | ((docs->counts[i] < 0) << 1);
+	}
+	if(bad & 2)
+		return fail(m, TRLDA_ERR_ARG, "Word counts should not be negative.");
+	if(bad)
+		return fail(m, TRLDA_ERR_ARG, "Word ID out of range.");
+	CUDA_TRY(m, m->ho_doc_ptr.ensure(sizeof(int64_t) * (B + 1)));
+	CUDA_TRY(m, m->ho_word_ids.ensure(sizeof(int32_t) * std::max<int64_t>(N, 1)));
+	CUDA_TRY(m, m->ho_counts.ensure(sizeof(int32_t) * std::max<int64_t>(N, 1)));
+	if(B)
+		CUDA_TRY(m, cudaMemcpyAsync(m->ho_doc_ptr.p, docs->doc_ptr, sizeof(int64_t) * (B + 1), cudaMemcpyHostToDevice, m->stream));
+	if(N) {
+		CUDA_TRY(m, cudaMemcpyAsync(m->ho_word_ids.p, docs->word_ids, sizeof(int32_t) * N, cudaMemcpyHostToDevice, m->stream));
+		CUDA_TRY(m, cudaMemcpyAsync(m->ho_counts.p, docs->counts, sizeof(int32_t) * N, cudaMemcpyHostToDevice, m->stream));
+	}
+	m->stats.h2d_bytes += (B ? sizeof(int64_t) * (B + 1) : 0) + sizeof(int32_t) * 2 * N;
+	out->B = B;
+	out->N = N;
+	out->doc_ptr = m->ho_doc_ptr.as<int64_t>();
+	out->word_ids = m->ho_word_ids.as<int32_t>();
+	out->counts = m->ho_counts.as<int32_t>();
+	*tokens = total;
+	return TRLDA_OK;
+}
+
+int trlda_predictive_log_likelihood(trlda_model* m, const trlda_docs* observed, const trlda_docs* held_out, const double* latents,
+                                    int latents_rows, int64_t latents_cols, const trlda_params* params, double* total_out,
+                                    int64_t* tokens_out, double* per_doc_out) {
+	std::lock_guard<std::recursive_mutex> lock__(m->mu);
+	if(params->inference_method != TRLDA_INFERENCE_VI)
+		return fail(m, TRLDA_ERR_UNSUPPORTED, "Only variational inference ('VI') is implemented on the device.");
+	if(m->lambda_sharded)
+		return fail(m, TRLDA_ERR_UNSUPPORTED, "predictive_log_likelihood: lambda is sharded over ranks.");
+	if(!observed || !held_out)
+		return fail(m, TRLDA_ERR_ARG, "Documents must be given in CSR form.");
+	if(latents && (latents_rows != m->K || latents_cols != observed->num_docs))
+		return fail(m, TRLDA_ERR_ARG, "Initial gamma has wrong dimensionality.");
+	if(held_out->num_docs != observed->num_docs)
+		return fail(m, TRLDA_ERR_ARG, "Observed and held-out documents differ in number.");
+	TRY(set_device(m));
+	DeviceDocs ho;
+	int64_t tokens = 0;
+	TRY(upload_held_out(m, held_out, &ho, &tokens));
+	// gamma of the observed part: the E-step of trlda_update_variables / trlda_lower_bound, with every route it has
+	TRY(upload_docs(m, observed));
+	TRY(prepare_beta(m));                                                      // also leaves rows = row sums of lambda
+	TRY(run_estep(m, latents ? GAMMA_HOST : GAMMA_FRESH, latents, params->max_iter_inference, params->threshold));
+	const int64_t B = m->mb.docs.B;
+	double* per_doc = m->doc_stat.as<double>();                                // free after the E-step; holds >= B values
+	double* sc = m->scalars.as<double>();
+	{
+		Launch l(m, KK_ELBO);
+		launch_heldout_loglik(ho, m->K, m->lambda(), m->rows.as<double>(), m->gamma.as<double>(), per_doc, m->stream);
+	}
+	{
+		Launch l(m, KK_REDUCE);
+		launch_sum(per_doc, B, sc + 16, sc, m->stream);
+	}
+	TRY(check_launch(m, "heldout_loglik"));
+	// the local total and token count, summed over ranks in one exchange (counts are exact in a double below 2^53)
+	double* h = m->readback.as<double>();
+	h[0] = (double) tokens;
+	CUDA_TRY(m, cudaMemcpyAsync(sc + 1, h, sizeof(double), cudaMemcpyHostToDevice, m->stream));
+	TRY(allreduce(m, sc, 2, ncclDouble));
+	double r[2];
+	TRY(read_back(m, sc, 2, r));
+	if(total_out)
+		*total_out = r[0];
+	if(tokens_out)
+		*tokens_out = (int64_t) r[1];
 	if(per_doc_out && B) {
 		CUDA_TRY(m, cudaMemcpy(per_doc_out, per_doc, sizeof(double) * B, cudaMemcpyDeviceToHost));
 		m->stats.d2h_bytes += sizeof(double) * B;

@@ -585,6 +585,38 @@ PyObject* LDA_lower_bound(LDAObject* self, PyObject* args, PyObject* kwds) {
 	return PyFloat_FromDouble(bound);
 }
 
+// predictive_log_likelihood (no reference counterpart): document completion, trlda_predictive_log_likelihood
+PyObject* LDA_predictive_log_likelihood(LDAObject* self, PyObject* args, PyObject* kwds) {
+	REQUIRE_MODEL(self, nullptr);
+	const char* kwlist[] = {"docs", "held_out", "latents", "max_iter", nullptr};
+	Documents documents, held_out;
+	trlda_params params;
+	trlda_params_default(&params);
+	PyObject* latents = nullptr;
+	if(!PyArg_ParseTupleAndKeywords(args, kwds, "O&O&|Oi", const_cast<char**>(kwlist), &docs_converter, &documents,
+			&docs_converter, &held_out, &latents, &params.max_iter_inference))
+		return nullptr;
+	npy_intp rows = 0, cols = 0;
+	PyObject* latents_arr = nullptr;
+	if(latents && latents != Py_None) {
+		latents_arr = as_farray(latents, &rows, &cols, "`latents`");
+		if(!latents_arr)
+			return nullptr;
+	}
+	int status;
+	double total = 0.;
+	int64_t tokens = 0;
+	const double* l = latents_arr ? static_cast<const double*>(PyArray_DATA((PyArrayObject*) latents_arr)) : nullptr;
+	Py_BEGIN_ALLOW_THREADS
+	status = trlda_predictive_log_likelihood(self->m, &documents.view, &held_out.view, l, (int) rows, (int64_t) cols, &params,
+	                                         &total, &tokens, nullptr);
+	Py_END_ALLOW_THREADS
+	Py_XDECREF(latents_arr);
+	if(status != TRLDA_OK)
+		return raise_status(self->m, status);
+	return Py_BuildValue("(dL)", total, (long long) tokens);
+}
+
 PyObject* LDA_str(PyObject* self_) {                                      // ldainterface.cpp:473-490
 	LDAObject* self = (LDAObject*) self_;
 	REQUIRE_MODEL(self, nullptr);
@@ -864,6 +896,17 @@ const char* update_variables_doc =
 	"Computes beliefs over topic assignments for the given documents (E-step) on the GPU.  Returns a tuple of the\n"
 	"K x N Dirichlet parameters gamma and the K x W sufficient statistics (float64, Fortran order).";
 
+const char* predictive_log_likelihood_doc =
+	"predictive_log_likelihood(docs, held_out, latents=None, max_iter=100)\n\n"
+	"Document-completion predictive log-likelihood (Hoffman, Blei, Wang & Paisley 2013, section 5) on the GPU.  gamma is\n"
+	"fitted on `docs` (the observed part of each document, the E-step of update_variables; `latents` is the initial\n"
+	"gamma, a fresh draw if None), then every held-out token w of document d is scored with\n"
+	"log sum_k E[theta_dk] E[beta_kw].  `held_out` has one document for each of `docs`, and both take the list or the\n"
+	"(doc_ptr, word_ids, counts) form; trlda.utils.split_documents makes such a pair.  Returns the tuple\n"
+	"(log_likelihood, num_tokens): the summed log-likelihood and the number of held-out tokens.  The per-word figure is\n"
+	"log_likelihood / num_tokens and the perplexity exp(-log_likelihood / num_tokens); returning the pair lets batches\n"
+	"of held-out documents be added up.  The model's parameters are not changed.";
+
 PyGetSetDef LDA_getset[] = {
 	{"num_topics", (getter) LDA_num_topics, nullptr, "Number of topics.", nullptr},
 	{"num_words", (getter) LDA_num_words, nullptr, "Number of words.", nullptr},
@@ -880,6 +923,8 @@ PyMethodDef LDA_methods[] = {
 	{"do_e_step", (PyCFunction) LDA_update_variables, METH_VARARGS | METH_KEYWORDS, update_variables_doc},   // module.cpp:99-106
 	{"lower_bound", (PyCFunction) LDA_lower_bound, METH_VARARGS | METH_KEYWORDS,
 		"lower_bound(docs, num_documents=-1, inference_method='VI', max_iter=100, num_samples=1, burn_in=2)"},
+	{"predictive_log_likelihood", (PyCFunction) LDA_predictive_log_likelihood, METH_VARARGS | METH_KEYWORDS,
+		predictive_log_likelihood_doc},
 	{nullptr, nullptr, 0, nullptr}};
 
 PyGetSetDef OnlineLDA_getset[] = {

@@ -2,7 +2,7 @@
 
 `load_users` / `load_users_as_dict` (collaborative-filtering loaders) are outside the scope of this build."""
 from .load_documents import load_documents, load_documents_csr
-from .._sample import random_select, sample_dirichlet
+from .._sample import random_select, sample_dirichlet, split_documents
 
 
 def polygamma(n, x):
@@ -11,4 +11,4 @@ def polygamma(n, x):
 	return _trlda.polygamma(n, x)
 
 
-__all__ = ['load_documents', 'load_documents_csr', 'random_select', 'sample_dirichlet', 'polygamma']
+__all__ = ['load_documents', 'load_documents_csr', 'random_select', 'sample_dirichlet', 'split_documents', 'polygamma']
