@@ -180,6 +180,19 @@ TRLDA_API int trlda_predictive_log_likelihood(trlda_model* m, const trlda_docs* 
         const double* latents, int latents_rows, int64_t latents_cols, const trlda_params* params,
         double* total_out, int64_t* tokens_out, double* per_doc_out);
 
+/* The n most probable words of every topic, in the order of E[beta_kw] = lambda_kw / sum_w lambda_kw: descending,
+ * ties broken by the smaller word id.  ids_out is n x K column-major (topic k's list at ids_out + k*n, rank order);
+ * prob_out (may be NULL) receives the matching E[beta_kw].  1 <= n <= min(32, V).  No reference counterpart. */
+TRLDA_API int trlda_top_words(trlda_model* m, int n, int32_t* ids_out, double* prob_out);
+
+/* For every topic k and ranks i, j < n of its list ids[k*n ..]: counts_out[(k*n + j)*n + i] = number of documents of
+ * `docs` that contain both word ids[k*n+i] and word ids[k*n+j] (the diagonal: documents containing the word).
+ * A word is contained in a document when one of its pairs there has a count > 0; duplicate ids count once.
+ * *num_docs_out = number of documents (empty ones included).  Multi-GPU: `docs` is this rank's shard; counts and
+ * num_docs are summed over ranks.  ids is n x K like trlda_top_words' output; 1 <= n <= 32.  No reference counterpart. */
+TRLDA_API int trlda_cooccurrence(trlda_model* m, const trlda_docs* docs, const int32_t* ids, int n,
+                                 int64_t* counts_out, int64_t* num_docs_out);
+
 /* ---- parity seams ---------------------------------------------------------------------------------------------
  * The reference draws gamma0 (lda.cpp:135) and Cumulative's lambda (cumulativelda.cpp:60) from libc rand()
  * inside updateParameters and offers no way to pass them in.  These two calls install values that the NEXT

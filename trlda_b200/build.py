@@ -46,7 +46,7 @@ def build_library(force=False, verbose=False):
 	headers.append(os.path.join(ROOT, 'include', 'trlda_b200.h'))
 	sources = [os.path.join(CSRC, 'kernels.cu'), os.path.join(CSRC, 'estep_stream.cu'),
 		os.path.join(CSRC, 'estep_tmem.cu'), os.path.join(CSRC, 'sample.cu'), os.path.join(CSRC, 'csc.cu'), os.path.join(CSRC, 'ingest.cu'),
-		os.path.join(CSRC, 'model.cu')]
+		os.path.join(CSRC, 'topics.cu'), os.path.join(CSRC, 'model.cu')]
 	objects = []
 	rebuilt = False
 	for src in sources:

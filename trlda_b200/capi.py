@@ -107,6 +107,8 @@ PROTOTYPES = {
 	'trlda_lower_bound': (C.c_int, [C.c_void_p, _P(Docs), _dbl, C.c_int, C.c_int64, _P(Params), C.c_int64, _dbl, _dbl]),
 	'trlda_predictive_log_likelihood': (C.c_int, [C.c_void_p, _P(Docs), _P(Docs), _dbl, C.c_int, C.c_int64, _P(Params), _dbl,
 		_P(C.c_int64), _dbl]),
+	'trlda_top_words': (C.c_int, [C.c_void_p, C.c_int, _P(C.c_int32), _dbl]),
+	'trlda_cooccurrence': (C.c_int, [C.c_void_p, _P(Docs), _P(C.c_int32), C.c_int, _P(C.c_int64), _P(C.c_int64)]),
 	'trlda_inject_initial_gamma': (C.c_int, [C.c_void_p, _dbl, C.c_int, C.c_int64]),
 	'trlda_inject_initial_lambda': (C.c_int, [C.c_void_p, _dbl, C.c_int, C.c_int]),
 	'trlda_comm_unique_id': (C.c_int, [C.c_void_p]),
@@ -375,6 +377,26 @@ class Model(object):
 			self.h, C.byref(docs.c), C.byref(held_out.c), _dptr(latents), rows, cols, C.byref(params),
 			C.byref(total), C.byref(tokens), _dptr(per_doc)))
 		return total.value, tokens.value, per_doc
+
+	def top_words(self, n=10):
+		"""the n most probable words of every topic: (ids[K, n] int32, probs[K, n]), each row in rank order"""
+		ids = np.empty((self.K, max(int(n), 0)), dtype=np.int32)
+		probs = np.empty((self.K, max(int(n), 0)))
+		self._check(self._lib.trlda_top_words(self.h, int(n), ids.ctypes.data_as(_P(C.c_int32)), _dptr(probs)))
+		return ids, probs
+
+	def cooccurrence(self, docs, ids):
+		"""document frequencies of the words of `ids` (K x n, e.g. top_words' ids): (counts[K, n, n] int64, num_docs) with
+		counts[k, i, j] = documents of `docs` that contain both ids[k, i] and ids[k, j]"""
+		ids = np.ascontiguousarray(ids, dtype=np.int32)
+		if ids.ndim != 2 or ids.shape[0] != self.K:
+			raise ValueError('ids must be a K x n array')
+		n = ids.shape[1]
+		counts = np.empty((self.K, n, n), dtype=np.int64)
+		num_docs = C.c_int64(0)
+		self._check(self._lib.trlda_cooccurrence(self.h, C.byref(docs.c), ids.ctypes.data_as(_P(C.c_int32)), n,
+			counts.ctypes.data_as(_P(C.c_int64)), C.byref(num_docs)))
+		return counts, num_docs.value
 
 	# ---- multi-GPU / instrumentation --------------------------------------------------------------------------------
 	def comm_init(self, unique_id, rank, nranks):

@@ -234,6 +234,20 @@ void launch_elbo_beta(const double* lambda, const double* psi_rows, int K, int V
 // over the pairs of `held_out` (CSR arrays only), s_dk = gamma_dk / rows_k; lambda K x V and rows K are fp64
 void launch_heldout_loglik(const DeviceDocs& held_out, int K, const double* lambda, const double* rows, const double* gamma,
                            double* per_doc, cudaStream_t s);
+// topics.cu: the n (<= 32) most probable words of every topic of lambda (K x V, fp64), ordered by value descending, then
+// word id ascending.  The candidate pass cuts the words into top_words_chunks(K, V, n) chunks and writes every chunk's
+// best n of every topic to cand_v / cand_id (chunks x K x n); the merge pass writes topic k's list to ids + k*n and
+// lambda_kw / rows_k to prob + k*n.
+int top_words_chunks(int K, int V, int n);
+void launch_top_words_candidates(const double* lambda, int K, int V, int n, int chunks, double* cand_v, int32_t* cand_id,
+                                 cudaStream_t s);
+void launch_top_words_merge(const double* cand_v, const int32_t* cand_id, const double* rows, int K, int n, int chunks,
+                            int32_t* ids, double* prob, cudaStream_t s);
+// counts[(k n + j) n + i] += number of documents of `docs` (CSR arrays only) holding both the words of ranks i and j of topic
+// k's list (a pair counts when its count is > 0).  map_ptr (V + 1) / map_entry: for word w, the entries topic * 32 + rank
+// of the lists it is on, at map_entry[map_ptr[w] .. map_ptr[w + 1])
+void launch_cooccurrence(const DeviceDocs& docs, int K, int n, const int32_t* map_ptr, const int32_t* map_entry,
+                         unsigned long long* counts, cudaStream_t s);
 // out[k] = lgamma(in[k])
 void launch_lgamma_vector(const double* in, int K, double* out, cudaStream_t s);
 

@@ -268,7 +268,12 @@ struct trlda_model {
 	// per-minibatch E-step buffers
 	DevBuf gamma, etheta, etheta32, weight, doc_stat, iterations, wordcount;
 	DevBuf gibbs_occ, gibbs_topics;            // Gibbs E-step scratch: occurrences before each document, one topic per occurrence
-	DevBuf ho_doc_ptr, ho_word_ids, ho_counts; // held-out CSR of trlda_predictive_log_likelihood
+	// side CSR of the evaluation calls (the held-out part of trlda_predictive_log_likelihood, the corpus of
+	// trlda_cooccurrence): it never replaces the live minibatch
+	DevBuf ho_doc_ptr, ho_word_ids, ho_counts;
+	// trlda_top_words: row sums of lambda, the per-chunk candidate lists and the result; trlda_cooccurrence: the inverse map
+	// of the top words and the counters
+	DevBuf topic_rows, top_cand_v, top_cand_id, top_ids, top_prob, co_map_ptr, co_map, co_counts;
 	bool gamma_valid = false;
 
 	// parity seams
@@ -2210,8 +2215,9 @@ int trlda_lower_bound(trlda_model* m, const trlda_docs* docs, const double* late
 	return TRLDA_OK;
 }
 
-// checks the held-out CSR like upload_docs does, sums its counts and copies it into the model's held-out buffers
-static int upload_held_out(trlda_model* m, const trlda_docs* docs, DeviceDocs* out, int64_t* tokens) {
+// checks a CSR like upload_docs does, sums its counts and copies it into the model's side buffers (ho_*), leaving the live
+// minibatch alone
+static int upload_side_docs(trlda_model* m, const trlda_docs* docs, DeviceDocs* out, int64_t* tokens) {
 	if(!docs || docs->num_docs < 0 || (docs->num_docs > 0 && !docs->doc_ptr))
 		return fail(m, TRLDA_ERR_ARG, "Documents must be given in CSR form.");
 	const int64_t B = docs->num_docs;
@@ -2271,7 +2277,7 @@ int trlda_predictive_log_likelihood(trlda_model* m, const trlda_docs* observed, 
 	TRY(set_device(m));
 	DeviceDocs ho;
 	int64_t tokens = 0;
-	TRY(upload_held_out(m, held_out, &ho, &tokens));
+	TRY(upload_side_docs(m, held_out, &ho, &tokens));
 	// gamma of the observed part: the E-step of trlda_update_variables / trlda_lower_bound, with every route it has
 	TRY(upload_docs(m, observed));
 	TRY(prepare_beta(m));                                                      // also leaves rows = row sums of lambda
@@ -2304,6 +2310,105 @@ int trlda_predictive_log_likelihood(trlda_model* m, const trlda_docs* observed, 
 		m->stats.d2h_bytes += sizeof(double) * B;
 	}
 	consume_injections(m);
+	return TRLDA_OK;
+}
+
+static const int kMaxTopWords = 32;   // one 32-bit mask per topic in k_cooccurrence, one warp lane per rank in the merge
+
+int trlda_top_words(trlda_model* m, int n, int32_t* ids_out, double* prob_out) {
+	std::lock_guard<std::recursive_mutex> lock__(m->mu);
+	if(n < 1 || n > kMaxTopWords || n > m->V)
+		return fail(m, TRLDA_ERR_ARG, "Number of top words must lie in [1, min(32, number of words)].");
+	if(!ids_out)
+		return fail(m, TRLDA_ERR_ARG, "top_words: no output buffer.");
+	if(m->lambda_sharded)
+		return fail(m, TRLDA_ERR_UNSUPPORTED, "top_words: lambda is sharded over ranks.");
+	TRY(set_device(m));
+	const int K = m->K, V = m->V, chunks = top_words_chunks(K, V, n);
+	const size_t listed = (size_t) K * n, cands = (size_t) chunks * listed;
+	CUDA_TRY(m, m->topic_rows.ensure(sizeof(double) * K));
+	CUDA_TRY(m, m->top_cand_v.ensure(sizeof(double) * cands));
+	CUDA_TRY(m, m->top_cand_id.ensure(sizeof(int32_t) * cands));
+	CUDA_TRY(m, m->top_ids.ensure(sizeof(int32_t) * listed));
+	CUDA_TRY(m, m->top_prob.ensure(sizeof(double) * listed));
+	TRY(compute_rows(m, m->lambda(), m->topic_rows.as<double>()));   // the row sums prepare_beta uses
+	{
+		Launch l(m, KK_MISC);
+		launch_top_words_candidates(m->lambda(), K, V, n, chunks, m->top_cand_v.as<double>(), m->top_cand_id.as<int32_t>(), m->stream);
+	}
+	{
+		Launch l(m, KK_MISC);
+		launch_top_words_merge(m->top_cand_v.as<double>(), m->top_cand_id.as<int32_t>(), m->topic_rows.as<double>(), K, n, chunks,
+		                       m->top_ids.as<int32_t>(), m->top_prob.as<double>(), m->stream);
+	}
+	TRY(check_launch(m, "top_words"));
+	CUDA_TRY(m, cudaMemcpyAsync(ids_out, m->top_ids.p, sizeof(int32_t) * listed, cudaMemcpyDeviceToHost, m->stream));
+	if(prob_out)
+		CUDA_TRY(m, cudaMemcpyAsync(prob_out, m->top_prob.p, sizeof(double) * listed, cudaMemcpyDeviceToHost, m->stream));
+	CUDA_TRY(m, cudaStreamSynchronize(m->stream));
+	m->stats.d2h_bytes += (sizeof(int32_t) + (prob_out ? sizeof(double) : 0)) * listed;
+	return TRLDA_OK;
+}
+
+int trlda_cooccurrence(trlda_model* m, const trlda_docs* docs, const int32_t* ids, int n, int64_t* counts_out,
+                       int64_t* num_docs_out) {
+	std::lock_guard<std::recursive_mutex> lock__(m->mu);
+	if(n < 1 || n > kMaxTopWords)
+		return fail(m, TRLDA_ERR_ARG, "Number of top words must lie in [1, min(32, number of words)].");
+	if(!ids || !counts_out)
+		return fail(m, TRLDA_ERR_ARG, "cooccurrence: no top words or no output buffer.");
+	const int K = m->K, V = m->V;
+	// the inverse map: for every word, the (topic * 32 + rank) entries of the lists it is on
+	std::vector<int32_t> map_ptr((size_t) V + 1, 0), map((size_t) K * n);
+	for(int k = 0; k < K; ++k) {
+		const int32_t* list = ids + (size_t) k * n;
+		for(int i = 0; i < n; ++i) {
+			if(list[i] < 0 || list[i] >= V)
+				return fail(m, TRLDA_ERR_ARG, "Word ID out of range.");
+			for(int j = 0; j < i; ++j)
+				if(list[j] == list[i])
+					return fail(m, TRLDA_ERR_ARG, "Top words of a topic must be distinct.");
+			++map_ptr[(size_t) list[i] + 1];
+		}
+	}
+	for(int w = 0; w < V; ++w)
+		map_ptr[(size_t) w + 1] += map_ptr[w];
+	{
+		std::vector<int32_t> next(map_ptr.begin(), map_ptr.end() - 1);
+		for(int k = 0; k < K; ++k)
+			for(int i = 0; i < n; ++i)
+				map[next[ids[(size_t) k * n + i]]++] = k * kMaxTopWords + i;
+	}
+	TRY(set_device(m));
+	TRY(ensure_small(m));
+	DeviceDocs d;
+	int64_t tokens = 0;
+	TRY(upload_side_docs(m, docs, &d, &tokens));
+	const size_t cells = (size_t) K * n * n;
+	CUDA_TRY(m, m->co_map_ptr.ensure(sizeof(int32_t) * map_ptr.size()));
+	CUDA_TRY(m, m->co_map.ensure(sizeof(int32_t) * map.size()));
+	CUDA_TRY(m, m->co_counts.ensure(sizeof(int64_t) * (cells + 1)));    // the counters, then the document count
+	CUDA_TRY(m, cudaMemcpyAsync(m->co_map_ptr.p, map_ptr.data(), sizeof(int32_t) * map_ptr.size(), cudaMemcpyHostToDevice, m->stream));
+	CUDA_TRY(m, cudaMemcpyAsync(m->co_map.p, map.data(), sizeof(int32_t) * map.size(), cudaMemcpyHostToDevice, m->stream));
+	m->stats.h2d_bytes += sizeof(int32_t) * (map_ptr.size() + map.size());
+	CUDA_TRY(m, cudaMemsetAsync(m->co_counts.p, 0, sizeof(int64_t) * cells, m->stream));
+	int64_t* h = m->readback.as<int64_t>();
+	h[0] = d.B;
+	CUDA_TRY(m, cudaMemcpyAsync(m->co_counts.as<int64_t>() + cells, h, sizeof(int64_t), cudaMemcpyHostToDevice, m->stream));
+	{
+		Launch l(m, KK_MISC);
+		launch_cooccurrence(d, K, n, m->co_map_ptr.as<int32_t>(), m->co_map.as<int32_t>(),
+		                    reinterpret_cast<unsigned long long*>(m->co_counts.p), m->stream);
+	}
+	TRY(check_launch(m, "cooccurrence"));
+	// counters and document count summed over ranks in one exchange; integers, so the sum is exact in any order
+	TRY(allreduce(m, m->co_counts.p, cells + 1, ncclInt64));
+	CUDA_TRY(m, cudaMemcpyAsync(counts_out, m->co_counts.p, sizeof(int64_t) * cells, cudaMemcpyDeviceToHost, m->stream));
+	CUDA_TRY(m, cudaMemcpyAsync(h, m->co_counts.as<int64_t>() + cells, sizeof(int64_t), cudaMemcpyDeviceToHost, m->stream));
+	CUDA_TRY(m, cudaStreamSynchronize(m->stream));   // also: the host vectors of the inverse map outlive their copies
+	m->stats.d2h_bytes += sizeof(int64_t) * (cells + 1);
+	if(num_docs_out)
+		*num_docs_out = h[0];
 	return TRLDA_OK;
 }
 

@@ -617,6 +617,81 @@ PyObject* LDA_predictive_log_likelihood(LDAObject* self, PyObject* args, PyObjec
 	return Py_BuildValue("(dL)", total, (long long) tokens);
 }
 
+// top_words (no reference counterpart): trlda_top_words
+PyObject* LDA_top_words(LDAObject* self, PyObject* args, PyObject* kwds) {
+	REQUIRE_MODEL(self, nullptr);
+	const char* kwlist[] = {"num_words", nullptr};
+	int n = 10;
+	if(!PyArg_ParseTupleAndKeywords(args, kwds, "|i", const_cast<char**>(kwlist), &n))
+		return nullptr;
+	npy_intp dims[2] = {trlda_num_topics(self->m), std::max(n, 0)};
+	PyObject* ids = PyArray_SimpleNew(2, dims, NPY_INT32);
+	PyObject* probs = ids ? PyArray_SimpleNew(2, dims, NPY_DOUBLE) : nullptr;
+	if(!probs) {
+		Py_XDECREF(ids);
+		return nullptr;
+	}
+	int status;
+	int32_t* i = static_cast<int32_t*>(PyArray_DATA((PyArrayObject*) ids));
+	double* p = static_cast<double*>(PyArray_DATA((PyArrayObject*) probs));
+	Py_BEGIN_ALLOW_THREADS
+	status = trlda_top_words(self->m, n, i, p);
+	Py_END_ALLOW_THREADS
+	if(status != TRLDA_OK) {
+		Py_DECREF(ids);
+		Py_DECREF(probs);
+		return raise_status(self->m, status);
+	}
+	PyObject* result = Py_BuildValue("(OO)", ids, probs);
+	Py_DECREF(ids);
+	Py_DECREF(probs);
+	return result;
+}
+
+// cooccurrence (no reference counterpart): trlda_cooccurrence
+PyObject* LDA_cooccurrence(LDAObject* self, PyObject* args, PyObject* kwds) {
+	REQUIRE_MODEL(self, nullptr);
+	const char* kwlist[] = {"docs", "top_words", nullptr};
+	Documents documents;
+	PyObject* top_words = nullptr;
+	if(!PyArg_ParseTupleAndKeywords(args, kwds, "O&O", const_cast<char**>(kwlist), &docs_converter, &documents, &top_words))
+		return nullptr;
+	const int K = trlda_num_topics(self->m);
+	// any integer array: ids beyond int32 become -1, which the library rejects as out of range
+	PyObject* arr = PyArray_FROM_OTF(top_words, NPY_INT64, NPY_ARRAY_IN_ARRAY);
+	if(!arr)
+		return nullptr;
+	PyArrayObject* a = (PyArrayObject*) arr;
+	if(PyArray_NDIM(a) != 2 || PyArray_DIM(a, 0) != K) {
+		Py_DECREF(arr);
+		PyErr_SetString(PyExc_ValueError, "`top_words` should be a num_topics x n array of word IDs.");
+		return nullptr;
+	}
+	const npy_intp n = PyArray_DIM(a, 1);
+	const int64_t* src = static_cast<const int64_t*>(PyArray_DATA(a));
+	std::vector<int32_t> ids((size_t) K * n);
+	for(size_t j = 0; j < ids.size(); ++j)
+		ids[j] = src[j] < INT32_MIN || src[j] > INT32_MAX ? -1 : (int32_t) src[j];
+	Py_DECREF(arr);
+	npy_intp dims[3] = {K, n, n};
+	PyObject* counts = PyArray_SimpleNew(3, dims, NPY_INT64);
+	if(!counts)
+		return nullptr;
+	int status;
+	int64_t num_docs = 0;
+	int64_t* c = static_cast<int64_t*>(PyArray_DATA((PyArrayObject*) counts));
+	Py_BEGIN_ALLOW_THREADS
+	status = trlda_cooccurrence(self->m, &documents.view, ids.data(), (int) std::min<npy_intp>(n, INT32_MAX), c, &num_docs);
+	Py_END_ALLOW_THREADS
+	if(status != TRLDA_OK) {
+		Py_DECREF(counts);
+		return raise_status(self->m, status);
+	}
+	PyObject* result = Py_BuildValue("(OL)", counts, (long long) num_docs);
+	Py_DECREF(counts);
+	return result;
+}
+
 PyObject* LDA_str(PyObject* self_) {                                      // ldainterface.cpp:473-490
 	LDAObject* self = (LDAObject*) self_;
 	REQUIRE_MODEL(self, nullptr);
@@ -907,6 +982,23 @@ const char* predictive_log_likelihood_doc =
 	"log_likelihood / num_tokens and the perplexity exp(-log_likelihood / num_tokens); returning the pair lets batches\n"
 	"of held-out documents be added up.  The model's parameters are not changed.";
 
+const char* top_words_doc =
+	"top_words(num_words=10)\n\n"
+	"The num_words (1 to 32, at most num_words of the model) most probable words of every topic, on the GPU: words ordered\n"
+	"by E[beta_kw] = lambda_kw / sum_w lambda_kw, descending, ties broken by the smaller word id.  Returns the tuple\n"
+	"(ids, probs) of two num_topics x num_words arrays, int32 word ids and their float64 E[beta_kw], each row in rank\n"
+	"order.  Only the lists leave the device, not lambda.";
+
+const char* cooccurrence_doc =
+	"cooccurrence(docs, top_words)\n\n"
+	"Document frequencies of each topic's top words in `docs` (the list or the (doc_ptr, word_ids, counts) form), counted\n"
+	"on the GPU.  `top_words` is a num_topics x n integer array of word IDs (1 <= n <= 32, distinct within a row), e.g.\n"
+	"the ids of top_words().  Returns the tuple (counts, num_docs): counts[k, i, j] is the number of documents that\n"
+	"contain both top_words[k, i] and top_words[k, j] (the diagonal: documents that contain the word), num_docs the\n"
+	"number of documents.  A word is in a document when one of its pairs there has a positive count.  Both are integers,\n"
+	"so the results of several batches of documents can be added up; trlda.utils.topic_coherence does that and turns\n"
+	"them into UMass or NPMI coherence.  The model's parameters are not changed.";
+
 PyGetSetDef LDA_getset[] = {
 	{"num_topics", (getter) LDA_num_topics, nullptr, "Number of topics.", nullptr},
 	{"num_words", (getter) LDA_num_words, nullptr, "Number of words.", nullptr},
@@ -925,6 +1017,8 @@ PyMethodDef LDA_methods[] = {
 		"lower_bound(docs, num_documents=-1, inference_method='VI', max_iter=100, num_samples=1, burn_in=2)"},
 	{"predictive_log_likelihood", (PyCFunction) LDA_predictive_log_likelihood, METH_VARARGS | METH_KEYWORDS,
 		predictive_log_likelihood_doc},
+	{"top_words", (PyCFunction) LDA_top_words, METH_VARARGS | METH_KEYWORDS, top_words_doc},
+	{"cooccurrence", (PyCFunction) LDA_cooccurrence, METH_VARARGS | METH_KEYWORDS, cooccurrence_doc},
 	{nullptr, nullptr, 0, nullptr}};
 
 PyGetSetDef OnlineLDA_getset[] = {

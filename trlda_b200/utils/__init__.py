@@ -3,6 +3,7 @@
 `load_users` / `load_users_as_dict` (collaborative-filtering loaders) are outside the scope of this build."""
 from .load_documents import load_documents, load_documents_csr
 from .._sample import random_select, sample_dirichlet, split_documents
+from .._coherence import coherence_from_counts, topic_coherence
 
 
 def polygamma(n, x):
@@ -11,4 +12,5 @@ def polygamma(n, x):
 	return _trlda.polygamma(n, x)
 
 
-__all__ = ['load_documents', 'load_documents_csr', 'random_select', 'sample_dirichlet', 'split_documents', 'polygamma']
+__all__ = ['load_documents', 'load_documents_csr', 'random_select', 'sample_dirichlet', 'split_documents', 'coherence_from_counts',
+	'topic_coherence', 'polygamma']
