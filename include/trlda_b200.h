@@ -193,6 +193,19 @@ TRLDA_API int trlda_top_words(trlda_model* m, int n, int32_t* ids_out, double* p
 TRLDA_API int trlda_cooccurrence(trlda_model* m, const trlda_docs* docs, const int32_t* ids, int n,
                                  int64_t* counts_out, int64_t* num_docs_out);
 
+/* Distances between the topics of m and those of `other` (NULL: m itself), with p_i = lambda_i / sum_w lambda_iw the
+ * E[beta] of topic i as in trlda_top_words (lambda in fp64 in both precision modes):
+ *   TRLDA_DISTANCE_HELLINGER  D_ij = sqrt(max(0, 1 - sum_w sqrt(p_iw q_jw))), symmetric, in [0, 1];
+ *   TRLDA_DISTANCE_KL         D_ij = KL(p_i || q_j) = sum_w p_iw log p_iw - sum_w p_iw log q_jw, clamped at 0.
+ * out is K_m x K_other column-major: out[j*K_m + i] = D(topic i of m, topic j of other).  The result is reproducible bit
+ * for bit, and a self-comparison under Hellinger is exactly symmetric.  Both models must have the same V and live on
+ * the same device; a negative entry of lambda, or a zero one in `other` under KL, is an error (TRLDA_ERR_ARG).  A sharded
+ * lambda gives TRLDA_ERR_UNSUPPORTED.  Multi-GPU: every rank computes the whole matrix from its own replica, no
+ * exchange.  Training state is not changed.  No reference counterpart. */
+#define TRLDA_DISTANCE_HELLINGER 0
+#define TRLDA_DISTANCE_KL        1
+TRLDA_API int trlda_topic_distances(trlda_model* m, trlda_model* other, int metric, double* out);
+
 /* ---- parity seams ---------------------------------------------------------------------------------------------
  * The reference draws gamma0 (lda.cpp:135) and Cumulative's lambda (cumulativelda.cpp:60) from libc rand()
  * inside updateParameters and offers no way to pass them in.  These two calls install values that the NEXT

@@ -15,6 +15,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, 'libtrlda_b200.so')
 
 KIND = {'online': 0, 'batch': 1, 'cumulative': 2}
+DISTANCE = {'hellinger': 0, 'kullback_leibler': 1}
 PRECISION = {'fp64': 0, 'mixed': 1}
 NUM_KERNEL_KINDS = 12
 
@@ -109,6 +110,7 @@ PROTOTYPES = {
 		_P(C.c_int64), _dbl]),
 	'trlda_top_words': (C.c_int, [C.c_void_p, C.c_int, _P(C.c_int32), _dbl]),
 	'trlda_cooccurrence': (C.c_int, [C.c_void_p, _P(Docs), _P(C.c_int32), C.c_int, _P(C.c_int64), _P(C.c_int64)]),
+	'trlda_topic_distances': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, _dbl]),
 	'trlda_inject_initial_gamma': (C.c_int, [C.c_void_p, _dbl, C.c_int, C.c_int64]),
 	'trlda_inject_initial_lambda': (C.c_int, [C.c_void_p, _dbl, C.c_int, C.c_int]),
 	'trlda_comm_unique_id': (C.c_int, [C.c_void_p]),
@@ -397,6 +399,14 @@ class Model(object):
 		self._check(self._lib.trlda_cooccurrence(self.h, C.byref(docs.c), ids.ctypes.data_as(_P(C.c_int32)), n,
 			counts.ctypes.data_as(_P(C.c_int64)), C.byref(num_docs)))
 		return counts, num_docs.value
+
+	def topic_distances(self, other=None, metric='hellinger'):
+		"""distances between the topics of this model and those of `other` (None: this model): D[K, K_other] in Fortran
+		order, D[i, j] = hellinger or kullback_leibler distance between E[beta] of topic i here and of topic j there"""
+		k_other = self.K if other is None else other.K
+		out = np.empty((self.K, k_other), order='F')
+		self._check(self._lib.trlda_topic_distances(self.h, None if other is None else other.h, DISTANCE[metric], _dptr(out)))
+		return out
 
 	# ---- multi-GPU / instrumentation --------------------------------------------------------------------------------
 	def comm_init(self, unique_id, rank, nranks):

@@ -248,6 +248,34 @@ void launch_top_words_merge(const double* cand_v, const int32_t* cand_id, const 
 // of the lists it is on, at map_entry[map_ptr[w] .. map_ptr[w + 1])
 void launch_cooccurrence(const DeviceDocs& docs, int K, int n, const int32_t* map_ptr, const int32_t* map_entry,
                          unsigned long long* counts, cudaStream_t s);
+// topics.cu: distances between the topics of two lambdas (K_A x V and K_B x V, fp64) through C = f(P_A) g(P_B)^T,
+// p_kw = lambda_kw / rows_k.  The words are cut into chunks of plan.chunk; per chunk the prepare pass writes f(P_A) and
+// g(P_B) word-major (words x ld, topics padded with zeros) and the product pass adds the chunk to plan.splits partials of C
+// (ld_x x ld_y each); the finish pass sums the partials in order and applies the metric's epilogue.
+enum { DIST_OP_NONE = 0, DIST_OP_SQRT = 1, DIST_OP_IDENTITY = 2, DIST_OP_LOG = 3 };
+enum { DIST_BAD_NEGATIVE = 1, DIST_BAD_ZERO = 2, DIST_BAD_EMPTY_ROW = 4 };   // bits of the prepare pass's flag
+struct DistancePlan {
+	int ld_x, ld_y;   // K_A and K_B rounded up to the product's tile
+	int splits;       // partials of C: the words of a chunk are split into this many equal runs, one per CTA layer
+	int chunk;        // words per chunk, a multiple of splits * the product's stage depth
+};
+// one_operand: X and Y are the same scratch (a self-comparison under Hellinger)
+DistancePlan distance_plan(int KA, int KB, int V, bool one_operand);
+int distance_chunk_words(const DistancePlan& plan, int remaining);   // rows of a chunk with `remaining` words left
+int distance_entropy_parts(int words);                               // entropy partials the prepare pass writes per chunk
+// x[r ld + k] = op_x(p_k,w0+r) for r < words (0 beyond V or K); y likewise when not null.  entropy_part (may be null):
+// per part of the chunk, sum_w p log p of every topic.  flag |= DIST_BAD_* for negative entries, zeros under DIST_OP_LOG,
+// and topics whose row sum is not positive
+void launch_distance_prepare(const double* lambda, int K, int V, int ld, int w0, int words, const double* rows, int op_x,
+                             double* x, int op_y, double* y, double* entropy_part, int* flag, cudaStream_t s);
+// entropy[k] = (first ? 0 : entropy[k]) + the chunk's parts, in order
+void launch_distance_entropy(const double* entropy_part, int parts, int K, int ld, bool first, double* entropy, cudaStream_t s);
+// partial[s] (ld_x x ld_y, column-major) = (first ? 0 : partial[s]) + X_s^T Y_s over split s of the chunk's words
+void launch_distance_product(const DistancePlan& plan, const double* x, const double* y, int words, bool first,
+                             double* partial, cudaStream_t s);
+// out[j KA + i] = sqrt(max(0, 1 - C_ij)) (metric 0) or max(0, entropy_i - C_ij) (metric 1), C = sum of the partials
+void launch_distance_finish(const DistancePlan& plan, const double* partial, int KA, int KB, int metric, const double* entropy,
+                            double* out, cudaStream_t s);
 // out[k] = lgamma(in[k])
 void launch_lgamma_vector(const double* in, int K, double* out, cudaStream_t s);
 

@@ -274,6 +274,11 @@ struct trlda_model {
 	// trlda_top_words: row sums of lambda, the per-chunk candidate lists and the result; trlda_cooccurrence: the inverse map
 	// of the top words and the counters
 	DevBuf topic_rows, top_cand_v, top_cand_id, top_ids, top_prob, co_map_ptr, co_map, co_counts;
+	// trlda_topic_distances: row sums of the other model's lambda, the prepared operands of one chunk of words, the entropy
+	// partials and entropies, the split partials of the product, the result and the prepare pass's flag; other_ready orders
+	// this model's stream after the other model's work
+	DevBuf dist_rows, dist_x, dist_y, dist_hpart, dist_h, dist_partial, dist_out, dist_flag;
+	cudaEvent_t other_ready = nullptr;
 	bool gamma_valid = false;
 
 	// parity seams
@@ -321,6 +326,8 @@ struct trlda_model {
 		}
 		if(fork_event)
 			cudaEventDestroy(fork_event);
+		if(other_ready)
+			cudaEventDestroy(other_ready);
 		if(long_stream)
 			cudaStreamDestroy(long_stream);
 		if(long_join)
@@ -441,17 +448,20 @@ int allreduce(trlda_model* m, void* buf, size_t count, ncclDataType_t type) {
 	return TRLDA_OK;
 }
 
-// rows = row sums of `matrix`
-int compute_rows(trlda_model* m, const double* matrix, double* out) {
+// rows = row sums of `matrix` (K x V; K = m->K unless given, as for the other model's lambda in trlda_topic_distances)
+int compute_rows(trlda_model* m, const double* matrix, double* out, int K = 0) {
+	if(K <= 0)
+		K = m->K;
 	int P = rowsum_num_partials(m->V);
-	CUDA_TRY(m, m->partials.ensure(sizeof(double) * (size_t) std::max(P, colsum_num_partials(std::max<int64_t>(m->mb.docs.B, 1))) * m->K));
+	CUDA_TRY(m, m->partials.ensure(sizeof(double) * (size_t) std::max(P, colsum_num_partials(std::max<int64_t>(m->mb.docs.B, 1))) *
+	                               std::max(K, m->K)));
 	{
 		Launch l(m, KK_ROWSUM);
-		launch_rowsum(matrix, m->K, m->V, m->partials.as<double>(), &P, m->stream);
+		launch_rowsum(matrix, K, m->V, m->partials.as<double>(), &P, m->stream);
 	}
 	{
 		Launch l(m, KK_REDUCE);
-		launch_reduce_partials(m->partials.as<double>(), P, m->K, out, m->stream);
+		launch_reduce_partials(m->partials.as<double>(), P, K, out, m->stream);
 	}
 	return check_launch(m, "rowsum");
 }
@@ -1837,6 +1847,7 @@ int trlda_create(int kind, int num_words, int num_topics, int64_t num_documents,
 	if(const char* tm = getenv("TRLDA_ESTEP_TMEM"))
 		m->tmem_mode = atoi(tm) != 0;
 	cudaEventCreateWithFlags(&m->fork_event, cudaEventDisableTiming);
+	cudaEventCreateWithFlags(&m->other_ready, cudaEventDisableTiming);
 	for(int i = 0; i < trlda_model::kAuxStreams; ++i) {
 		cudaStreamCreateWithFlags(&m->aux[i], cudaStreamNonBlocking);
 		cudaEventCreateWithFlags(&m->join_event[i], cudaEventDisableTiming);
@@ -2410,6 +2421,105 @@ int trlda_cooccurrence(trlda_model* m, const trlda_docs* docs, const int32_t* id
 	if(num_docs_out)
 		*num_docs_out = h[0];
 	return TRLDA_OK;
+}
+
+// trlda_topic_distances with both mutexes held; b is m itself or the other model
+static int topic_distances(trlda_model* m, trlda_model* b, int metric, double* out) {
+	if(metric != TRLDA_DISTANCE_HELLINGER && metric != TRLDA_DISTANCE_KL)
+		return fail(m, TRLDA_ERR_ARG, "Unknown distance metric.");
+	if(!out)
+		return fail(m, TRLDA_ERR_ARG, "topic_distances: no output buffer.");
+	if(b->V != m->V)
+		return fail(m, TRLDA_ERR_ARG, "The two models must have the same number of words.");
+	if(b->device != m->device)
+		return fail(m, TRLDA_ERR_ARG, "The two models must be on the same device.");
+	if(m->lambda_sharded || b->lambda_sharded)
+		return fail(m, TRLDA_ERR_UNSUPPORTED, "topic_distances: lambda is sharded over ranks.");
+	TRY(set_device(m));
+	TRY(ensure_small(m));
+	const bool self = b == m, kl = metric == TRLDA_DISTANCE_KL;
+	const int KA = m->K, KB = b->K, V = m->V;
+	const DistancePlan plan = distance_plan(KA, KB, V, self && !kl);    // a self-comparison under Hellinger: X = Y
+	const int max_parts = distance_entropy_parts(plan.chunk);
+	CUDA_TRY(m, m->topic_rows.ensure(sizeof(double) * KA));
+	CUDA_TRY(m, m->dist_rows.ensure(sizeof(double) * KB));
+	CUDA_TRY(m, m->dist_x.ensure(sizeof(double) * plan.chunk * plan.ld_x));
+	if(!(self && !kl))
+		CUDA_TRY(m, m->dist_y.ensure(sizeof(double) * plan.chunk * plan.ld_y));
+	if(kl) {
+		CUDA_TRY(m, m->dist_hpart.ensure(sizeof(double) * max_parts * plan.ld_x));
+		CUDA_TRY(m, m->dist_h.ensure(sizeof(double) * KA));
+	}
+	CUDA_TRY(m, m->dist_partial.ensure(sizeof(double) * plan.splits * plan.ld_x * plan.ld_y));
+	CUDA_TRY(m, m->dist_out.ensure(sizeof(double) * KA * KB));
+	CUDA_TRY(m, m->dist_flag.ensure(sizeof(int)));
+	CUDA_TRY(m, cudaMemsetAsync(m->dist_flag.p, 0, sizeof(int), m->stream));
+	if(!self) {
+		// the other model's lambda is read on this model's stream: after whatever its own stream has queued
+		CUDA_TRY(m, cudaEventRecord(m->other_ready, b->stream));
+		CUDA_TRY(m, cudaStreamWaitEvent(m->stream, m->other_ready, 0));
+	}
+	double* rows_a = m->topic_rows.as<double>();
+	double* rows_b = self ? rows_a : m->dist_rows.as<double>();
+	TRY(compute_rows(m, m->lambda(), rows_a));            // the row sums of prepare_beta and trlda_top_words
+	if(!self)
+		TRY(compute_rows(m, b->lambda(), rows_b, KB));
+	double* x = m->dist_x.as<double>();
+	double* y = self && !kl ? x : m->dist_y.as<double>();
+	const int op_x = kl ? DIST_OP_IDENTITY : DIST_OP_SQRT, op_y = kl ? DIST_OP_LOG : DIST_OP_SQRT;
+	int* flag = m->dist_flag.as<int>();
+	double* hpart = kl ? m->dist_hpart.as<double>() : nullptr;
+	for(int w0 = 0; w0 < V; w0 += plan.chunk) {
+		const bool first = w0 == 0;
+		const int words = distance_chunk_words(plan, V - w0);
+		{
+			Launch l(m, KK_MISC);   // f(P_A), and g(P_A) too for a self-comparison under KL
+			launch_distance_prepare(m->lambda(), KA, V, plan.ld_x, w0, words, rows_a, op_x, x, self && kl ? op_y : DIST_OP_NONE,
+			                        self && kl ? y : nullptr, hpart, flag, m->stream);
+		}
+		if(!self) {
+			Launch l(m, KK_MISC);
+			launch_distance_prepare(b->lambda(), KB, V, plan.ld_y, w0, words, rows_b, op_y, y, DIST_OP_NONE, nullptr, nullptr,
+			                        flag, m->stream);
+		}
+		if(kl) {
+			Launch l(m, KK_MISC);
+			launch_distance_entropy(hpart, distance_entropy_parts(words), KA, plan.ld_x, first, m->dist_h.as<double>(), m->stream);
+		}
+		{
+			Launch l(m, KK_MISC);
+			launch_distance_product(plan, x, y, words, first, m->dist_partial.as<double>(), m->stream);
+		}
+	}
+	{
+		Launch l(m, KK_MISC);
+		launch_distance_finish(plan, m->dist_partial.as<double>(), KA, KB, metric, kl ? m->dist_h.as<double>() : nullptr,
+		                       m->dist_out.as<double>(), m->stream);
+	}
+	TRY(check_launch(m, "topic_distances"));
+	int* h = m->readback.as<int>();
+	CUDA_TRY(m, cudaMemcpyAsync(h, flag, sizeof(int), cudaMemcpyDeviceToHost, m->stream));
+	CUDA_TRY(m, cudaStreamSynchronize(m->stream));
+	const int bad = h[0];
+	if(bad & DIST_BAD_NEGATIVE)
+		return fail(m, TRLDA_ERR_ARG, "topic_distances: lambda has a negative entry.");
+	if(bad & DIST_BAD_EMPTY_ROW)
+		return fail(m, TRLDA_ERR_ARG, "topic_distances: a topic's lambda sums to zero.");
+	if(bad & DIST_BAD_ZERO)
+		return fail(m, TRLDA_ERR_ARG, "topic_distances: the Kullback-Leibler distance needs a positive lambda in the second model.");
+	CUDA_TRY(m, cudaMemcpyAsync(out, m->dist_out.p, sizeof(double) * KA * KB, cudaMemcpyDeviceToHost, m->stream));
+	CUDA_TRY(m, cudaStreamSynchronize(m->stream));
+	m->stats.d2h_bytes += sizeof(double) * KA * KB + sizeof(int);
+	return TRLDA_OK;
+}
+
+int trlda_topic_distances(trlda_model* m, trlda_model* other, int metric, double* out) {
+	if(!other || other == m) {
+		std::scoped_lock lock__(m->mu);
+		return topic_distances(m, m, metric, out);
+	}
+	std::scoped_lock lock__(m->mu, other->mu);   // std::lock's deadlock avoidance, whatever order other callers use
+	return topic_distances(m, other, metric, out);
 }
 
 int trlda_debug_global_csc(trlda_model* m, const int32_t* len, const int32_t* ids, int ranks, int64_t max_docs, int64_t max_pairs,

@@ -692,6 +692,49 @@ PyObject* LDA_cooccurrence(LDAObject* self, PyObject* args, PyObject* kwds) {
 	return result;
 }
 
+extern PyTypeObject LDA_type;
+
+// topic_distances (no reference counterpart): trlda_topic_distances
+PyObject* LDA_topic_distances(LDAObject* self, PyObject* args, PyObject* kwds) {
+	REQUIRE_MODEL(self, nullptr);
+	const char* kwlist[] = {"other", "metric", nullptr};
+	PyObject* other = Py_None;
+	const char* metric = "hellinger";
+	if(!PyArg_ParseTupleAndKeywords(args, kwds, "|Os", const_cast<char**>(kwlist), &other, &metric))
+		return nullptr;
+	LDAObject* o = self;
+	if(other != Py_None) {
+		if(!PyObject_TypeCheck(other, &LDA_type)) {
+			PyErr_SetString(PyExc_TypeError, "`other` should be a model (OnlineLDA, BatchLDA or CumulativeLDA).");
+			return nullptr;
+		}
+		o = (LDAObject*) other;
+		REQUIRE_MODEL(o, nullptr);
+	}
+	int code;
+	if(!strcmp(metric, "hellinger"))
+		code = TRLDA_DISTANCE_HELLINGER;
+	else if(!strcmp(metric, "kullback_leibler"))
+		code = TRLDA_DISTANCE_KL;
+	else {
+		PyErr_SetString(PyExc_ValueError, "`metric` should be either 'hellinger' or 'kullback_leibler'.");
+		return nullptr;
+	}
+	PyObject* out = new_farray(trlda_num_topics(self->m), trlda_num_topics(o->m));
+	if(!out)
+		return nullptr;
+	int status;
+	double* d = static_cast<double*>(PyArray_DATA((PyArrayObject*) out));
+	Py_BEGIN_ALLOW_THREADS
+	status = trlda_topic_distances(self->m, o->m, code, d);
+	Py_END_ALLOW_THREADS
+	if(status != TRLDA_OK) {
+		Py_DECREF(out);
+		return raise_status(self->m, status);
+	}
+	return out;
+}
+
 PyObject* LDA_str(PyObject* self_) {                                      // ldainterface.cpp:473-490
 	LDAObject* self = (LDAObject*) self_;
 	REQUIRE_MODEL(self, nullptr);
@@ -999,6 +1042,25 @@ const char* cooccurrence_doc =
 	"so the results of several batches of documents can be added up; trlda.utils.topic_coherence does that and turns\n"
 	"them into UMass or NPMI coherence.  The model's parameters are not changed.";
 
+const char* topic_distances_doc =
+	"topic_distances(other=None, metric='hellinger')\n\n"
+	"Distances between the topics of this model and those of `other` (another model with the same num_words on the same\n"
+	"GPU; None: this model), computed on the GPU from E[beta_k] = lambda_k / sum_w lambda_kw.  Returns a float64 array\n"
+	"of shape (num_topics, other.num_topics) in Fortran order, D[i, j] between topic i here and topic j there.\n\n"
+	"metric='hellinger': D_ij = sqrt(max(0, 1 - sum_w sqrt(p_iw q_jw))), symmetric and in [0, 1].\n"
+	"metric='kullback_leibler': D_ij = KL(p_i || q_j) = sum_w p_iw log(p_iw / q_jw), clamped at 0; other's lambda\n"
+	"must be positive.\n\n"
+	"The inner sum is accumulated in float64 over the vocabulary, so its rounding error is about num_words * 1e-16:\n"
+	"distances below about 1e-5 (Hellinger, the square root of that error) and 1e-9 (Kullback-Leibler) are not\n"
+	"resolved, and a topic's distance to itself comes out at that floor rather than 0.  The result is reproducible\n"
+	"bit for bit, the same in both precision modes, and exactly symmetric for model.topic_distances().\n\n"
+	"To match the topics of two runs (the order of topics is arbitrary), e.g. with scipy:\n\n"
+	"    from scipy.optimize import linear_sum_assignment\n"
+	"    d = model.topic_distances(other)\n"
+	"    rows, cols = linear_sum_assignment(d)   # topic rows[i] here is topic cols[i] there\n"
+	"    print(d[rows, cols].mean())\n\n"
+	"The model's parameters are not changed.";
+
 PyGetSetDef LDA_getset[] = {
 	{"num_topics", (getter) LDA_num_topics, nullptr, "Number of topics.", nullptr},
 	{"num_words", (getter) LDA_num_words, nullptr, "Number of words.", nullptr},
@@ -1019,6 +1081,7 @@ PyMethodDef LDA_methods[] = {
 		predictive_log_likelihood_doc},
 	{"top_words", (PyCFunction) LDA_top_words, METH_VARARGS | METH_KEYWORDS, top_words_doc},
 	{"cooccurrence", (PyCFunction) LDA_cooccurrence, METH_VARARGS | METH_KEYWORDS, cooccurrence_doc},
+	{"topic_distances", (PyCFunction) LDA_topic_distances, METH_VARARGS | METH_KEYWORDS, topic_distances_doc},
 	{nullptr, nullptr, 0, nullptr}};
 
 PyGetSetDef OnlineLDA_getset[] = {

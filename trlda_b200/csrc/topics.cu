@@ -1,6 +1,7 @@
-// topics.cu — looking at a trained model: the most probable words of every topic (trlda_top_words) and how many documents
+// topics.cu — looking at a trained model: the most probable words of every topic (trlda_top_words), how many documents
 // of a corpus contain each of those words and each pair of them (trlda_cooccurrence), the counts behind the document
-// co-occurrence coherence measures (UMass, NPMI).  Neither has a counterpart in the reference.
+// co-occurrence coherence measures (UMass, NPMI), and the Hellinger / Kullback-Leibler distances between the topics of one
+// or two models (trlda_topic_distances).  None has a counterpart in the reference.
 #include "kernels.cuh"
 
 #include <algorithm>
@@ -167,6 +168,182 @@ __global__ void __launch_bounds__(CO_THREADS) k_cooccurrence(DeviceDocs docs, in
 	}
 }
 
+// ---- distances between topics ------------------------------------------------------------------------------------------
+// D = epilogue(C), C = f(P_A) g(P_B)^T: Hellinger f = g = sqrt, D = sqrt(max(0, 1 - C)); Kullback-Leibler f = identity,
+// g = log, D = max(0, H_i - C) with the row entropy H_i = sum_w p_iw log p_iw.  lambda is read in fp64 in both modes.
+//
+// Prepare: CTAs of 32 topics x 8 rows of words; a warp reads 32 consecutive topics of one lambda column (coalesced) and
+// writes them to the same place of a word-major scratch whose rows are padded to the product's tile with zeros.  The entropy
+// of a topic over the CTA's 64 words is summed per thread in word order, then over the 8 threads in order.
+// Product: fp64 register tiles, plain DFMA (sm_100's tensor cores have no f64 kind).  CTA (I, J, s) owns the 128 x 128 tile
+// (I, J) of partial s and walks the words of split s in stages of 8: every stage is 8 coalesced runs of 128 consecutive
+// topics per operand, double-buffered in shared memory through registers; each thread keeps an 8 x 8 block (rows
+// tr*4 + {0..3} and 64 + tr*4 + {0..3}, columns likewise with tc) and does one fma per element and word.  Every element of
+// C is thus one fma chain over its split's words in word order, started from the partial of the previous chunk; with
+// f = g and X = Y, C_ij and C_ji are the same chain with the two factors swapped, so a self-comparison is exactly symmetric.
+// The partials are added in split order by the finish pass: the result is reproducible bit for bit from call to call.
+constexpr int DIST_TILE = 128;
+constexpr int DIST_BK = 8;
+constexpr int DIST_THREADS = 256;
+constexpr int DIST_PREP_WORDS = 64;           // words per prepare CTA
+constexpr size_t DIST_SCRATCH = 256u << 20;   // bytes of prepared operands per chunk, at most (unless one stage exceeds it)
+
+__device__ __forceinline__ double distance_op(int op, double p) {
+	return op == DIST_OP_SQRT ? sqrt(p) : op == DIST_OP_LOG ? log(p) : p;
+}
+
+__global__ void __launch_bounds__(256) k_distance_prepare(const double* __restrict__ lambda, int K, int V, int ld, int w0,
+                                                          int words, const double* __restrict__ rows, int op_x,
+                                                          double* __restrict__ x, int op_y, double* __restrict__ y,
+                                                          double* __restrict__ entropy_part, int* __restrict__ flag) {
+	__shared__ double h_s[8][32];
+	const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
+	const int k = blockIdx.x * 32 + tx;   // < ld
+	const bool topic = k < K;
+	const double r = topic ? rows[k] : 1.;
+	const bool logs = op_x == DIST_OP_LOG || (y && op_y == DIST_OP_LOG);
+	int bad = topic && !(r > 0.) ? DIST_BAD_EMPTY_ROW : 0;
+	double h = 0.;
+	#pragma unroll 4
+	for(int i = 0; i < DIST_PREP_WORDS / 8; ++i) {
+		const int row = blockIdx.y * DIST_PREP_WORDS + i * 8 + ty;
+		if(row >= words)
+			break;
+		const int w = w0 + row;
+		double vx = 0., vy = 0.;
+		if(topic && w < V) {
+			const double v = __ldg(lambda + (int64_t) w * K + k);
+			bad |= v < 0. ? DIST_BAD_NEGATIVE : 0;
+			bad |= logs && v == 0. ? DIST_BAD_ZERO : 0;
+			const double p = v / r;
+			vx = distance_op(op_x, p);
+			if(y)
+				vy = distance_op(op_y, p);
+			if(entropy_part && p > 0.)
+				h += p * log(p);
+		}
+		x[(int64_t) row * ld + k] = vx;
+		if(y)
+			y[(int64_t) row * ld + k] = vy;
+	}
+	if(bad)
+		atomicOr(flag, bad);
+	if(entropy_part) {
+		h_s[ty][tx] = h;
+		__syncthreads();
+		if(ty == 0 && topic) {
+			double sum = h_s[0][tx];
+			#pragma unroll
+			for(int t = 1; t < 8; ++t)
+				sum += h_s[t][tx];
+			entropy_part[(int64_t) blockIdx.y * ld + k] = sum;
+		}
+	}
+}
+
+__global__ void k_distance_entropy(const double* __restrict__ entropy_part, int parts, int K, int ld, int first,
+                                   double* __restrict__ entropy) {
+	const int k = blockIdx.x * blockDim.x + threadIdx.x;
+	if(k >= K)
+		return;
+	double acc = first ? 0. : entropy[k];
+	for(int p = 0; p < parts; ++p)
+		acc += entropy_part[(int64_t) p * ld + k];
+	entropy[k] = acc;
+}
+
+__global__ void __launch_bounds__(DIST_THREADS, 1) k_distance_product(const double* __restrict__ x, int ld_x,
+                                                                      const double* __restrict__ y, int ld_y,
+                                                                      int split_words, int first,
+                                                                      double* __restrict__ partial) {
+	__shared__ __align__(16) double xs[2][DIST_BK][DIST_TILE];
+	__shared__ __align__(16) double ys[2][DIST_BK][DIST_TILE];
+	const int t = threadIdx.x, tr = t & 15, tc = t >> 4;
+	const int i0 = blockIdx.x * DIST_TILE, j0 = blockIdx.y * DIST_TILE;
+	double* out = partial + (int64_t) blockIdx.z * ld_x * ld_y;
+
+	// element (a, b) of the thread's block: row i0 + orow(a), column j0 + orow(b)
+	auto orow = [](int q, int a) { return (a < 4 ? 0 : 64) + q * 4 + (a & 3); };
+	double acc[8][8];
+	#pragma unroll
+	for(int a = 0; a < 8; ++a)
+		#pragma unroll
+		for(int b = 0; b < 8; ++b)
+			acc[a][b] = first ? 0. : out[(int64_t) (j0 + orow(tc, b)) * ld_x + i0 + orow(tr, a)];
+
+	// stage loads: thread t moves topics (2t) % 128, +1 of words t / 64 and t / 64 + 4, in both operands
+	const int lw = t >> 6, lt = (2 * t) & (DIST_TILE - 1);
+	const double* xp = x + ((int64_t) blockIdx.z * split_words + lw) * ld_x + i0 + lt;
+	const double* yp = y + ((int64_t) blockIdx.z * split_words + lw) * ld_y + j0 + lt;
+	double2 rx0 = __ldg(reinterpret_cast<const double2*>(xp)), rx1 = __ldg(reinterpret_cast<const double2*>(xp + 4 * ld_x));
+	double2 ry0 = __ldg(reinterpret_cast<const double2*>(yp)), ry1 = __ldg(reinterpret_cast<const double2*>(yp + 4 * ld_y));
+	*reinterpret_cast<double2*>(&xs[0][lw][lt]) = rx0;
+	*reinterpret_cast<double2*>(&xs[0][lw + 4][lt]) = rx1;
+	*reinterpret_cast<double2*>(&ys[0][lw][lt]) = ry0;
+	*reinterpret_cast<double2*>(&ys[0][lw + 4][lt]) = ry1;
+	__syncthreads();
+
+	const int steps = split_words / DIST_BK;
+	for(int s = 0; s < steps; ++s) {
+		const int cur = s & 1;
+		const bool more = s + 1 < steps;
+		if(more) {
+			xp += (int64_t) DIST_BK * ld_x;
+			yp += (int64_t) DIST_BK * ld_y;
+			rx0 = __ldg(reinterpret_cast<const double2*>(xp));
+			rx1 = __ldg(reinterpret_cast<const double2*>(xp + 4 * ld_x));
+			ry0 = __ldg(reinterpret_cast<const double2*>(yp));
+			ry1 = __ldg(reinterpret_cast<const double2*>(yp + 4 * ld_y));
+		}
+		#pragma unroll
+		for(int k = 0; k < DIST_BK; ++k) {
+			double av[8], bv[8];
+			#pragma unroll
+			for(int h = 0; h < 4; ++h) {
+				const double2 a2 = *reinterpret_cast<const double2*>(&xs[cur][k][(h < 2 ? 0 : 64) + tr * 4 + (h & 1) * 2]);
+				const double2 b2 = *reinterpret_cast<const double2*>(&ys[cur][k][(h < 2 ? 0 : 64) + tc * 4 + (h & 1) * 2]);
+				av[2 * h] = a2.x;
+				av[2 * h + 1] = a2.y;
+				bv[2 * h] = b2.x;
+				bv[2 * h + 1] = b2.y;
+			}
+			#pragma unroll
+			for(int a = 0; a < 8; ++a)
+				#pragma unroll
+				for(int b = 0; b < 8; ++b)
+					acc[a][b] = fma(av[a], bv[b], acc[a][b]);
+		}
+		if(more) {
+			*reinterpret_cast<double2*>(&xs[cur ^ 1][lw][lt]) = rx0;
+			*reinterpret_cast<double2*>(&xs[cur ^ 1][lw + 4][lt]) = rx1;
+			*reinterpret_cast<double2*>(&ys[cur ^ 1][lw][lt]) = ry0;
+			*reinterpret_cast<double2*>(&ys[cur ^ 1][lw + 4][lt]) = ry1;
+		}
+		__syncthreads();
+	}
+
+	#pragma unroll
+	for(int b = 0; b < 8; ++b) {
+		double* col = out + (int64_t) (j0 + orow(tc, b)) * ld_x + i0;
+		#pragma unroll
+		for(int a = 0; a < 8; a += 2)
+			*reinterpret_cast<double2*>(col + orow(tr, a)) = make_double2(acc[a][b], acc[a + 1][b]);
+	}
+}
+
+__global__ void k_distance_finish(const double* __restrict__ partial, int splits, int ld_x, int ld_y, int KA, int KB,
+                                  int metric, const double* __restrict__ entropy, double* __restrict__ out) {
+	const int64_t n = (int64_t) KA * KB, stride = (int64_t) ld_x * ld_y;
+	for(int64_t idx = (int64_t) blockIdx.x * blockDim.x + threadIdx.x; idx < n; idx += (int64_t) gridDim.x * blockDim.x) {
+		const int j = (int) (idx / KA), i = (int) (idx - (int64_t) j * KA);
+		const double* p = partial + (int64_t) j * ld_x + i;
+		double c = p[0];
+		for(int s = 1; s < splits; ++s)
+			c += p[s * stride];
+		out[idx] = metric == 0 ? sqrt(fmax(0., 1. - c)) : fmax(0., entropy[i] - c);
+	}
+}
+
 int sm_count() {
 	static const int count = [] {
 		int device = 0, c = 148;
@@ -210,6 +387,65 @@ void launch_cooccurrence(const DeviceDocs& docs, int K, int n, const int32_t* ma
 		return;
 	k_cooccurrence<<<(unsigned) std::min<int64_t>(docs.B, sm_count() * 8), CO_THREADS, (size_t) K * 8, s>>>(
 		docs, K, n, map_ptr, map_entry, counts);
+}
+
+DistancePlan distance_plan(int KA, int KB, int V, bool one_operand) {
+	DistancePlan p;
+	p.ld_x = (KA + DIST_TILE - 1) / DIST_TILE * DIST_TILE;
+	p.ld_y = (KB + DIST_TILE - 1) / DIST_TILE * DIST_TILE;
+	// splits: with fewer tiles than SMs, the smallest count in [lo, 4 lo] whose last wave is fullest (one CTA per SM);
+	// each split keeps at least 64 words
+	const int sms = sm_count(), tiles = (p.ld_x / DIST_TILE) * (p.ld_y / DIST_TILE);
+	p.splits = 1;
+	if(tiles < sms) {
+		const int lo = (sms + tiles - 1) / tiles;
+		double best = 0.;
+		for(int s = lo; s <= 4 * lo; ++s) {
+			const int ctas = tiles * s;
+			const double fill = (double) ctas / ((double) ((ctas + sms - 1) / sms) * sms);
+			if(fill > best + 1e-12) {
+				best = fill;
+				p.splits = s;
+			}
+		}
+	}
+	p.splits = std::max(1, std::min(p.splits, V / 64));
+	const int step = p.splits * DIST_BK;
+	const size_t per_word = sizeof(double) * (size_t) (p.ld_x + (one_operand ? 0 : p.ld_y));
+	const int64_t fit = (int64_t) (DIST_SCRATCH / per_word) / step * step;
+	const int64_t all = ((int64_t) V + step - 1) / step * step;
+	p.chunk = (int) std::max<int64_t>(step, std::min(fit, all));
+	return p;
+}
+
+int distance_chunk_words(const DistancePlan& plan, int remaining) {
+	const int step = plan.splits * DIST_BK;
+	return (std::min(plan.chunk, remaining) + step - 1) / step * step;
+}
+
+int distance_entropy_parts(int words) { return (words + DIST_PREP_WORDS - 1) / DIST_PREP_WORDS; }
+
+void launch_distance_prepare(const double* lambda, int K, int V, int ld, int w0, int words, const double* rows, int op_x,
+                             double* x, int op_y, double* y, double* entropy_part, int* flag, cudaStream_t s) {
+	const dim3 grid((unsigned) (ld / 32), (unsigned) distance_entropy_parts(words));
+	k_distance_prepare<<<grid, 256, 0, s>>>(lambda, K, V, ld, w0, words, rows, op_x, x, op_y, y, entropy_part, flag);
+}
+
+void launch_distance_entropy(const double* entropy_part, int parts, int K, int ld, bool first, double* entropy, cudaStream_t s) {
+	k_distance_entropy<<<(K + 255) / 256, 256, 0, s>>>(entropy_part, parts, K, ld, first ? 1 : 0, entropy);
+}
+
+void launch_distance_product(const DistancePlan& plan, const double* x, const double* y, int words, bool first,
+                             double* partial, cudaStream_t s) {
+	const dim3 grid((unsigned) (plan.ld_x / DIST_TILE), (unsigned) (plan.ld_y / DIST_TILE), (unsigned) plan.splits);
+	k_distance_product<<<grid, DIST_THREADS, 0, s>>>(x, plan.ld_x, y, plan.ld_y, words / plan.splits, first ? 1 : 0, partial);
+}
+
+void launch_distance_finish(const DistancePlan& plan, const double* partial, int KA, int KB, int metric, const double* entropy,
+                            double* out, cudaStream_t s) {
+	const int64_t n = (int64_t) KA * KB;
+	const unsigned blocks = (unsigned) std::min<int64_t>((n + 255) / 256, (int64_t) sm_count() * 16);
+	k_distance_finish<<<blocks, 256, 0, s>>>(partial, plan.splits, plan.ld_x, plan.ld_y, KA, KB, metric, entropy, out);
 }
 
 }  // namespace trlda

@@ -10,6 +10,26 @@ form `load_documents` produces (python/utils/load_documents.py:41-44).
 import numpy as np
 
 
+def _topic_weights(seed, k, num_words, eta):
+	"""unnormalised beta_k ~ Dirichlet(eta 1_V) of topic k of corpus `seed`: standard_gamma(eta, V) from the topic's own
+	stream, floored at 1e-300 so that every word has positive probability"""
+	topic_rng = np.random.Generator(np.random.PCG64([seed, k]))
+	return np.maximum(topic_rng.standard_gamma(eta, size=num_words), 1e-300)
+
+
+def make_topics(num_words, num_topics, eta=.2, seed=0):
+	"""
+	The topics make_corpus(..., num_words, num_topics, eta=eta, seed=seed) draws its words from: a num_topics x num_words
+	float64 array whose row k is beta_k (sums to 1).  Useful as the lambda of a reference model, e.g. to check with
+	topic_distances that training recovers the topics.
+	"""
+	topics = np.empty((num_topics, num_words))
+	for k in range(num_topics):
+		beta = _topic_weights(seed, k, num_words, eta)
+		topics[k] = beta / beta.sum()
+	return topics
+
+
 def make_corpus(num_docs, num_words, num_topics, alpha=.1, eta=.2, mean_length=150, seed=0, doc_seed=None):
 	"""
 	Returns the minibatch in CSR form: (doc_ptr[int64, B+1], word_ids[int32, N], counts[int32, N]).
@@ -48,9 +68,7 @@ def make_corpus(num_docs, num_words, num_topics, alpha=.1, eta=.2, mean_length=1
 		lo, hi = bounds[k], bounds[k + 1]
 		if lo == hi:
 			continue
-		topic_rng = np.random.Generator(np.random.PCG64([seed, k]))
-		beta = np.maximum(topic_rng.standard_gamma(eta, size=num_words), 1e-300)
-		cdf = np.cumsum(beta)
+		cdf = np.cumsum(_topic_weights(seed, k, num_words, eta))
 		cdf /= cdf[-1]
 		idx = order[lo:hi]
 		words[idx] = np.minimum(np.searchsorted(cdf, v[idx], side='right'), num_words - 1)
