@@ -180,6 +180,15 @@ TRLDA_API int trlda_predictive_log_likelihood(trlda_model* m, const trlda_docs* 
         const double* latents, int latents_rows, int64_t latents_cols, const trlda_params* params,
         double* total_out, int64_t* tokens_out, double* per_doc_out);
 
+/* The n most probable topics of every (word, count) pair of `docs` under the variational distribution the E-step fits:
+ * gamma as trlda_update_variables computes it (bitwise), then phi_djk = softmax_k(psi(gamma_dk) + psi(lambda_kw) - psi(sum_v lambda_kv)),
+ * in fp64 from lambda in fp64 in both precision modes.  topics_out and probs_out (may be NULL) are N x n pair-major: pair j's
+ * list at topics_out + j*n, ranked by descending score, equal scores by the smaller topic id.  gamma_out (K x B, may be NULL).
+ * 1 <= n <= min(32, K).  Multi-GPU: docs is this rank's shard, outputs are this rank's, no exchange.  No reference counterpart. */
+TRLDA_API int trlda_word_topics(trlda_model* m, const trlda_docs* docs, const double* latents, int latents_rows,
+                                int64_t latents_cols, const trlda_params* params, int n,
+                                int32_t* topics_out, double* probs_out, double* gamma_out);
+
 /* The n most probable words of every topic, in the order of E[beta_kw] = lambda_kw / sum_w lambda_kw: descending,
  * ties broken by the smaller word id.  ids_out is n x K column-major (topic k's list at ids_out + k*n, rank order);
  * prob_out (may be NULL) receives the matching E[beta_kw].  1 <= n <= min(32, V).  No reference counterpart. */

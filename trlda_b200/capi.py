@@ -108,6 +108,8 @@ PROTOTYPES = {
 	'trlda_lower_bound': (C.c_int, [C.c_void_p, _P(Docs), _dbl, C.c_int, C.c_int64, _P(Params), C.c_int64, _dbl, _dbl]),
 	'trlda_predictive_log_likelihood': (C.c_int, [C.c_void_p, _P(Docs), _P(Docs), _dbl, C.c_int, C.c_int64, _P(Params), _dbl,
 		_P(C.c_int64), _dbl]),
+	'trlda_word_topics': (C.c_int, [C.c_void_p, _P(Docs), _dbl, C.c_int, C.c_int64, _P(Params), C.c_int, _P(C.c_int32), _dbl,
+		_dbl]),
 	'trlda_top_words': (C.c_int, [C.c_void_p, C.c_int, _P(C.c_int32), _dbl]),
 	'trlda_cooccurrence': (C.c_int, [C.c_void_p, _P(Docs), _P(C.c_int32), C.c_int, _P(C.c_int64), _P(C.c_int64)]),
 	'trlda_topic_distances': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, _dbl]),
@@ -379,6 +381,22 @@ class Model(object):
 			self.h, C.byref(docs.c), C.byref(held_out.c), _dptr(latents), rows, cols, C.byref(params),
 			C.byref(total), C.byref(tokens), _dptr(per_doc)))
 		return total.value, tokens.value, per_doc
+
+	def word_topics(self, docs, n=1, latents=None, max_iter=100, threshold=1e-3):
+		"""the n most probable topics of every pair of `docs` under the fitted phi: (topics[N, n] int32, probs[N, n],
+		gamma[K, B]), row j for the j-th pair, each row ranked by descending phi (equal phi: the smaller topic first)"""
+		params = default_params(max_iter_inference=max_iter, threshold=threshold)
+		rows, cols = 0, 0
+		if latents is not None:
+			latents = _fortran(latents)
+			rows, cols = latents.shape
+		pairs = int(docs.doc_ptr[-1])
+		topics = np.empty((pairs, max(int(n), 0)), dtype=np.int32)
+		probs = np.empty((pairs, max(int(n), 0)))
+		gamma = np.empty((self.K, docs.num_docs), order='F')
+		self._check(self._lib.trlda_word_topics(self.h, C.byref(docs.c), _dptr(latents), rows, cols, C.byref(params), int(n),
+			topics.ctypes.data_as(_P(C.c_int32)), _dptr(probs), _dptr(gamma)))
+		return topics, probs, gamma
 
 	def top_words(self, n=10):
 		"""the n most probable words of every topic: (ids[K, n] int32, probs[K, n]), each row in rank order"""

@@ -276,6 +276,17 @@ void launch_distance_product(const DistancePlan& plan, const double* x, const do
 // out[j KA + i] = sqrt(max(0, 1 - C_ij)) (metric 0) or max(0, entropy_i - C_ij) (metric 1), C = sum of the partials
 void launch_distance_finish(const DistancePlan& plan, const double* partial, int KA, int KB, int metric, const double* entropy,
                             double* out, cudaStream_t s);
+// topics.cu: the n (<= 32) most probable topics of every pair under phi_jk = softmax_k(psi(gamma_dk) + psi(lambda_kw) -
+// psi_rows_k), fp64.  The words are taken in chunks of word_topics_chunk_words(K) ids.  The table pass writes
+// table[(w - w0) K + k] = psi(lambda_kw) - psi_rows_k for the words w in [w0, w0 + count) that have pairs (word_ptr).  The
+// pair pass takes the pairs of the words [w0, w1) from the word-sorted token list of `docs` (word_ptr, tok_doc, tok_src,
+// word_ids); psi_gamma is K x B.  Pair j's topics go to topics + j*n (ranked by descending score, equal scores by the smaller
+// topic), their phi to probs (may be null).
+int word_topics_chunk_words(int K);
+void launch_word_topics_table(const double* lambda, int K, int w0, int count, const int32_t* word_ptr, const double* psi_rows,
+                              double* table, cudaStream_t s);
+void launch_word_topics_pairs(const DeviceDocs& docs, int w0, int w1, const double* table, const double* psi_gamma, int K, int n,
+                              int32_t* topics, double* probs, cudaStream_t s);
 // out[k] = lgamma(in[k])
 void launch_lgamma_vector(const double* in, int K, double* out, cudaStream_t s);
 

@@ -279,6 +279,9 @@ struct trlda_model {
 	// this model's stream after the other model's work
 	DevBuf dist_rows, dist_x, dist_y, dist_hpart, dist_h, dist_partial, dist_out, dist_flag;
 	cudaEvent_t other_ready = nullptr;
+	// trlda_word_topics: the call's document lengths, the scratch and the result of its word-sorted token list, the log-beta
+	// table of one chunk of words, psi(gamma) and the results
+	DevBuf wt_len, wt_scratch, wt_word_ptr, wt_tok_doc, wt_tok_src, wt_table, wt_psi_gamma, wt_topics, wt_probs;
 	bool gamma_valid = false;
 
 	// parity seams
@@ -2320,6 +2323,91 @@ int trlda_predictive_log_likelihood(trlda_model* m, const trlda_docs* observed, 
 		CUDA_TRY(m, cudaMemcpy(per_doc_out, per_doc, sizeof(double) * B, cudaMemcpyDeviceToHost));
 		m->stats.d2h_bytes += sizeof(double) * B;
 	}
+	consume_injections(m);
+	return TRLDA_OK;
+}
+
+static const int kMaxWordTopics = 32;   // one warp lane per rank in k_word_topics_pairs
+
+int trlda_word_topics(trlda_model* m, const trlda_docs* docs, const double* latents, int latents_rows, int64_t latents_cols,
+                      const trlda_params* params, int n, int32_t* topics_out, double* probs_out, double* gamma_out) {
+	std::lock_guard<std::recursive_mutex> lock__(m->mu);
+	if(params->inference_method != TRLDA_INFERENCE_VI)
+		return fail(m, TRLDA_ERR_UNSUPPORTED, "Only variational inference ('VI') is implemented on the device.");
+	if(m->lambda_sharded)
+		return fail(m, TRLDA_ERR_UNSUPPORTED, "word_topics: lambda is sharded over ranks.");
+	if(n < 1 || n > kMaxWordTopics || n > m->K)
+		return fail(m, TRLDA_ERR_ARG, "Number of topics per word must lie in [1, min(32, number of topics)].");
+	if(!topics_out)
+		return fail(m, TRLDA_ERR_ARG, "word_topics: no output buffer.");
+	if(!docs)
+		return fail(m, TRLDA_ERR_ARG, "Documents must be given in CSR form.");
+	if(latents && (latents_rows != m->K || latents_cols != docs->num_docs))
+		return fail(m, TRLDA_ERR_ARG, "Initial gamma has wrong dimensionality.");
+	// gamma exactly as trlda_update_variables fits it (upload_docs also checks the CSR)
+	TRY(upload_docs(m, docs));
+	TRY(prepare_beta(m));                                                      // also leaves psi_rows of lambda
+	TRY(run_estep(m, latents ? GAMMA_HOST : GAMMA_FRESH, latents, params->max_iter_inference, params->threshold));
+	const int K = m->K, V = m->V;
+	const int64_t B = m->mb.docs.B, N = m->mb.docs.N;
+	const int chunk = std::min(word_topics_chunk_words(K), V);
+	CUDA_TRY(m, m->wt_len.ensure(sizeof(int32_t) * std::max<int64_t>(B, 1)));
+	CUDA_TRY(m, m->wt_scratch.ensure(sizeof(int32_t) * global_csc_scratch_ints(B, N, 0, V)));
+	CUDA_TRY(m, m->wt_word_ptr.ensure(sizeof(int32_t) * ((size_t) V + 1)));
+	CUDA_TRY(m, m->wt_tok_doc.ensure(sizeof(int32_t) * std::max<int64_t>(N, 1)));
+	CUDA_TRY(m, m->wt_tok_src.ensure(sizeof(int32_t) * std::max<int64_t>(N, 1)));
+	CUDA_TRY(m, m->wt_table.ensure(sizeof(double) * (size_t) chunk * K));
+	CUDA_TRY(m, m->wt_psi_gamma.ensure(sizeof(double) * (size_t) K * std::max<int64_t>(B, 1)));
+	CUDA_TRY(m, m->wt_topics.ensure(sizeof(int32_t) * (size_t) std::max<int64_t>(N, 1) * n));
+	if(probs_out)
+		CUDA_TRY(m, m->wt_probs.ensure(sizeof(double) * (size_t) std::max<int64_t>(N, 1) * n));
+	// the call's own word-sorted token list (a word's pairs in CSR order), built on the device by the builder of the
+	// multi-GPU exchange with this rank's documents as the only segment.  The live minibatch's list is not used: on several
+	// GPUs it covers the whole gathered minibatch.
+	DeviceDocs wt = m->mb.docs;
+	wt.word_ptr = m->wt_word_ptr.as<int32_t>();
+	wt.tok_doc = m->wt_tok_doc.as<int32_t>();
+	wt.tok_src = m->wt_tok_src.as<int32_t>();
+	{
+		Launch l(m, KK_MISC);
+		launch_doc_lengths(wt.doc_ptr, B, B, m->wt_len.as<int32_t>(), m->stream);
+		launch_global_csc(m->wt_len.as<int32_t>(), wt.word_ids, 1, B, N, 0, V, V, m->wt_scratch.as<int32_t>(),
+		                  m->wt_word_ptr.as<int32_t>(), m->wt_tok_doc.as<int32_t>(), m->wt_tok_src.as<int32_t>(), m->stream);
+	}
+	double* psi_gamma = m->wt_psi_gamma.as<double>();
+	// psi(gamma), in runs of whole documents that keep the element count in an int
+	const int64_t run = std::max<int64_t>(1, INT_MAX / K);
+	for(int64_t d0 = 0; d0 < B; d0 += run) {
+		Launch l(m, KK_MISC);
+		launch_psi_vector(m->gamma.as<double>() + d0 * K, (int) (std::min(run, B - d0) * K), psi_gamma + d0 * K, m->stream);
+	}
+	for(int w0 = 0; w0 < V && N > 0; w0 += chunk) {
+		const int count = std::min(chunk, V - w0);
+		{
+			Launch l(m, KK_MISC);
+			launch_word_topics_table(m->lambda(), K, w0, count, wt.word_ptr, m->psi_rows.as<double>(), m->wt_table.as<double>(),
+			                         m->stream);
+		}
+		{
+			Launch l(m, KK_MISC);
+			launch_word_topics_pairs(wt, w0, w0 + count, m->wt_table.as<double>(), psi_gamma, K, n, m->wt_topics.as<int32_t>(),
+			                         probs_out ? m->wt_probs.as<double>() : nullptr, m->stream);
+		}
+	}
+	TRY(check_launch(m, "word_topics"));
+	if(N) {
+		CUDA_TRY(m, cudaMemcpyAsync(topics_out, m->wt_topics.p, sizeof(int32_t) * (size_t) N * n, cudaMemcpyDeviceToHost, m->stream));
+		m->stats.d2h_bytes += sizeof(int32_t) * (size_t) N * n;
+		if(probs_out) {
+			CUDA_TRY(m, cudaMemcpyAsync(probs_out, m->wt_probs.p, sizeof(double) * (size_t) N * n, cudaMemcpyDeviceToHost, m->stream));
+			m->stats.d2h_bytes += sizeof(double) * (size_t) N * n;
+		}
+	}
+	if(gamma_out && B) {
+		CUDA_TRY(m, cudaMemcpyAsync(gamma_out, m->gamma.p, sizeof(double) * (size_t) K * B, cudaMemcpyDeviceToHost, m->stream));
+		m->stats.d2h_bytes += sizeof(double) * (size_t) K * B;
+	}
+	CUDA_TRY(m, cudaStreamSynchronize(m->stream));
 	consume_injections(m);
 	return TRLDA_OK;
 }

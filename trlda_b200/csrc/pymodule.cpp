@@ -617,6 +617,58 @@ PyObject* LDA_predictive_log_likelihood(LDAObject* self, PyObject* args, PyObjec
 	return Py_BuildValue("(dL)", total, (long long) tokens);
 }
 
+// word_topics (no reference counterpart): trlda_word_topics
+PyObject* LDA_word_topics(LDAObject* self, PyObject* args, PyObject* kwds) {
+	REQUIRE_MODEL(self, nullptr);
+	const char* kwlist[] = {"docs", "num_topics", "latents", "max_iter", "threshold", nullptr};
+	Documents documents;
+	trlda_params params;
+	trlda_params_default(&params);
+	int n = 1;
+	PyObject* latents = nullptr;
+	if(!PyArg_ParseTupleAndKeywords(args, kwds, "O&|iOid", const_cast<char**>(kwlist), &docs_converter, &documents, &n, &latents,
+			&params.max_iter_inference, &params.threshold))
+		return nullptr;
+	npy_intp rows = 0, cols = 0;
+	PyObject* latents_arr = nullptr;
+	if(latents && latents != Py_None) {
+		latents_arr = as_farray(latents, &rows, &cols, "`latents`");
+		if(!latents_arr)
+			return nullptr;
+	}
+	const trlda_docs& view = documents.view;
+	npy_intp dims[2] = {view.num_docs > 0 ? (npy_intp) view.doc_ptr[view.num_docs] : 0, std::max(n, 0)};
+	PyObject* topics = PyArray_SimpleNew(2, dims, NPY_INT32);
+	PyObject* probs = topics ? PyArray_SimpleNew(2, dims, NPY_DOUBLE) : nullptr;
+	PyObject* gamma = probs ? new_farray(trlda_num_topics(self->m), view.num_docs) : nullptr;
+	if(!gamma) {
+		Py_XDECREF(topics);
+		Py_XDECREF(probs);
+		Py_XDECREF(latents_arr);
+		return nullptr;
+	}
+	int status;
+	const double* l = latents_arr ? static_cast<const double*>(PyArray_DATA((PyArrayObject*) latents_arr)) : nullptr;
+	int32_t* t = static_cast<int32_t*>(PyArray_DATA((PyArrayObject*) topics));
+	double* p = static_cast<double*>(PyArray_DATA((PyArrayObject*) probs));
+	double* g = static_cast<double*>(PyArray_DATA((PyArrayObject*) gamma));
+	Py_BEGIN_ALLOW_THREADS
+	status = trlda_word_topics(self->m, &view, l, (int) rows, (int64_t) cols, &params, n, t, p, g);
+	Py_END_ALLOW_THREADS
+	Py_XDECREF(latents_arr);
+	if(status != TRLDA_OK) {
+		Py_DECREF(topics);
+		Py_DECREF(probs);
+		Py_DECREF(gamma);
+		return raise_status(self->m, status);
+	}
+	PyObject* result = Py_BuildValue("(OOO)", topics, probs, gamma);
+	Py_DECREF(topics);
+	Py_DECREF(probs);
+	Py_DECREF(gamma);
+	return result;
+}
+
 // top_words (no reference counterpart): trlda_top_words
 PyObject* LDA_top_words(LDAObject* self, PyObject* args, PyObject* kwds) {
 	REQUIRE_MODEL(self, nullptr);
@@ -1025,6 +1077,20 @@ const char* predictive_log_likelihood_doc =
 	"log_likelihood / num_tokens and the perplexity exp(-log_likelihood / num_tokens); returning the pair lets batches\n"
 	"of held-out documents be added up.  The model's parameters are not changed.";
 
+const char* word_topics_doc =
+	"word_topics(docs, num_topics=1, latents=None, max_iter=100, threshold=0.001)\n\n"
+	"The num_topics (1 to 32, at most the model's num_topics) most probable topics of every (word, count) pair of `docs`\n"
+	"(the list or the (doc_ptr, word_ids, counts) form), computed on the GPU.  gamma is fitted exactly as update_variables\n"
+	"fits it (`latents` is the initial gamma, a fresh draw if None), then pair j with word w in document d gets\n"
+	"phi_jk = exp(s_jk) / sum_k' exp(s_jk'),  s_jk = psi(gamma_dk) + psi(lambda_kw) - psi(sum_v lambda_kv),\n"
+	"the responsibility of topic k for the word that the E-step uses, evaluated in float64 in both precision modes.\n"
+	"Returns the tuple (topics, probs, gamma): int32 and float64 arrays of shape (num_pairs, num_topics), row j for the j-th\n"
+	"pair in the given order, its topics by descending phi (equal phi: the smaller topic id first) and their phi; and\n"
+	"gamma (num_topics x num_documents, float64, Fortran order), the same as update_variables returns.  Pairs with count 0\n"
+	"and repeated words get rows like any other pair.  A token's topic is topics[j, 0]; the tokens of topic k in the batch\n"
+	"are counts[topics[:, 0] == k].sum().  Like update_variables, the call replaces the minibatch held on the GPU; the\n"
+	"model's parameters are not changed.";
+
 const char* top_words_doc =
 	"top_words(num_words=10)\n\n"
 	"The num_words (1 to 32, at most num_words of the model) most probable words of every topic, on the GPU: words ordered\n"
@@ -1079,6 +1145,7 @@ PyMethodDef LDA_methods[] = {
 		"lower_bound(docs, num_documents=-1, inference_method='VI', max_iter=100, num_samples=1, burn_in=2)"},
 	{"predictive_log_likelihood", (PyCFunction) LDA_predictive_log_likelihood, METH_VARARGS | METH_KEYWORDS,
 		predictive_log_likelihood_doc},
+	{"word_topics", (PyCFunction) LDA_word_topics, METH_VARARGS | METH_KEYWORDS, word_topics_doc},
 	{"top_words", (PyCFunction) LDA_top_words, METH_VARARGS | METH_KEYWORDS, top_words_doc},
 	{"cooccurrence", (PyCFunction) LDA_cooccurrence, METH_VARARGS | METH_KEYWORDS, cooccurrence_doc},
 	{"topic_distances", (PyCFunction) LDA_topic_distances, METH_VARARGS | METH_KEYWORDS, topic_distances_doc},

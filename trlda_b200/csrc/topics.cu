@@ -1,8 +1,10 @@
 // topics.cu — looking at a trained model: the most probable words of every topic (trlda_top_words), how many documents
 // of a corpus contain each of those words and each pair of them (trlda_cooccurrence), the counts behind the document
 // co-occurrence coherence measures (UMass, NPMI), and the Hellinger / Kullback-Leibler distances between the topics of one
-// or two models (trlda_topic_distances).  None has a counterpart in the reference.
+// or two models (trlda_topic_distances), and the most probable topics of every word of a document (trlda_word_topics).
+// None has a counterpart in the reference.
 #include "kernels.cuh"
+#include "special.cuh"
 
 #include <algorithm>
 #include <climits>
@@ -344,6 +346,142 @@ __global__ void k_distance_finish(const double* __restrict__ partial, int splits
 	}
 }
 
+// ---- topics of the words of documents --------------------------------------------------------------------------------
+// s_jk = psi(gamma_dk) + (psi(lambda_kw) - psi_rows_k) for pair j (word w, document d), phi_jk = softmax_k(s_jk), in fp64
+// from lambda in fp64 in both modes.  The second term is the same for every pair of word w, so the table pass evaluates it
+// once per (word of the call, topic) for one chunk of word ids, skipping the ids the call does not contain; psi(gamma) is
+// filled once per call.  The pair pass walks the chunk's pairs in the call's word-sorted token list (a word's pairs are
+// consecutive, so its table column is re-read from L1 / L2; a CTA takes a contiguous run of them, so that its warps share
+// the columns), one warp per pair with the lanes striding over k:
+//   1. s_jk for k = lane, lane + 32, ...: the lane's WT_LIST best (s, k) in registers, in the order of ranks_before
+//      (s descending, then k ascending; a total order);
+//   2. Sigma_k exp(s_jk - max): lane-strided in k order, then an xor butterfly, so the bits depend on K alone;
+//   3. n rounds of a warp arg-max over the lanes' list heads.  Only the winning lane pops its head; a lane whose list runs
+//      dry rescans its topics for the best WT_LIST ranked after the last one it gave.  Round r's result stays in lane r,
+//      and lanes < n write the pair's row at its original position.
+constexpr int WT_THREADS = 256;
+constexpr int WT_LIST = 4;                       // per-lane candidates kept in registers when n > 1
+constexpr size_t WT_TABLE = 256u << 20;          // bytes of the log-beta table per chunk, at most
+
+__global__ void __launch_bounds__(256) k_word_topics_table(const double* __restrict__ lambda, int K, int w0, int count,
+                                                           const int32_t* __restrict__ word_ptr,
+                                                           const double* __restrict__ psi_rows, double* __restrict__ table) {
+	for(int u = blockIdx.x; u < count; u += gridDim.x) {
+		if(word_ptr[w0 + u + 1] == word_ptr[w0 + u])
+			continue;
+		const double* col = lambda + (int64_t) (w0 + u) * K;
+		double* out = table + (int64_t) u * K;
+		for(int k = threadIdx.x; k < K; k += blockDim.x)
+			out[k] = digamma(__ldg(col + k)) - psi_rows[k];
+	}
+}
+
+// inserts (v, id) into the sorted list (lv, lk) of M entries, dropping the last one
+template <int M>
+__device__ __forceinline__ void list_insert(double (&lv)[M], int (&lk)[M], double v, int id) {
+	#pragma unroll
+	for(int i = 0; i < M; ++i)
+		if(ranks_before(v, id, lv[i], lk[i])) {
+			const double tv = lv[i];
+			const int tk = lk[i];
+			lv[i] = v;
+			lk[i] = id;
+			v = tv;
+			id = tk;
+		}
+}
+
+// the lane's best M entries ranked after (after_v, after_k) (M entries of -inf / INT_MAX when there are fewer)
+template <int M>
+__device__ __forceinline__ void lane_best(const double* __restrict__ g, const double* __restrict__ t, int K, int lane,
+                                          double after_v, int after_k, double (&lv)[M], int (&lk)[M]) {
+	#pragma unroll
+	for(int i = 0; i < M; ++i) {
+		lv[i] = -INFINITY;
+		lk[i] = INT_MAX;
+	}
+	#pragma unroll 4
+	for(int k = lane; k < K; k += 32) {
+		const double s = g[k] + t[k];
+		if(ranks_before(after_v, after_k, s, k) && ranks_before(s, k, lv[M - 1], lk[M - 1]))
+			list_insert<M>(lv, lk, s, k);
+	}
+}
+
+// a / b for 1 <= b <= 2^31 (b is a sum of exp(s - max) with one term 1), without the slow path of the fp64 division: a
+// float seed of 1/b, two Newton steps, and one correction of the quotient
+__device__ __forceinline__ double divide_by_sum(double a, double b) {
+	double r = (double) __fdividef(1.f, (float) b);
+	r = fma(r, fma(-b, r, 1.), r);
+	r = fma(r, fma(-b, r, 1.), r);
+	const double q = a * r;
+	return fma(fma(-q, b, a), r, q);
+}
+
+template <int M>
+__global__ void __launch_bounds__(WT_THREADS) k_word_topics_pairs(DeviceDocs docs, int w0, int w1,
+                                                                  const double* __restrict__ table,
+                                                                  const double* __restrict__ psi_gamma, int K, int n,
+                                                                  int32_t* __restrict__ topics, double* __restrict__ probs) {
+	const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = WT_THREADS / 32;
+	const int p0 = docs.word_ptr[w0], p1 = docs.word_ptr[w1];
+	const int per_cta = (p1 - p0 + (int) gridDim.x - 1) / (int) gridDim.x;
+	const int begin = p0 + (int) blockIdx.x * per_cta, end = min(p1, begin + per_cta);
+	for(int p = begin + warp; p < end; p += nw) {
+		const int64_t j = docs.tok_src[p];
+		const double* g = psi_gamma + (int64_t) docs.tok_doc[p] * K;
+		const double* t = table + (int64_t) (docs.word_ids[j] - w0) * K;
+		double lv[M];
+		int lk[M];
+		lane_best<M>(g, t, K, lane, INFINITY, -1, lv, lk);
+		// the maximum: a warp arg-max of the list heads
+		double top = lv[0];
+		#pragma unroll
+		for(int o = 16; o > 0; o >>= 1)
+			top = fmax(top, __shfl_xor_sync(0xffffffffu, top, o));
+		double sum = 0.;
+		#pragma unroll 2   // 4 spills registers around the branches of exp
+		for(int k = lane; k < K; k += 32)
+			sum += exp(g[k] + t[k] - top);
+		sum = warp_sum(sum);
+		int my_k = 0;
+		double my_v = -INFINITY;
+		for(int r = 0; r < n; ++r) {
+			double bv = lv[0];
+			int bk = lk[0];
+			#pragma unroll
+			for(int o = 16; o > 0; o >>= 1) {
+				const double ov = __shfl_xor_sync(0xffffffffu, bv, o);
+				const int ok = __shfl_xor_sync(0xffffffffu, bk, o);
+				if(ranks_before(ov, ok, bv, bk)) {
+					bv = ov;
+					bk = ok;
+				}
+			}
+			if(lane == r) {
+				my_k = bk;
+				my_v = bv;
+			}
+			if(r + 1 < n && (bk & 31) == lane) {   // the winner's head was taken
+				#pragma unroll
+				for(int i = 0; i + 1 < M; ++i) {
+					lv[i] = lv[i + 1];
+					lk[i] = lk[i + 1];
+				}
+				lv[M - 1] = -INFINITY;
+				lk[M - 1] = INT_MAX;
+				if(lk[0] == INT_MAX)
+					lane_best<M>(g, t, K, lane, bv, bk, lv, lk);
+			}
+		}
+		if(lane < n) {
+			topics[j * n + lane] = my_k;
+			if(probs)
+				probs[j * n + lane] = divide_by_sum(exp(my_v - top), sum);   // the same exp as in the sum
+		}
+	}
+}
+
 int sm_count() {
 	static const int count = [] {
 		int device = 0, c = 148;
@@ -439,6 +577,27 @@ void launch_distance_product(const DistancePlan& plan, const double* x, const do
                              double* partial, cudaStream_t s) {
 	const dim3 grid((unsigned) (plan.ld_x / DIST_TILE), (unsigned) (plan.ld_y / DIST_TILE), (unsigned) plan.splits);
 	k_distance_product<<<grid, DIST_THREADS, 0, s>>>(x, plan.ld_x, y, plan.ld_y, words / plan.splits, first ? 1 : 0, partial);
+}
+
+int word_topics_chunk_words(int K) { return (int) std::max<size_t>(1, std::min<size_t>(INT_MAX, WT_TABLE / (sizeof(double) * (size_t) K))); }
+
+void launch_word_topics_table(const double* lambda, int K, int w0, int count, const int32_t* word_ptr, const double* psi_rows,
+                              double* table, cudaStream_t s) {
+	if(count > 0)
+		k_word_topics_table<<<(unsigned) std::min(count, sm_count() * 16), std::min(256, (K + 31) / 32 * 32), 0, s>>>(
+			lambda, K, w0, count, word_ptr, psi_rows, table);
+}
+
+void launch_word_topics_pairs(const DeviceDocs& docs, int w0, int w1, const double* table, const double* psi_gamma, int K, int n,
+                              int32_t* topics, double* probs, cudaStream_t s) {
+	if(docs.N == 0)
+		return;
+	// the chunk's pairs are counted on the device; the grid is sized for all of the call's, at least 32 per CTA
+	const unsigned grid = (unsigned) std::min<int64_t>((docs.N + 31) / 32, (int64_t) sm_count() * 32);
+	if(n == 1)
+		k_word_topics_pairs<1><<<grid, WT_THREADS, 0, s>>>(docs, w0, w1, table, psi_gamma, K, n, topics, probs);
+	else
+		k_word_topics_pairs<WT_LIST><<<grid, WT_THREADS, 0, s>>>(docs, w0, w1, table, psi_gamma, K, n, topics, probs);
 }
 
 void launch_distance_finish(const DistancePlan& plan, const double* partial, int KA, int KB, int metric, const double* entropy,
