@@ -215,6 +215,30 @@ TRLDA_API int trlda_cooccurrence(trlda_model* m, const trlda_docs* docs, const i
 #define TRLDA_DISTANCE_KL        1
 TRLDA_API int trlda_topic_distances(trlda_model* m, trlda_model* other, int metric, double* out);
 
+/* Similar documents by topic.  gamma is K x cols column-major, as trlda_update_variables returns it (Gibbs theta too);
+ * a document's topic proportions are theta_d = gamma_d / sum_k gamma_dk, and the distance of two documents is the
+ * Hellinger distance of theirs, D(q, d) = sqrt(max(0, 1 - C_qd)), C_qd = sum_k sqrt(theta_qk theta_dk), in fp64 in both
+ * precision modes.  A negative, NaN or infinite entry, or a column whose sum is not positive, is an error
+ * (TRLDA_ERR_ARG), found before any result is written.
+ *
+ * trlda_index_documents replaces the model's document index with the cols documents of gamma (cols == 0: no index).
+ * The index stays on the device, sqrt(theta) in fp64 (8 bytes a topic and document), until it is replaced or the model is
+ * destroyed; building it stages gamma through a bounded buffer.  On any failure the model is left with no index.  At most
+ * INT32_MAX documents.
+ *
+ * trlda_similar_documents returns, for each of the Q = cols query documents, the n indexed documents nearest to it:
+ * ids_out and dist_out (may be NULL) are Q x n query-major, query q's list at ids_out + q*n, ordered by C descending and
+ * then by the smaller document id (distances non-decreasing; exact ties go to the smaller id).  The result is
+ * reproducible bit for bit and does not depend on the other queries of the call.  1 <= n <= min(32, indexed documents);
+ * Q = 0 does nothing.
+ *
+ * Neither call changes lambda, alpha, eta, the update count or the minibatches held on the device, and training does not
+ * change the index.  Multi-GPU: every rank searches its own index, no exchange; ids are local to the rank's index.  No
+ * reference counterpart. */
+TRLDA_API int trlda_index_documents(trlda_model* m, const double* gamma, int rows, int64_t cols);
+TRLDA_API int trlda_similar_documents(trlda_model* m, const double* gamma, int rows, int64_t cols, int n,
+                                      int64_t* ids_out, double* dist_out);
+
 /* ---- parity seams ---------------------------------------------------------------------------------------------
  * The reference draws gamma0 (lda.cpp:135) and Cumulative's lambda (cumulativelda.cpp:60) from libc rand()
  * inside updateParameters and offers no way to pass them in.  These two calls install values that the NEXT

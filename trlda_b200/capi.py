@@ -113,6 +113,8 @@ PROTOTYPES = {
 	'trlda_top_words': (C.c_int, [C.c_void_p, C.c_int, _P(C.c_int32), _dbl]),
 	'trlda_cooccurrence': (C.c_int, [C.c_void_p, _P(Docs), _P(C.c_int32), C.c_int, _P(C.c_int64), _P(C.c_int64)]),
 	'trlda_topic_distances': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, _dbl]),
+	'trlda_index_documents': (C.c_int, [C.c_void_p, _dbl, C.c_int, C.c_int64]),
+	'trlda_similar_documents': (C.c_int, [C.c_void_p, _dbl, C.c_int, C.c_int64, C.c_int, _P(C.c_int64), _dbl]),
 	'trlda_inject_initial_gamma': (C.c_int, [C.c_void_p, _dbl, C.c_int, C.c_int64]),
 	'trlda_inject_initial_lambda': (C.c_int, [C.c_void_p, _dbl, C.c_int, C.c_int]),
 	'trlda_comm_unique_id': (C.c_int, [C.c_void_p]),
@@ -425,6 +427,23 @@ class Model(object):
 		out = np.empty((self.K, k_other), order='F')
 		self._check(self._lib.trlda_topic_distances(self.h, None if other is None else other.h, DISTANCE[metric], _dptr(out)))
 		return out
+
+	def index_documents(self, gamma):
+		"""replaces the document index with sqrt(theta) of the columns of gamma (K x D), theta_d = gamma_d / sum_k gamma_dk;
+		D = 0 frees it.  The index stays on the device until replaced; it is not pickled"""
+		gamma = _fortran(gamma)
+		self._check(self._lib.trlda_index_documents(self.h, _dptr(gamma), gamma.shape[0], gamma.shape[1]))
+
+	def similar_documents(self, gamma, n=10):
+		"""(ids int64 Q x n, dist float64 Q x n): the n indexed documents nearest to each column of gamma (K x Q) under
+		the Hellinger distance of the topic proportions, nearest first, exact ties to the smaller id"""
+		gamma = _fortran(gamma)
+		q = gamma.shape[1]
+		ids = np.empty((q, max(int(n), 0)), dtype=np.int64)
+		dist = np.empty((q, max(int(n), 0)))
+		self._check(self._lib.trlda_similar_documents(self.h, _dptr(gamma), gamma.shape[0], q, int(n),
+			ids.ctypes.data_as(_P(C.c_int64)), _dptr(dist)))
+		return ids, dist
 
 	# ---- multi-GPU / instrumentation --------------------------------------------------------------------------------
 	def comm_init(self, unique_id, rank, nranks):

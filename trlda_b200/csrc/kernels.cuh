@@ -237,12 +237,17 @@ void launch_heldout_loglik(const DeviceDocs& held_out, int K, const double* lamb
 // topics.cu: the n (<= 32) most probable words of every topic of lambda (K x V, fp64), ordered by value descending, then
 // word id ascending.  The candidate pass cuts the words into top_words_chunks(K, V, n) chunks and writes every chunk's
 // best n of every topic to cand_v / cand_id (chunks x K x n); the merge pass writes topic k's list to ids + k*n and
-// lambda_kw / rows_k to prob + k*n.
+// lambda_kw / rows_k to prob + k*n.  The candidate pass serves any K x V column-major matrix: its leading dimension ld
+// may exceed K, and its column ids start at id0 (id0 + V <= INT_MAX).
 int top_words_chunks(int K, int V, int n);
-void launch_top_words_candidates(const double* lambda, int K, int V, int n, int chunks, double* cand_v, int32_t* cand_id,
-                                 cudaStream_t s);
+void launch_top_words_candidates(const double* lambda, int K, int ld, int V, int id0, int n, int chunks, double* cand_v,
+                                 int32_t* cand_id, cudaStream_t s);
 void launch_top_words_merge(const double* cand_v, const int32_t* cand_id, const double* rows, int K, int n, int chunks,
                             int32_t* ids, double* prob, cudaStream_t s);
+// the same merge into a running list: starts from init_v / init_id (K x n, may be null; may equal v / ids) and writes the
+// merged values (hellinger: sqrt(max(0, 1 - value))) to v and their ids to ids
+void launch_top_n_merge(const double* cand_v, const int32_t* cand_id, int K, int n, int chunks, const double* init_v,
+                        const int32_t* init_id, bool hellinger, int32_t* ids, double* v, cudaStream_t s);
 // counts[(k n + j) n + i] += number of documents of `docs` (CSR arrays only) holding both the words of ranks i and j of topic
 // k's list (a pair counts when its count is > 0).  map_ptr (V + 1) / map_entry: for word w, the entries topic * 32 + rank
 // of the lists it is on, at map_entry[map_ptr[w] .. map_ptr[w + 1])
@@ -273,6 +278,9 @@ void launch_distance_entropy(const double* entropy_part, int parts, int K, int l
 // partial[s] (ld_x x ld_y, column-major) = (first ? 0 : partial[s]) + X_s^T Y_s over split s of the chunk's words
 void launch_distance_product(const DistancePlan& plan, const double* x, const double* y, int words, bool first,
                              double* partial, cudaStream_t s);
+// the same for the first cols_y (a multiple of 128) columns of a Y whose rows are ld_y apart; partial[s] is ld_x x cols_y
+void launch_distance_product(const double* x, int ld_x, const double* y, int64_t ld_y, int cols_y, int splits, int words, bool first,
+                             double* partial, cudaStream_t s);
 // out[j KA + i] = sqrt(max(0, 1 - C_ij)) (metric 0) or max(0, entropy_i - C_ij) (metric 1), C = sum of the partials
 void launch_distance_finish(const DistancePlan& plan, const double* partial, int KA, int KB, int metric, const double* entropy,
                             double* out, cudaStream_t s);
@@ -287,6 +295,16 @@ void launch_word_topics_table(const double* lambda, int K, int w0, int count, co
                               double* table, cudaStream_t s);
 void launch_word_topics_pairs(const DeviceDocs& docs, int w0, int w1, const double* table, const double* psi_gamma, int K, int n,
                               int32_t* topics, double* probs, cudaStream_t s);
+// topics.cu: similar documents.  Operands are sqrt(theta), theta = gamma / column sum, topic-major: element (k, c) at
+// k * ld + c, with similar_rows(K) rows (zero beyond K) and ld = similar_ld(columns) (the product's tile; zero beyond).
+int similar_rows(int K);
+int64_t similar_ld(int64_t cols);
+// out[k * ld + c] = sqrt(gamma_kc / sum_k gamma_kc) for k < K, c < cols (gamma K x cols column-major; the padding is left as
+// it is); *flag |= 1 for a negative or non-finite entry, or a column whose sum is not positive and finite
+void launch_similar_prepare(const double* gamma, int K, int cols, int64_t ld, double* out, int* flag, cudaStream_t s);
+// aff[d * lda + q] = sum_{k < K} query[k * ldq + q] * index[k * ld + d] for q < nq, d < docs, as one fma chain in k order
+void launch_similar_stream(const double* index, int64_t ld, int K, int docs, const double* query, int ldq, int nq, double* aff,
+                           int lda, cudaStream_t s);
 // out[k] = lgamma(in[k])
 void launch_lgamma_vector(const double* in, int K, double* out, cudaStream_t s);
 

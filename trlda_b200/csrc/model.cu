@@ -282,6 +282,11 @@ struct trlda_model {
 	// trlda_word_topics: the call's document lengths, the scratch and the result of its word-sorted token list, the log-beta
 	// table of one chunk of words, psi(gamma) and the results
 	DevBuf wt_len, wt_scratch, wt_word_ptr, wt_tok_doc, wt_tok_src, wt_table, wt_psi_gamma, wt_topics, wt_probs;
+	// trlda_index_documents: the document index (sqrt(theta) of sim_docs documents, similar_rows(K) x sim_ld, topic-major);
+	// trlda_similar_documents: a block of queries prepared the same way, one affinity block, the candidate lists of its
+	// chunks and of their first merge, the running lists of all queries and the prepare pass's flag
+	DevBuf sim_index, sim_query, sim_aff, sim_cand_v, sim_cand_id, sim_merge_v, sim_merge_id, sim_res_v, sim_res_id, sim_flag;
+	int64_t sim_docs = 0, sim_ld = 0;
 	bool gamma_valid = false;
 
 	// parity seams
@@ -2433,7 +2438,8 @@ int trlda_top_words(trlda_model* m, int n, int32_t* ids_out, double* prob_out) {
 	TRY(compute_rows(m, m->lambda(), m->topic_rows.as<double>()));   // the row sums prepare_beta uses
 	{
 		Launch l(m, KK_MISC);
-		launch_top_words_candidates(m->lambda(), K, V, n, chunks, m->top_cand_v.as<double>(), m->top_cand_id.as<int32_t>(), m->stream);
+		launch_top_words_candidates(m->lambda(), K, K, V, 0, n, chunks, m->top_cand_v.as<double>(), m->top_cand_id.as<int32_t>(),
+		                            m->stream);
 	}
 	{
 		Launch l(m, KK_MISC);
@@ -2608,6 +2614,192 @@ int trlda_topic_distances(trlda_model* m, trlda_model* other, int metric, double
 	}
 	std::scoped_lock lock__(m->mu, other->mu);   // std::lock's deadlock avoidance, whatever order other callers use
 	return topic_distances(m, other, metric, out);
+}
+
+// ---- similar documents ----------------------------------------------------------------------------------------------
+static const int kMaxNeighbors = 32;               // one warp lane per rank in the merge
+static const size_t kSimStage = 256u << 20;        // bytes of raw gamma on the device at a time
+static const size_t kSimAffinity = 256u << 20;     // bytes of one affinity block (queries x documents), at most
+static const int kSimQueryBlock = 8192;            // queries per block of the product path
+// at most this many queries take the streaming path: it reads the index once per group of 8 queries (1.45 ms a group at
+// K = 1000, D = 2^20 on a B200), the product path costs the same (11.4 ms) for any Q up to its 128-query tile (DESIGN.md §4.2)
+static const int kSimStreamMax = 56;
+
+static const char* kSimBadGamma = "Gamma must be finite and non-negative, with a positive sum in every column.";
+
+// sqrt(theta) of the cols columns of host gamma (K x cols) into out (element (k, c) at k * ld + c), staged through the
+// device in blocks of columns; the prepare pass raises m->sim_flag for bad columns
+static int prepare_columns(trlda_model* m, const double* gamma, int64_t cols, int64_t ld, double* out, DevBuf& stage) {
+	const int K = m->K;
+	const int64_t block = std::max<int64_t>(1, std::min<int64_t>(cols, (int64_t) (kSimStage / (sizeof(double) * K))));
+	CUDA_TRY(m, stage.ensure(sizeof(double) * K * block));
+	for(int64_t c0 = 0; c0 < cols; c0 += block) {
+		const int64_t nc = std::min(block, cols - c0);
+		CUDA_TRY(m, cudaMemcpyAsync(stage.p, gamma + c0 * K, sizeof(double) * K * nc, cudaMemcpyHostToDevice, m->stream));
+		m->stats.h2d_bytes += sizeof(double) * K * nc;
+		Launch l(m, KK_MISC);
+		launch_similar_prepare(stage.as<double>(), K, (int) nc, ld, out + c0, m->sim_flag.as<int>(), m->stream);
+	}
+	return TRLDA_OK;
+}
+
+// the prepare pass's flag, read back (the stream is synchronised)
+static int read_flag(trlda_model* m, int* bad) {
+	int* h = m->readback.as<int>();
+	CUDA_TRY(m, cudaMemcpyAsync(h, m->sim_flag.p, sizeof(int), cudaMemcpyDeviceToHost, m->stream));
+	CUDA_TRY(m, cudaStreamSynchronize(m->stream));
+	m->stats.d2h_bytes += sizeof(int);
+	*bad = h[0];
+	return TRLDA_OK;
+}
+
+static int index_documents(trlda_model* m, const double* gamma, int rows, int64_t cols) {
+	if(rows != m->K || cols < 0 || (cols > 0 && !gamma))
+		return fail(m, TRLDA_ERR_ARG, "Gamma has wrong dimensionality.");
+	if(cols > INT32_MAX)
+		return fail(m, TRLDA_ERR_ARG, "Too many documents to index.");
+	if(cols == 0)
+		return TRLDA_OK;
+	TRY(ensure_small(m));
+	const int64_t ld = similar_ld(cols);
+	const size_t bytes = sizeof(double) * (size_t) similar_rows(m->K) * ld;
+	CUDA_TRY(m, m->sim_index.ensure(bytes));
+	CUDA_TRY(m, m->sim_flag.ensure(sizeof(int)));
+	CUDA_TRY(m, cudaMemsetAsync(m->sim_index.p, 0, bytes, m->stream));
+	CUDA_TRY(m, cudaMemsetAsync(m->sim_flag.p, 0, sizeof(int), m->stream));
+	DevBuf stage;   // freed on return: only the index stays
+	TRY(prepare_columns(m, gamma, cols, ld, m->sim_index.as<double>(), stage));
+	TRY(check_launch(m, "index_documents"));
+	int bad = 0;
+	TRY(read_flag(m, &bad));
+	if(bad)
+		return fail(m, TRLDA_ERR_ARG, kSimBadGamma);
+	m->sim_docs = cols;
+	m->sim_ld = ld;
+	return TRLDA_OK;
+}
+
+int trlda_index_documents(trlda_model* m, const double* gamma, int rows, int64_t cols) {
+	std::lock_guard<std::recursive_mutex> lock__(m->mu);
+	TRY(set_device(m));
+	// the old index goes first, so that the two never take memory together, and a failure leaves no index
+	m->sim_index.release();
+	m->sim_docs = m->sim_ld = 0;
+	const int status = index_documents(m, gamma, rows, cols);
+	if(status != TRLDA_OK || m->sim_docs == 0) {
+		m->sim_index.release();
+		m->sim_docs = m->sim_ld = 0;
+	}
+	return status;
+}
+
+int trlda_similar_documents(trlda_model* m, const double* gamma, int rows, int64_t cols, int n, int64_t* ids_out,
+                            double* dist_out) {
+	std::lock_guard<std::recursive_mutex> lock__(m->mu);
+	if(rows != m->K || cols < 0 || (cols > 0 && !gamma))
+		return fail(m, TRLDA_ERR_ARG, "Gamma has wrong dimensionality.");
+	if(m->sim_docs == 0)
+		return fail(m, TRLDA_ERR_ARG, "similar_documents: no documents are indexed.");
+	if(n < 1 || n > kMaxNeighbors || n > m->sim_docs)
+		return fail(m, TRLDA_ERR_ARG, "Number of neighbors must lie in [1, min(32, number of indexed documents)].");
+	if(!ids_out)
+		return fail(m, TRLDA_ERR_ARG, "similar_documents: no output buffer.");
+	if(cols == 0)
+		return TRLDA_OK;
+	TRY(set_device(m));
+	TRY(ensure_small(m));
+	const int K = m->K, kp = similar_rows(K), D = (int) m->sim_docs;
+	const int64_t Q = cols, ld = m->sim_ld;
+	const char* env = getenv("TRLDA_SIMILAR_STREAM_MAX");   // measurement knob for the crossover of the two paths
+	const int stream_max = env ? std::max(0, std::min(atoi(env), kSimQueryBlock)) : kSimStreamMax;
+	const bool streaming = Q <= stream_max;
+	// streaming: every query in one block, affinity rows = queries; product: blocks of kSimQueryBlock, rows padded to the tile
+	const int qmax = (int) std::min<int64_t>(Q, streaming ? stream_max : kSimQueryBlock);
+	const int ldq_max = (int) similar_ld(qmax);
+	const int lda_max = streaming ? qmax : ldq_max;
+	const int64_t dblock = std::min<int64_t>(similar_ld(D), std::max<int64_t>(128, (int64_t) (kSimAffinity / (sizeof(double) * lda_max)) / 128 * 128));
+	// the top n of every query over an affinity block's chunks; many chunks are merged in two levels, G groups of P chunks
+	// (chunk p * G + g is chunk p of group g, so group g's lists are rows g * qb + q of a G * qb-row merge)
+	auto chunking = [&](int qb, int nd, int* groups) {
+		int chunks = top_words_chunks(qb, nd, n);
+		*groups = 1;
+		if(chunks > 32) {
+			*groups = (int) std::ceil(std::sqrt((double) chunks));
+			chunks = (chunks + *groups - 1) / *groups * *groups;
+		}
+		return chunks;
+	};
+	int groups = 1;
+	const int nd_max = (int) std::min<int64_t>(dblock, D), q_last = (int) (Q - (Q - 1) / qmax * qmax);
+	const size_t cands = std::max((size_t) chunking(qmax, nd_max, &groups) * qmax, (size_t) chunking(q_last, nd_max, &groups) * q_last) * n;
+	CUDA_TRY(m, m->sim_query.ensure(sizeof(double) * (size_t) kp * ldq_max));
+	CUDA_TRY(m, m->sim_aff.ensure(sizeof(double) * (size_t) lda_max * dblock));
+	CUDA_TRY(m, m->sim_cand_v.ensure(sizeof(double) * cands));
+	CUDA_TRY(m, m->sim_cand_id.ensure(sizeof(int32_t) * cands));
+	CUDA_TRY(m, m->sim_merge_v.ensure(sizeof(double) * cands));
+	CUDA_TRY(m, m->sim_merge_id.ensure(sizeof(int32_t) * cands));
+	CUDA_TRY(m, m->sim_res_v.ensure(sizeof(double) * (size_t) Q * n));
+	CUDA_TRY(m, m->sim_res_id.ensure(sizeof(int32_t) * (size_t) Q * n));
+	CUDA_TRY(m, m->sim_flag.ensure(sizeof(int)));
+	CUDA_TRY(m, cudaMemsetAsync(m->sim_flag.p, 0, sizeof(int), m->stream));
+	DevBuf stage;
+	double* aff = m->sim_aff.as<double>();
+	for(int64_t q0 = 0; q0 < Q; q0 += qmax) {
+		const int qb = (int) std::min<int64_t>(qmax, Q - q0);
+		const int ldq = (int) similar_ld(qb), lda = streaming ? qb : ldq;
+		double* run_v = m->sim_res_v.as<double>() + q0 * n;
+		int32_t* run_id = m->sim_res_id.as<int32_t>() + q0 * n;
+		CUDA_TRY(m, cudaMemsetAsync(m->sim_query.p, 0, sizeof(double) * (size_t) kp * ldq, m->stream));
+		TRY(prepare_columns(m, gamma + q0 * K, qb, ldq, m->sim_query.as<double>(), stage));
+		for(int64_t d0 = 0; d0 < D; d0 += dblock) {
+			const int nd = (int) std::min<int64_t>(dblock, D - d0);
+			const double* index = m->sim_index.as<double>() + d0;
+			{
+				Launch l(m, KK_MISC);
+				if(streaming)
+					launch_similar_stream(index, ld, K, nd, m->sim_query.as<double>(), ldq, qb, aff, lda, m->stream);
+				else
+					launch_distance_product(m->sim_query.as<double>(), ldq, index, ld, (int) similar_ld(nd), 1, kp, true, aff, m->stream);
+			}
+			int chunks = chunking(qb, nd, &groups);
+			{
+				Launch l(m, KK_MISC);
+				launch_top_words_candidates(aff, qb, lda, nd, (int) d0, n, chunks, m->sim_cand_v.as<double>(), m->sim_cand_id.as<int32_t>(),
+				                            m->stream);
+			}
+			const double* src_v = m->sim_cand_v.as<double>();
+			const int32_t* src_id = m->sim_cand_id.as<int32_t>();
+			if(groups > 1) {
+				Launch l(m, KK_MISC);
+				launch_top_n_merge(src_v, src_id, groups * qb, n, chunks / groups, nullptr, nullptr, false, m->sim_merge_id.as<int32_t>(),
+				                   m->sim_merge_v.as<double>(), m->stream);
+				src_v = m->sim_merge_v.as<double>();
+				src_id = m->sim_merge_id.as<int32_t>();
+				chunks = groups;
+			}
+			{
+				Launch l(m, KK_MISC);   // into the running list; the last block turns C into the distance
+				launch_top_n_merge(src_v, src_id, qb, n, chunks, d0 > 0 ? run_v : nullptr, d0 > 0 ? run_id : nullptr, d0 + nd >= D,
+				                   run_id, run_v, m->stream);
+			}
+		}
+	}
+	TRY(check_launch(m, "similar_documents"));
+	int bad = 0;
+	TRY(read_flag(m, &bad));
+	if(bad)
+		return fail(m, TRLDA_ERR_ARG, kSimBadGamma);
+	const size_t listed = (size_t) Q * n;
+	CUDA_TRY(m, m->readback.ensure(sizeof(int32_t) * listed));
+	int32_t* h = m->readback.as<int32_t>();
+	CUDA_TRY(m, cudaMemcpyAsync(h, m->sim_res_id.p, sizeof(int32_t) * listed, cudaMemcpyDeviceToHost, m->stream));
+	if(dist_out)
+		CUDA_TRY(m, cudaMemcpyAsync(dist_out, m->sim_res_v.p, sizeof(double) * listed, cudaMemcpyDeviceToHost, m->stream));
+	CUDA_TRY(m, cudaStreamSynchronize(m->stream));
+	m->stats.d2h_bytes += (sizeof(int32_t) + (dist_out ? sizeof(double) : 0)) * listed;
+	for(size_t i = 0; i < listed; ++i)
+		ids_out[i] = h[i];
+	return TRLDA_OK;
 }
 
 int trlda_debug_global_csc(trlda_model* m, const int32_t* len, const int32_t* ids, int ranks, int64_t max_docs, int64_t max_pairs,

@@ -787,6 +787,67 @@ PyObject* LDA_topic_distances(LDAObject* self, PyObject* args, PyObject* kwds) {
 	return out;
 }
 
+// index_documents (no reference counterpart): trlda_index_documents
+PyObject* LDA_index_documents(LDAObject* self, PyObject* args, PyObject* kwds) {
+	REQUIRE_MODEL(self, nullptr);
+	const char* kwlist[] = {"gamma", nullptr};
+	PyObject* gamma = nullptr;
+	if(!PyArg_ParseTupleAndKeywords(args, kwds, "O", const_cast<char**>(kwlist), &gamma))
+		return nullptr;
+	npy_intp rows = 0, cols = 0;
+	PyObject* arr = as_farray(gamma, &rows, &cols, "Gamma");
+	if(!arr)
+		return nullptr;
+	int status;
+	const double* g = static_cast<const double*>(PyArray_DATA((PyArrayObject*) arr));
+	Py_BEGIN_ALLOW_THREADS
+	status = trlda_index_documents(self->m, g, (int) rows, (int64_t) cols);
+	Py_END_ALLOW_THREADS
+	Py_DECREF(arr);
+	if(status != TRLDA_OK)
+		return raise_status(self->m, status);
+	Py_RETURN_NONE;
+}
+
+// similar_documents (no reference counterpart): trlda_similar_documents
+PyObject* LDA_similar_documents(LDAObject* self, PyObject* args, PyObject* kwds) {
+	REQUIRE_MODEL(self, nullptr);
+	const char* kwlist[] = {"gamma", "num_neighbors", nullptr};
+	PyObject* gamma = nullptr;
+	int n = 10;
+	if(!PyArg_ParseTupleAndKeywords(args, kwds, "O|i", const_cast<char**>(kwlist), &gamma, &n))
+		return nullptr;
+	npy_intp rows = 0, cols = 0;
+	PyObject* arr = as_farray(gamma, &rows, &cols, "Gamma");
+	if(!arr)
+		return nullptr;
+	npy_intp dims[2] = {cols, std::max(n, 0)};
+	PyObject* ids = PyArray_SimpleNew(2, dims, NPY_INT64);
+	PyObject* dist = ids ? PyArray_SimpleNew(2, dims, NPY_DOUBLE) : nullptr;
+	if(!dist) {
+		Py_XDECREF(ids);
+		Py_DECREF(arr);
+		return nullptr;
+	}
+	int status;
+	const double* g = static_cast<const double*>(PyArray_DATA((PyArrayObject*) arr));
+	int64_t* i = static_cast<int64_t*>(PyArray_DATA((PyArrayObject*) ids));
+	double* d = static_cast<double*>(PyArray_DATA((PyArrayObject*) dist));
+	Py_BEGIN_ALLOW_THREADS
+	status = trlda_similar_documents(self->m, g, (int) rows, (int64_t) cols, n, i, d);
+	Py_END_ALLOW_THREADS
+	Py_DECREF(arr);
+	if(status != TRLDA_OK) {
+		Py_DECREF(ids);
+		Py_DECREF(dist);
+		return raise_status(self->m, status);
+	}
+	PyObject* result = Py_BuildValue("(OO)", ids, dist);
+	Py_DECREF(ids);
+	Py_DECREF(dist);
+	return result;
+}
+
 PyObject* LDA_str(PyObject* self_) {                                      // ldainterface.cpp:473-490
 	LDAObject* self = (LDAObject*) self_;
 	REQUIRE_MODEL(self, nullptr);
@@ -1127,6 +1188,27 @@ const char* topic_distances_doc =
 	"    print(d[rows, cols].mean())\n\n"
 	"The model's parameters are not changed.";
 
+const char* index_documents_doc =
+	"index_documents(gamma)\n\n"
+	"Replaces the model's document index with the documents of `gamma` (num_topics x D, as update_variables returns it;\n"
+	"Gibbs theta works too), for similar_documents.  A document's topic proportions are theta_d = gamma_d / sum_k gamma_dk.\n"
+	"The index stays on the GPU, 8 bytes per topic and document (8.4 GB for 1000 topics and 2^20 documents), until it is\n"
+	"replaced, emptied with a gamma of 0 columns, or the model is deleted.  It is not pickled with the model, and training\n"
+	"does not change it.  Gamma must be finite and non-negative, with a positive sum in every column; on any error the\n"
+	"model is left with no index.  The model's parameters are not changed.";
+
+const char* similar_documents_doc =
+	"similar_documents(gamma, num_neighbors=10)\n\n"
+	"The num_neighbors indexed documents nearest to each of the Q query documents of `gamma` (num_topics x Q), under the\n"
+	"Hellinger distance of their topic proportions: D(q, d) = sqrt(max(0, 1 - sum_k sqrt(theta_qk theta_dk))), in float64\n"
+	"on the GPU.  Returns (ids, distances), int64 and float64 arrays of shape (Q, num_neighbors): row q lists the column\n"
+	"numbers of the indexed gamma, nearest first; exact ties go to the smaller id.  The result is reproducible bit for bit\n"
+	"and does not depend on the other queries.  1 <= num_neighbors <= min(32, indexed documents).  On several GPUs every\n"
+	"rank searches its own index.\n\n"
+	"    model.index_documents(model.update_variables(corpus)[0])\n"
+	"    ids, dist = model.similar_documents(model.update_variables(queries)[0], 10)\n\n"
+	"The model's parameters are not changed.";
+
 PyGetSetDef LDA_getset[] = {
 	{"num_topics", (getter) LDA_num_topics, nullptr, "Number of topics.", nullptr},
 	{"num_words", (getter) LDA_num_words, nullptr, "Number of words.", nullptr},
@@ -1149,6 +1231,8 @@ PyMethodDef LDA_methods[] = {
 	{"top_words", (PyCFunction) LDA_top_words, METH_VARARGS | METH_KEYWORDS, top_words_doc},
 	{"cooccurrence", (PyCFunction) LDA_cooccurrence, METH_VARARGS | METH_KEYWORDS, cooccurrence_doc},
 	{"topic_distances", (PyCFunction) LDA_topic_distances, METH_VARARGS | METH_KEYWORDS, topic_distances_doc},
+	{"index_documents", (PyCFunction) LDA_index_documents, METH_VARARGS | METH_KEYWORDS, index_documents_doc},
+	{"similar_documents", (PyCFunction) LDA_similar_documents, METH_VARARGS | METH_KEYWORDS, similar_documents_doc},
 	{nullptr, nullptr, 0, nullptr}};
 
 PyGetSetDef OnlineLDA_getset[] = {

@@ -1,8 +1,9 @@
 // topics.cu — looking at a trained model: the most probable words of every topic (trlda_top_words), how many documents
 // of a corpus contain each of those words and each pair of them (trlda_cooccurrence), the counts behind the document
 // co-occurrence coherence measures (UMass, NPMI), and the Hellinger / Kullback-Leibler distances between the topics of one
-// or two models (trlda_topic_distances), and the most probable topics of every word of a document (trlda_word_topics).
-// None has a counterpart in the reference.
+// or two models (trlda_topic_distances), the most probable topics of every word of a document (trlda_word_topics), and the
+// indexed documents nearest to a query document under the Hellinger distance of their topic proportions
+// (trlda_index_documents, trlda_similar_documents).  None has a counterpart in the reference.
 #include "kernels.cuh"
 #include "special.cuh"
 
@@ -35,8 +36,10 @@ __device__ __forceinline__ bool ranks_before(double a, int ia, double b, int ib)
 	return a > b || (a == b && ia < ib);
 }
 
-__global__ void __launch_bounds__(TOP_THREADS) k_top_words_candidates(const double* __restrict__ lambda, int K, int V, int n,
-                                                                       int chunk, double* __restrict__ cand_v,
+// row k of the K x V column-major matrix `lambda` (leading dimension ld); the ids of its columns start at id0
+__global__ void __launch_bounds__(TOP_THREADS) k_top_words_candidates(const double* __restrict__ lambda, int K, int ld,
+                                                                       int V, int id0, int n, int chunk,
+                                                                       double* __restrict__ cand_v,
                                                                        int32_t* __restrict__ cand_id) {
 	extern __shared__ double list_v[];                                          // n x TOP_THREADS, rank-major
 	int32_t* list_id = reinterpret_cast<int32_t*>(list_v + n * TOP_THREADS);   // n x TOP_THREADS
@@ -55,7 +58,7 @@ __global__ void __launch_bounds__(TOP_THREADS) k_top_words_candidates(const doub
 		double v[TOP_UNROLL];
 		#pragma unroll
 		for(int u = 0; u < TOP_UNROLL; ++u)
-			v[u] = w + u < w1 ? __ldg(col + (int64_t) (w + u) * K) : -INFINITY;
+			v[u] = w + u < w1 ? __ldg(col + (int64_t) (w + u) * ld) : -INFINITY;
 		#pragma unroll
 		for(int u = 0; u < TOP_UNROLL; ++u) {
 			if(v[u] > nth) {
@@ -65,7 +68,7 @@ __global__ void __launch_bounds__(TOP_THREADS) k_top_words_candidates(const doub
 					list_id[p * TOP_THREADS + t] = list_id[(p - 1) * TOP_THREADS + t];
 				}
 				list_v[p * TOP_THREADS + t] = v[u];
-				list_id[p * TOP_THREADS + t] = w + u;
+				list_id[p * TOP_THREADS + t] = id0 + w + u;
 				nth = list_v[(n - 1) * TOP_THREADS + t];
 			}
 		}
@@ -77,17 +80,35 @@ __global__ void __launch_bounds__(TOP_THREADS) k_top_words_candidates(const doub
 	}
 }
 
+// what the merge writes for a list entry of value v in row k
+struct MergeDivide {          // trlda_top_words: E[beta_kw] = lambda_kw / rows_k
+	const double* rows;
+	__device__ double operator()(double v, int k) const { return v / rows[k]; }
+};
+struct MergeKeep {            // a running list that later merges continue
+	__device__ double operator()(double v, int) const { return v; }
+};
+struct MergeHellinger {       // trlda_similar_documents: the Hellinger distance sqrt(max(0, 1 - C))
+	__device__ double operator()(double v, int) const { return sqrt(fmax(0., 1. - v)); }
+};
+
+// init_v / init_id (may be null): a sorted list per row to start from, in the layout of the output (row k at k*n); lane i
+// reads entry i before and writes entry i after the merge, so the output may be the initial list itself
+template <class Epilogue>
 __global__ void __launch_bounds__(TOP_MERGE_THREADS) k_top_words_merge(const double* __restrict__ cand_v,
-                                                                        const int32_t* __restrict__ cand_id,
-                                                                        const double* __restrict__ rows, int K, int n,
-                                                                        int chunks, int32_t* __restrict__ ids,
-                                                                        double* __restrict__ prob) {
+                                                                        const int32_t* __restrict__ cand_id, int K, int n,
+                                                                        int chunks, const double* init_v, const int32_t* init_id,
+                                                                        Epilogue epilogue, int32_t* ids, double* prob) {
 	const int lane = threadIdx.x & 31;
 	const int k = blockIdx.x * (TOP_MERGE_THREADS / 32) + (threadIdx.x >> 5);
 	if(k >= K)
 		return;
 	double best_v = -INFINITY;
 	int best_id = INT_MAX;
+	if(init_v && lane < n) {
+		best_v = init_v[(int64_t) k * n + lane];
+		best_id = init_id[(int64_t) k * n + lane];
+	}
 	const int r = 31 - lane;   // the chunk's list, reversed
 	for(int c = 0; c < chunks; ++c) {
 		const int64_t at = ((int64_t) c * K + k) * n + r;
@@ -110,7 +131,7 @@ __global__ void __launch_bounds__(TOP_MERGE_THREADS) k_top_words_merge(const dou
 	}
 	if(lane < n) {
 		ids[(int64_t) k * n + lane] = best_id;
-		prob[(int64_t) k * n + lane] = best_v / rows[k];
+		prob[(int64_t) k * n + lane] = epilogue(best_v, k);
 	}
 }
 
@@ -254,15 +275,16 @@ __global__ void k_distance_entropy(const double* __restrict__ entropy_part, int 
 	entropy[k] = acc;
 }
 
+// partial s holds ld_x x (gridDim.y tiles) elements; y's rows are ld_y apart, which may exceed the columns the grid covers
 __global__ void __launch_bounds__(DIST_THREADS, 1) k_distance_product(const double* __restrict__ x, int ld_x,
-                                                                      const double* __restrict__ y, int ld_y,
+                                                                      const double* __restrict__ y, int64_t ld_y,
                                                                       int split_words, int first,
                                                                       double* __restrict__ partial) {
 	__shared__ __align__(16) double xs[2][DIST_BK][DIST_TILE];
 	__shared__ __align__(16) double ys[2][DIST_BK][DIST_TILE];
 	const int t = threadIdx.x, tr = t & 15, tc = t >> 4;
 	const int i0 = blockIdx.x * DIST_TILE, j0 = blockIdx.y * DIST_TILE;
-	double* out = partial + (int64_t) blockIdx.z * ld_x * ld_y;
+	double* out = partial + (int64_t) blockIdx.z * ld_x * gridDim.y * DIST_TILE;
 
 	// element (a, b) of the thread's block: row i0 + orow(a), column j0 + orow(b)
 	auto orow = [](int q, int a) { return (a < 4 ? 0 : 64) + q * 4 + (a & 3); };
@@ -482,6 +504,106 @@ __global__ void __launch_bounds__(WT_THREADS) k_word_topics_pairs(DeviceDocs doc
 	}
 }
 
+// ---- similar documents ------------------------------------------------------------------------------------------------
+// C_qd = sum_k sqrt(theta_qk) sqrt(theta_dk), theta = gamma / column sum, D = sqrt(max(0, 1 - C)): the Hellinger distance of
+// the topic distributions of two documents.  The index holds sqrt(theta) of its D documents in the layout k_distance_product
+// reads: element (k, d) at k * ld + d, ld = D rounded up to DIST_TILE, with zero rows up to K rounded up to DIST_BK.
+// Prepare: one CTA per 32 columns of gamma.  Warp w sums columns w, w + 8, ... lane-strided in k order and then by an xor
+// butterfly, so a column's sum depends on K and its own values alone, and an equal query column gives a bitwise equal
+// operand.  The columns then go through a 32 x 32 shared-memory transpose: coalesced reads of gamma, coalesced writes of
+// runs of 32 documents.
+// Stream (few queries): one thread per document of the block and up to SIM_GROUP queries per CTA, the CTAs of one run of
+// documents for different query groups next to each other in the grid, so that they meet the same index lines in L2.  A
+// thread walks k ascending with acc_q = fma(q_qk, x_kd, acc_q) from 0: the chain of the product's element (q, d), whose
+// extra zero rows add nothing, so both paths give the same C bit for bit.
+constexpr int SIM_PREP_COLS = 32;
+constexpr int SIM_GROUP = 8;                  // queries per CTA of the streaming pass, an accumulator each
+constexpr int SIM_STREAM_THREADS = 256;
+constexpr int SIM_KT = 64;                    // topics of the queries staged in shared memory at a time
+
+__global__ void __launch_bounds__(256) k_similar_prepare(const double* __restrict__ gamma, int K, int cols, int64_t ld,
+                                                         double* __restrict__ out, int* __restrict__ flag) {
+	__shared__ double sum_s[SIM_PREP_COLS];
+	__shared__ double tile[SIM_PREP_COLS][SIM_PREP_COLS + 1];
+	const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+	const int c0 = blockIdx.x * SIM_PREP_COLS;
+	int bad = 0;
+	for(int j = warp; j < SIM_PREP_COLS; j += 8) {
+		const int c = c0 + j;
+		double sum = 0.;
+		if(c < cols) {
+			const double* col = gamma + (int64_t) c * K;
+			for(int k = lane; k < K; k += 32) {
+				const double v = col[k];
+				bad |= !(v >= 0.) || isinf(v);
+				sum += v;
+			}
+		}
+		sum = warp_sum(sum);
+		if(lane == 0) {
+			bad |= c < cols && !(sum > 0. && sum < INFINITY);
+			sum_s[j] = sum;
+		}
+	}
+	if(bad)
+		atomicOr(flag, 1);
+	__syncthreads();
+	for(int k0 = 0; k0 < K; k0 += SIM_PREP_COLS) {
+		for(int j = warp; j < SIM_PREP_COLS; j += 8) {
+			const int c = c0 + j, k = k0 + lane;
+			if(c < cols && k < K)
+				tile[j][lane] = sqrt(gamma[(int64_t) c * K + k] / sum_s[j]);
+		}
+		__syncthreads();
+		for(int j = warp; j < SIM_PREP_COLS; j += 8) {
+			const int k = k0 + j, c = c0 + lane;
+			if(k < K && c < cols)
+				out[(int64_t) k * ld + c] = tile[lane][j];
+		}
+		__syncthreads();
+	}
+}
+
+// aff[d * lda + q] = C_qd for the nq queries of `query` (element (k, q) at k * ldq + q) and the documents d < docs of
+// `index`; the grid is (document runs) x groups, group g taking queries g * SIM_GROUP ..
+template <int G>
+__global__ void __launch_bounds__(SIM_STREAM_THREADS) k_similar_stream(const double* __restrict__ index, int64_t ld, int K,
+                                                                       int docs, const double* __restrict__ query, int ldq,
+                                                                       int nq, int groups, double* __restrict__ aff,
+                                                                       int lda) {
+	__shared__ __align__(16) double qs[SIM_KT][G];
+	const int g = blockIdx.x % groups, q0 = g * SIM_GROUP;
+	const int d = (blockIdx.x / groups) * SIM_STREAM_THREADS + threadIdx.x;
+	const int mine = min(G, nq - q0);
+	double acc[G];
+	#pragma unroll
+	for(int i = 0; i < G; ++i)
+		acc[i] = 0.;
+	const double* col = index + min(d, docs - 1);
+	for(int k0 = 0; k0 < K; k0 += SIM_KT) {
+		const int kn = min(SIM_KT, K - k0);
+		__syncthreads();
+		for(int e = threadIdx.x; e < SIM_KT * G; e += SIM_STREAM_THREADS) {
+			const int kk = e / G, i = e - kk * G;
+			qs[kk][i] = kk < kn && i < mine ? query[(int64_t) (k0 + kk) * ldq + q0 + i] : 0.;
+		}
+		__syncthreads();
+		#pragma unroll 8
+		for(int kk = 0; kk < kn; ++kk) {
+			const double x = __ldg(col + (int64_t) (k0 + kk) * ld);
+			#pragma unroll
+			for(int i = 0; i < G; ++i)
+				acc[i] = fma(qs[kk][i], x, acc[i]);
+		}
+	}
+	if(d < docs) {
+		#pragma unroll
+		for(int i = 0; i < G; ++i)
+			if(i < mine)
+				aff[(int64_t) d * lda + q0 + i] = acc[i];
+	}
+}
+
 int sm_count() {
 	static const int count = [] {
 		int device = 0, c = 148;
@@ -506,17 +628,27 @@ int top_words_chunks(int K, int V, int n) {
 	return (V + chunk - 1) / chunk;
 }
 
-void launch_top_words_candidates(const double* lambda, int K, int V, int n, int chunks, double* cand_v, int32_t* cand_id,
-                                 cudaStream_t s) {
+void launch_top_words_candidates(const double* lambda, int K, int ld, int V, int id0, int n, int chunks, double* cand_v,
+                                 int32_t* cand_id, cudaStream_t s) {
 	const int chunk = (V + chunks - 1) / chunks;
 	const dim3 grid((unsigned) ((K + TOP_THREADS - 1) / TOP_THREADS), (unsigned) chunks);
-	k_top_words_candidates<<<grid, TOP_THREADS, top_words_smem(n), s>>>(lambda, K, V, n, chunk, cand_v, cand_id);
+	k_top_words_candidates<<<grid, TOP_THREADS, top_words_smem(n), s>>>(lambda, K, ld, V, id0, n, chunk, cand_v, cand_id);
 }
 
 void launch_top_words_merge(const double* cand_v, const int32_t* cand_id, const double* rows, int K, int n, int chunks,
                             int32_t* ids, double* prob, cudaStream_t s) {
 	const int per_block = TOP_MERGE_THREADS / 32;
-	k_top_words_merge<<<(K + per_block - 1) / per_block, TOP_MERGE_THREADS, 0, s>>>(cand_v, cand_id, rows, K, n, chunks, ids, prob);
+	k_top_words_merge<<<(K + per_block - 1) / per_block, TOP_MERGE_THREADS, 0, s>>>(cand_v, cand_id, K, n, chunks, nullptr,
+	                                                                                nullptr, MergeDivide{rows}, ids, prob);
+}
+
+void launch_top_n_merge(const double* cand_v, const int32_t* cand_id, int K, int n, int chunks, const double* init_v,
+                        const int32_t* init_id, bool hellinger, int32_t* ids, double* v, cudaStream_t s) {
+	const int per_block = TOP_MERGE_THREADS / 32, blocks = (K + per_block - 1) / per_block;
+	if(hellinger)
+		k_top_words_merge<<<blocks, TOP_MERGE_THREADS, 0, s>>>(cand_v, cand_id, K, n, chunks, init_v, init_id, MergeHellinger{}, ids, v);
+	else
+		k_top_words_merge<<<blocks, TOP_MERGE_THREADS, 0, s>>>(cand_v, cand_id, K, n, chunks, init_v, init_id, MergeKeep{}, ids, v);
 }
 
 void launch_cooccurrence(const DeviceDocs& docs, int K, int n, const int32_t* map_ptr, const int32_t* map_entry,
@@ -575,8 +707,13 @@ void launch_distance_entropy(const double* entropy_part, int parts, int K, int l
 
 void launch_distance_product(const DistancePlan& plan, const double* x, const double* y, int words, bool first,
                              double* partial, cudaStream_t s) {
-	const dim3 grid((unsigned) (plan.ld_x / DIST_TILE), (unsigned) (plan.ld_y / DIST_TILE), (unsigned) plan.splits);
-	k_distance_product<<<grid, DIST_THREADS, 0, s>>>(x, plan.ld_x, y, plan.ld_y, words / plan.splits, first ? 1 : 0, partial);
+	launch_distance_product(x, plan.ld_x, y, plan.ld_y, plan.ld_y, plan.splits, words, first, partial, s);
+}
+
+void launch_distance_product(const double* x, int ld_x, const double* y, int64_t ld_y, int cols_y, int splits, int words, bool first,
+                             double* partial, cudaStream_t s) {
+	const dim3 grid((unsigned) (ld_x / DIST_TILE), (unsigned) (cols_y / DIST_TILE), (unsigned) splits);
+	k_distance_product<<<grid, DIST_THREADS, 0, s>>>(x, ld_x, y, ld_y, words / splits, first ? 1 : 0, partial);
 }
 
 int word_topics_chunk_words(int K) { return (int) std::max<size_t>(1, std::min<size_t>(INT_MAX, WT_TABLE / (sizeof(double) * (size_t) K))); }
@@ -605,6 +742,31 @@ void launch_distance_finish(const DistancePlan& plan, const double* partial, int
 	const int64_t n = (int64_t) KA * KB;
 	const unsigned blocks = (unsigned) std::min<int64_t>((n + 255) / 256, (int64_t) sm_count() * 16);
 	k_distance_finish<<<blocks, 256, 0, s>>>(partial, plan.splits, plan.ld_x, plan.ld_y, KA, KB, metric, entropy, out);
+}
+
+int similar_rows(int K) { return (K + DIST_BK - 1) / DIST_BK * DIST_BK; }
+
+int64_t similar_ld(int64_t cols) { return (cols + DIST_TILE - 1) / DIST_TILE * DIST_TILE; }
+
+void launch_similar_prepare(const double* gamma, int K, int cols, int64_t ld, double* out, int* flag, cudaStream_t s) {
+	if(cols > 0)
+		k_similar_prepare<<<(unsigned) ((cols + SIM_PREP_COLS - 1) / SIM_PREP_COLS), 256, 0, s>>>(gamma, K, cols, ld, out, flag);
+}
+
+void launch_similar_stream(const double* index, int64_t ld, int K, int docs, const double* query, int ldq, int nq, double* aff,
+                           int lda, cudaStream_t s) {
+	if(docs <= 0 || nq <= 0)
+		return;
+	const int groups = (nq + SIM_GROUP - 1) / SIM_GROUP;
+	const unsigned grid = (unsigned) (((int64_t) docs + SIM_STREAM_THREADS - 1) / SIM_STREAM_THREADS * groups);
+	if(nq == 1)
+		k_similar_stream<1><<<grid, SIM_STREAM_THREADS, 0, s>>>(index, ld, K, docs, query, ldq, nq, groups, aff, lda);
+	else if(nq == 2)
+		k_similar_stream<2><<<grid, SIM_STREAM_THREADS, 0, s>>>(index, ld, K, docs, query, ldq, nq, groups, aff, lda);
+	else if(nq <= 4)
+		k_similar_stream<4><<<grid, SIM_STREAM_THREADS, 0, s>>>(index, ld, K, docs, query, ldq, nq, groups, aff, lda);
+	else
+		k_similar_stream<SIM_GROUP><<<grid, SIM_STREAM_THREADS, 0, s>>>(index, ld, K, docs, query, ldq, nq, groups, aff, lda);
 }
 
 }  // namespace trlda
